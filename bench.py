@@ -5,7 +5,7 @@ Objective API, the rooflines of the dominant kernels, parity against the CPU ora
 data that is timed, and the CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c1|c2|c3|c4|c5] [--no-target]
+                    [--workload c1|c2|c3|c4|c5] [--no-target] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -19,7 +19,11 @@ blocks all-reduced).  The same JSON line carries `target_config`: BASELINE.json 
 N=10M, K=50, G=100k) -- whole on one GPU at N = 1, and at N > 1 the SAME 10M problem cut into
 group-aligned shards by distributed.partition_groups (strong scaling), timed next to a 1-GPU run of
 the whole problem on rank 0 in the same process so that the speed-up is measured on one box.
-Prints ONE JSON line.
+Prints ONE JSON line.  --steps is the number of timed steps behind `value` / `ms_per_step` (for c5: timed
+launches per family).  The other timed loops -- e2e, the per-kernel durations, target_config -- run bounded
+counts of their own, reported in their sections, so that C4's 150 ms steps keep a run short.  With
+--dump-outputs DIR the results of the last timed step are also written as .npy files: the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -50,6 +54,7 @@ WORKLOADS = {
 METRIC = "GLMM obs/sec for ELBO+grad+sparse Hessian"
 UNIT = "obs/s"
 CPU_SAMPLE = dict(N=500_000, G=5_000)   # bounded sample of the workload for the CPU arm
+DUMP_BYTES = 64 * 10 ** 6               # --dump-outputs: all .npy files together
 
 
 # ------------------------------------------------------------------------------------------
@@ -271,12 +276,40 @@ def make_model(ctx, wl, mode):
     return model, model.local, Nl
 
 
-def time_workload(ctx, wl, mode, steps, warmup, sampler=None, kernel_steps=30):
+def last_step_outputs(torch, model, csr):
+    """What a caller of the timed step receives -- KL, gradient and sparse Hessian of the last evaluation --
+    as float64 host arrays.  The Hessian goes out as COO triplets (row, col, value) in CSR order.  When all
+    of them would take the total past DUMP_BYTES (C3, C4), entry positions drawn with a fixed seed stand in
+    for them: two builds that produce the same pattern write the same positions."""
+    kl = model.kl_tensor().reshape(1).cpu().numpy()
+    grad = model.grad_tensor().cpu().numpy()
+    crow, val = csr.crow_indices.long(), csr.values
+    nnz = val.numel()
+    room = (DUMP_BYTES - 8 * (kl.size + grad.size) - 4096) // 24     # 4096: the five .npy headers
+    if nnz <= room:
+        pos = torch.arange(nnz, device=val.device)
+    else:
+        pos = torch.from_numpy(np.unique(np.random.default_rng(0).integers(0, nnz, size=room))).to(val.device)
+    row = torch.searchsorted(crow, pos, right=True) - 1
+    return {"kl": kl, "grad": grad, "hessian_row": row.double().cpu().numpy(),
+            "hessian_col": csr.col_indices[pos].double().cpu().numpy(), "hessian_value": val[pos].cpu().numpy()}
+
+
+def write_outputs(path, outputs):
+    os.makedirs(path, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), arr)
+    print("outputs of the last timed step: %s (%s)" % (
+        path, ", ".join("%s %d" % (n, a.size) for n, a in outputs.items())), file=sys.stderr)
+
+
+def time_workload(ctx, wl, mode, steps, warmup, sampler=None, kernel_steps=30, dump=False):
     """Device-timed steps of one workload.  Returns a dict (identical on every rank for the reduced
     entries).  Timing discipline: garbage collector off and every rank synchronised BEFORE the last
     barrier; one untimed step after the barrier (the first collective after a barrier pays a
     re-synchronisation); then straight into the timed loop.  L2 flushed (256 MiB write) before every
-    timed step, outside the events."""
+    timed step, outside the events.  With ``dump`` the result carries ``outputs``: the last timed
+    step's results on the host (last_step_outputs)."""
     torch, dist, lib, nat = ctx.torch, ctx.dist, ctx.lib, ctx.nat
     sharded = mode in ("weak", "strong")
     model, local, N_local = make_model(ctx, wl, mode)
@@ -327,6 +360,7 @@ def time_workload(ctx, wl, mode, steps, warmup, sampler=None, kernel_steps=30):
         step_ms.append(e0.elapsed_time(e1))
     torch.cuda.synchronize()
     gc.enable()
+    outputs = last_step_outputs(torch, local, csr) if dump else None
     launches = (lib.lrvb_launch_count() - launches0) // max(1, steps)
     wait = peer.stats() if peer is not None else None
     if peer is not None:
@@ -347,7 +381,7 @@ def time_workload(ctx, wl, mode, steps, warmup, sampler=None, kernel_steps=30):
                per_rank_ms={"mean": [round(v, 5) for v in per_rank[:, 0]],
                             "median": [round(v, 5) for v in per_rank[:, 1]],
                             "max": [round(v, 5) for v in per_rank[:, 3]]},
-               model=model, local=local, x_dev=x_dev, mode=mode)
+               model=model, local=local, x_dev=x_dev, mode=mode, outputs=outputs)
     if sharded:
         res["collective_wait_us"] = {
             "mean_per_call_max_over_ranks": float(per_rank[:, 5].max()),
@@ -734,7 +768,9 @@ def run_ours(args, wl):
 
     if args.workload == "c5":
         import bench_ef
-        line = bench_ef.run_ours(ctx, args)
+        line, outputs = bench_ef.run_ours(ctx, args, dump=args.dump_outputs is not None and rank == 0)
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         if rank == 0:
             os.write(result_fd, (json.dumps(line) + "\n").encode())
         if world > 1:
@@ -745,11 +781,12 @@ def run_ours(args, wl):
         return
 
     K, G, Q = wl["K"], wl["G"], wl["Q"]
-    if wl["N"] * K >= 10 ** 9:                 # C3 / C4 as the headline workload: steps of 6 - 150 ms
-        args.steps = min(args.steps, 20 if K <= 64 else 5)
     mode = "single" if world == 1 else "weak"
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    res = time_workload(ctx, wl, mode, args.steps, args.warmup, sampler=sampler)
+    res = time_workload(ctx, wl, mode, args.steps, args.warmup, sampler=sampler,
+                        dump=args.dump_outputs is not None and rank == 0)
+    if res["outputs"] is not None:
+        write_outputs(args.dump_outputs, res.pop("outputs"))
     peak_tf = measure_dgemm_tflops(torch) if rank == 0 else 1.0
     cov = cov_entry(ctx, res["model"], K, G, peak_tf, ncov=20 if K <= 64 else 3)
     if args.workload == "c4" and world == 1:
@@ -865,13 +902,23 @@ def ctx_single(ctx):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of the headline measurement (c5: launches per family); the e2e, "
+                         "kernel-time and target_config loops keep their own bounded counts, reported beside them")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS) + ["c5"])
     ap.add_argument("--no-target", action="store_true",
                     help="skip the target_config (C3) section of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy, float64, 64 MB at most: "
+                         "KL, gradient and Hessian (COO; a seeded sample of its entries where they do not fit), "
+                         "or for c5 each family's terms on a seeded sample of the factors; rank 0's at N > 1")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3   # timing rules: W >= 3
     wl = WORKLOADS.get(args.workload)

@@ -84,7 +84,17 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
-def run_ours(ctx, args):
+def sample_factors(n_values):
+    """Sorted factor indices drawn with a fixed seed: the factors whose results --dump-outputs writes when
+    ``n_values`` float64 values per factor would take all 1M factors past bench.DUMP_BYTES."""
+    import bench
+    n = min(M, (bench.DUMP_BYTES - 4096) // (8 * n_values))      # 4096: the .npy headers
+    return np.sort(np.random.default_rng(0).choice(M, size=n, replace=False))
+
+
+def run_ours(ctx, args, dump=False):
+    """Returns (JSON line, outputs): with ``dump``, outputs holds the results of the last timed launch of
+    each family of the step, on the host for the factors of sample_factors; otherwise None."""
     torch, nat, lib, vb = ctx.torch, ctx.nat, ctx.lib, ctx.vb
     ef = vb.ExponentialFamilies
     dev = ctx.device
@@ -97,37 +107,44 @@ def run_ours(ctx, args):
     sp = ctypes.c_void_p(st.cuda_stream)
     P = nat.ptr
     cases = [
-        # name, launch, algorithmic bytes per factor (8 x (inputs + outputs))
-        ("gamma entropy + E log (fused)", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, P(out1), P(out2), sp), 32),
-        ("gamma entropy", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, P(out1), None, sp), 24),
-        ("E log gamma", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, None, P(out2), sp), 24),
-        ("dirichlet (d=5) entropy + E log (fused)", lambda: lib.lrvb_ef_dirichlet_terms(P(inp["alpha"]), 5, M, P(out1), P(outd), sp), 88),
-        ("dirichlet (d=5) entropy", lambda: lib.lrvb_ef_dirichlet_terms(P(inp["alpha"]), 5, M, P(out1), None, sp), 48),
-        ("beta entropy", lambda: lib.lrvb_ef_beta_entropy(P(inp["tau"]), M, P(out1), sp), 24),
-        ("uvn entropy", lambda: lib.lrvb_ef_uvn_entropy(P(inp["info"]), M, P(out1), sp), 16),
+        # name, launch, algorithmic bytes per factor (8 x (inputs + outputs)), results kept by --dump-outputs
+        ("gamma entropy + E log (fused)", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, P(out1), P(out2), sp), 32,
+         (("gamma_entropy", out1), ("gamma_e_log", out2))),
+        ("gamma entropy", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, P(out1), None, sp), 24, ()),
+        ("E log gamma", lambda: lib.lrvb_ef_gamma_terms(P(inp["shape"]), P(inp["rate"]), M, None, P(out2), sp), 24, ()),
+        ("dirichlet (d=5) entropy + E log (fused)", lambda: lib.lrvb_ef_dirichlet_terms(P(inp["alpha"]), 5, M, P(out1), P(outd), sp), 88,
+         (("dirichlet_entropy", out1), ("dirichlet_e_log", outd))),
+        ("dirichlet (d=5) entropy", lambda: lib.lrvb_ef_dirichlet_terms(P(inp["alpha"]), 5, M, P(out1), None, sp), 48, ()),
+        ("beta entropy", lambda: lib.lrvb_ef_beta_entropy(P(inp["tau"]), M, P(out1), sp), 24, (("beta_entropy", out1),)),
+        ("uvn entropy", lambda: lib.lrvb_ef_uvn_entropy(P(inp["info"]), M, P(out1), sp), 16, (("uvn_entropy", out1),)),
     ]
     rows = []
     total_ms = 0.0
+    outputs, pick = None, None
+    if dump:
+        outputs = {}
+        pick = torch.from_numpy(sample_factors(10)).to(dev)   # 10 values per factor: 2 gamma, 6 dirichlet, beta, uvn
     launches0 = lib.lrvb_launch_count()
-    reps = max(20, args.steps)
-    for name, fn, bpf in cases:
+    for name, fn, bpf, keep in cases:
         with torch.cuda.stream(st):
-            for _ in range(3):
+            for _ in range(args.warmup):
                 nat.check(fn())
             st.synchronize()
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph, stream=st):
-                for _ in range(10):
+                for _ in range(args.steps):
                     nat.check(fn())
-            graph.replay()
+            graph.replay()                  # untimed: the first replay uploads the graph
             st.synchronize()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(st)
-            for _ in range(reps // 10 + 1):
-                graph.replay()
+            graph.replay()
             e1.record(st)
             e1.synchronize()
-            ms = e0.elapsed_time(e1) / (10 * (reps // 10 + 1))
+            ms = e0.elapsed_time(e1) / args.steps
+        if outputs is not None:
+            for oname, buf in keep:
+                outputs[oname] = buf[..., pick].cpu().numpy()
         gbs = M * bpf / (ms * 1e-3) / 1e9
         rows.append({"family": name, "us": 1e3 * ms, "factors_per_s": M / (ms * 1e-3), "bytes_per_factor": bpf,
                      "achieved_gbs": gbs, "frac_of_hbm": gbs / hbm})
@@ -135,16 +152,16 @@ def run_ours(ctx, args):
             total_ms += ms
     launches = lib.lrvb_launch_count() - launches0
     # Wishart (k = 2) through the Python function (its C entry point synchronises for the PD status)
-    for _ in range(3):
+    for _ in range(args.warmup):
         ef.wishart_entropy(inp["df"], inp["v"])
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(10):
+    for _ in range(args.steps):
         ef.wishart_entropy(inp["df"], inp["v"])
     e1.record()
     e1.synchronize()
-    wms = e0.elapsed_time(e1) / 10
+    wms = e0.elapsed_time(e1) / args.steps
     rows.append({"family": "wishart (k=2) entropy, Python call incl. status sync", "us": 1e3 * wms,
                  "factors_per_s": M / (wms * 1e-3), "bytes_per_factor": 48,
                  "achieved_gbs": M * 48 / (wms * 1e-3) / 1e9, "frac_of_hbm": M * 48 / (wms * 1e-3) / 1e9 / hbm})
@@ -180,14 +197,14 @@ def run_ours(ctx, args):
         ts.append(time.perf_counter() - t)
     dom = max(rows[:7], key=lambda r: r["us"])
     line = {
-        "metric": METRIC, "value": M / (total_ms * 1e-3), "unit": UNIT, "n_gpus": ctx.world, "steps": reps,
-        "warmup": 3, "ms_per_step": total_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "metric": METRIC, "value": M / (total_ms * 1e-3), "unit": UNIT, "n_gpus": ctx.world, "steps": args.steps,
+        "warmup": args.warmup, "ms_per_step": total_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f64", "data": "synthetic",
         "config": {"workload": "mean-field EF entropy / E-log terms over 1M local factors (BASELINE configs[4]): "
                                "a step = Gamma (entropy + E log) + Dirichlet d=5 (entropy + E log) + Beta entropy "
                                "+ UVN entropy, one launch per family",
-                   "timing": "CUDA-graph replay of the C-ABI launches (10 per graph), CUDA events on the launching "
-                             "stream.  A family's inputs (8 - 40 MB) are smaller than the 126 MB L2 and are "
+                   "timing": "per family, --steps C-ABI launches captured in one CUDA graph and replayed once, CUDA "
+                             "events on the launching stream.  A family's inputs (8 - 40 MB) are smaller than the 126 MB L2 and are "
                              "re-read by consecutive launches, so they may be L2-resident: frac_of_hbm measures "
                              "the kernels' rate against the HBM roofline figure, not DRAM efficiency (these "
                              "kernels are bound by fp64 special-function throughput)",
@@ -206,4 +223,4 @@ def run_ours(ctx, args):
                          "sample": "%d of the 1M factors, every family once, numpy / scipy.special; median of 3" % (M // 4)},
         "clocks": None,
     }
-    return line
+    return line, outputs

@@ -14,6 +14,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_cabi_library_loads_and_exports_every_declared_symbol(vb):
+    import subprocess
+    import sys
     from lrvb_b200 import _native as nat
     lib = nat.load()
     header = open(os.path.join(ROOT, "include", "lrvb_b200.h")).read()
@@ -23,7 +25,15 @@ def test_cabi_library_loads_and_exports_every_declared_symbol(vb):
     for name in declared:
         assert hasattr(lib, name), name
     assert lib.lrvb_version() >= 100
-    assert lib.lrvb_launch_count() == 0   # nothing launched: no compute without a GPU
+    # nothing launched: the launch counter is per process and GPU tests of this session may already have
+    # launched kernels here, so the library is loaded and queried again in a fresh interpreter
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "from lrvb_b200 import _native as nat\n"
+            "lib = nat.load(); lib.lrvb_version(); print(lib.lrvb_launch_count())" % ROOT)
+    flags = ["-s"] if sys.flags.no_user_site else []
+    r = subprocess.run([sys.executable] + flags + ["-c", code], capture_output=True, text=True, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.split()[-1] == "0", r.stdout
 
 
 def test_no_cpu_fallback(vb):
