@@ -223,6 +223,34 @@ int lrvb_glmm_solve_finish(lrvb_glmm* h, const double* Sinv_dev, const double* r
  *   L_g^{-1} + L_g^{-1} B_g S^{-1} B_g^T L_g^{-1}. */
 int lrvb_glmm_local_cov(lrvb_glmm* h, const double* Sinv_dev, double* cov_dev, void* stream);
 
+/* ---- prediction on new rows ---------------------------------------------------------------
+ * At the free point free_dev (D,) (free coordinates; no evaluation over the training rows is needed), for M
+ * new rows X_dev (M,K) row-major fp64 (16-byte aligned,
+ * K must equal the handle's K) with group ids g_dev (M,) int32 in [-1, G) (-1 = population level: mu in
+ * place of u_g).  order_dev (M,) int64 or NULL: the order in which the rows are visited, a permutation of
+ * [0, M) (e.g. a stable sort by group, so that rows of one group read its blocks from cache); every row is
+ * read from and written to its own place, so the result does not depend on it.  Output:
+ *   out_dev (4, M) row-major = [eta_mean, eta_var_mfvb, prob, prob_var_mfvb]
+ * with eta = u_g + x.beta under q and prob = E_q[sigma(eta)] by the model's Gauss-Hermite rule.
+ * A row whose group id is outside [-1, G) gets NaN.  LRVB_EINVAL for a K other than the handle's, M < 0,
+ * NULL pointers or an X that is not 16-byte aligned. */
+int lrvb_glmm_predict(lrvb_glmm* h, const double* free_dev, const double* X_dev, int32_t K, const int32_t* g_dev, const int64_t* order_dev,
+                      int64_t M, double* out_dev, void* stream);
+/* The block of H^-1 between beta and every group's (u.mean_g, u.info_g), cross_dev (G, 2, 2K):
+ * cross[g][r][j] = (H^-1)[4 + j, (u.mean_g, u.info_g)_r] = -(S^-1 B_g^T L_g^-1)[4 + j, r], given
+ * Sinv_dev = S^-1 (lrvb_glmm_schur + lrvb_spd_inverse).  Once per optimum.  Needs a cached Hessian in
+ * free coordinates (LRVB_ESTATE otherwise). */
+int lrvb_glmm_predict_cross(lrvb_glmm* h, const double* Sinv_dev, double* cross_dev, void* stream);
+/* lrvb_glmm_predict plus the linear-response variances j H^-1 j^T of prob and eta (j = their gradient
+ * with respect to the free parameters) from the arrowhead pieces Sinv_dev (Dg,Dg), cross_dev (above) and
+ * localcov_dev (G,3) (lrvb_glmm_local_cov): out_dev (6, M) = [eta_mean, eta_var_mfvb, prob,
+ * prob_var_mfvb, prob_var_lr, eta_var_lr].  The quadratic forms run on the FP64 tensor cores.  Needs a
+ * cached Hessian in free coordinates (LRVB_ESTATE otherwise); allocates a (3K x K) scratch in the
+ * handle on first use. */
+int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
+                         const double* X_dev, int32_t K, const int32_t* g_dev, const int64_t* order_dev, int64_t M,
+                         double* out_dev, void* stream);
+
 /* ---- batched exponential-family terms (ExponentialFamilies.py) --------------------------
  * All pointers dev; M = number of factors. */
 /* :33-35 gamma_entropy per factor, out (M,). */

@@ -16,12 +16,13 @@ accepts it in place of ``fun``.
 import ctypes
 import os
 import weakref
+from collections import namedtuple
 from dataclasses import dataclass
 
 import numpy as np
 
 from . import _native as nat
-from ._tensors import PointKey, is_torch, to_device
+from ._tensors import PointKey, is_torch, like_input, to_device
 from .GammaParams import GammaParam
 from .NormalParams import UVNParam, UVNParamVector
 from .ParameterDictionary import ModelParamsDict
@@ -37,6 +38,14 @@ class GLMMPrior:
     beta_info: float = 0.01
     tau_shape: float = 3.0
     tau_rate: float = 3.0
+
+
+Prediction = namedtuple("Prediction", ["eta_mean", "eta_var_mfvb", "prob", "prob_var_mfvb", "prob_var_lr",
+                                       "eta_var_lr"])
+Prediction.__doc__ = """Per-row predictions for new observations (``LogisticGLMM.predict``,
+``LinearResponseCovariances.get_prediction_variances``): the linear predictor eta = u_g + x.beta and
+prob = E_q[sigma(eta)] with their mean-field variances and, from the linear-response pass, their LRVB
+variances (None where not computed)."""
 
 
 class _DevView(object):
@@ -726,6 +735,127 @@ class LogisticGLMM(object):
         nat.check(self._lib.lrvb_glmm_local_cov(self._h, nat.ptr(Sinv), nat.ptr(cov),
                                                 nat.stream_ptr()))
         return cov
+
+    # ---- prediction on new rows (csrc/predict.cu) --------------------------------------------
+    def _check_prediction_rows(self, X_new, groups_new):
+        """Checks new rows on the host -> (g (M,) int64, numpy or torch as given, M)."""
+        if len(X_new.shape) != 2 or int(X_new.shape[1]) != self.K:
+            raise ValueError("X_new must be (M, K) with K = {}, got shape {}".format(self.K, tuple(X_new.shape)))
+        M = int(X_new.shape[0])
+        if is_torch(groups_new):
+            import torch
+            g = groups_new.reshape(-1)
+            if g.dtype.is_floating_point or g.dtype.is_complex or g.dtype == torch.bool:
+                raise ValueError("group ids must be integers, got dtype {}".format(g.dtype))
+            g = g.to(torch.int64)
+            lo, hi = (int(g.min()), int(g.max())) if g.numel() else (0, 0)
+        else:
+            g = np.asarray(groups_new).reshape(-1)
+            if not np.issubdtype(g.dtype, np.integer):
+                if not np.issubdtype(g.dtype, np.floating) or not np.all(np.floor(g) == g):
+                    raise ValueError("group ids must be integers")
+            g = g.astype(np.int64)
+            lo, hi = (int(g.min()), int(g.max())) if g.size else (0, 0)
+        if int(np.prod(g.shape)) != M:
+            raise ValueError("Wrong size for groups_new.  Expected {}, got {}".format(M, int(np.prod(g.shape))))
+        if lo < -1 or hi >= self.G:
+            raise ValueError("group ids must lie in [-1, {}) (-1: population level), got [{}, {}]".format(
+                self.G, lo, hi))
+        return g, M
+
+    def _prediction_rows(self, X_new, groups_new):
+        """Checks new rows before any kernel runs -> (X (M,K) fp64 CUDA, g (M,) int32 CUDA, M)."""
+        torch = nat.require_cuda()
+        g, M = self._check_prediction_rows(X_new, groups_new)
+        X = to_device(X_new)
+        if X.numel() and X.data_ptr() % 16:
+            X = X.clone()
+        return X, to_device(g, torch.int32), M
+
+    def _prediction_result(self, out, nfields, like):
+        f = [like_input(out[i], *like) for i in range(nfields)]
+        return Prediction(*(f + [None] * (6 - nfields)))
+
+    def predict(self, free, X_new, groups_new):
+        """Predictions for new rows ``X_new`` (M, K) in groups ``groups_new`` (M,), integer ids in [-1, G)
+        (-1: population level, the random effect at its mean mu -- lme4's ``re.form = NA``), at the free
+        point ``free`` (read directly: no pass over the training rows): a ``Prediction`` with eta_mean, eta_var_mfvb, prob, prob_var_mfvb in the caller's row
+        order (numpy for numpy input, CUDA tensors for CUDA tensor input); the LR fields are None."""
+        torch = nat.require_cuda()
+        X, g, M = self._prediction_rows(X_new, groups_new)
+        f = to_device(free).reshape(-1)
+        if f.numel() != self.D:
+            raise ValueError("Wrong size for parameter {}.  Expected {}, got {}".format(
+                self.glmm_par.name, self.D, f.numel()))
+        out = torch.empty(4, M, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_predict(self._h, nat.ptr(f), nat.ptr(X), self.K, nat.ptr(g), None, M, nat.ptr(out),
+                                              nat.stream_ptr()))
+        return self._prediction_result(out, 4, (X_new, groups_new))
+
+    def prediction_cross(self, Sinv):
+        """(G, 2, 2K) block of H^-1 between beta and every group's (u.mean_g, u.info_g), at the cached Hessian."""
+        torch = nat.require_cuda()
+        cross = torch.empty(self.G, 2, 2 * self.K, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_predict_cross(self._h, nat.ptr(Sinv), nat.ptr(cross), nat.stream_ptr()))
+        return cross
+
+    def predict_lr(self, Sinv, cross, local_cov, X_new, groups_new):
+        """``predict`` plus the LRVB variances at the cached Hessian from its arrowhead pieces: S^-1
+        (``global_covariance``), ``prediction_cross`` and ``local_cov``.  The rows are visited group by
+        group (a stable sort of the ids, no copy of X) so that each group's blocks are read from cache."""
+        torch = nat.require_cuda()
+        X, g, M = self._prediction_rows(X_new, groups_new)
+        order = None
+        if M > 1:
+            _, perm = group_sort(g)
+            order = perm.to(torch.int64).contiguous()
+        out = torch.empty(6, M, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_predict_lr(self._h, nat.ptr(Sinv), nat.ptr(cross), nat.ptr(local_cov),
+                                                 nat.ptr(X), self.K, nat.ptr(g), nat.ptr(order), M, nat.ptr(out),
+                                                 nat.stream_ptr()))
+        return self._prediction_result(out, 6, (X_new, groups_new))
+
+    def prediction_jacobian(self, free, X_new, groups_new, quantity="prob"):
+        """d prob / d free (or d eta / d free) of new rows as scipy CSR (M, D): a x on beta.mean, b x~ on
+        beta.info (x~_k = -x_k^2 (i_k - lb) / i_k^2), a on u.mean_g and b d_g on u.info_g (d_g = -(i_g - lb) /
+        i_g^2; mu's columns for g = -1), with a = dp/dz_m, b = dp/dz_v (a = 1, b = 0 for eta).  Assembled on
+        the host (host inputs never visit the device) with 2K + 2 entries per row: meant for small M, e.g. covariances BETWEEN rows through
+        ``LinearResponseCovariances.get_lr_covariance_factors``."""
+        import scipy.sparse
+        if quantity not in ("prob", "eta"):
+            raise ValueError("quantity must be 'prob' or 'eta'")
+        g, M = self._check_prediction_rows(X_new, groups_new)
+        Xh = X_new.detach().cpu().numpy() if is_torch(X_new) else X_new
+        Xh = np.ascontiguousarray(Xh, dtype=np.float64)
+        gh = g.cpu().numpy() if is_torch(g) else g
+        f = free.detach().cpu().numpy() if is_torch(free) else np.asarray(free, dtype=np.float64)
+        f = f.reshape(-1)
+        if f.size != self.D:
+            raise ValueError("Wrong size for parameter {}.  Expected {}, got {}".format(
+                self.glmm_par.name, self.D, f.size))
+        K, G, Dg, lb = self.K, self.G, self.Dg, self.lower_bounds
+        pop = gh < 0
+        gs = np.where(pop, 0, gh)
+        beta_i = np.exp(f[4 + K:Dg]) + lb["beta_info"]
+        u_m, u_i = f[Dg:Dg + G], np.exp(f[Dg + G:]) + lb["u_info"]
+        mu_i = np.exp(f[1]) + lb["mu_info"]
+        info = np.where(pop, mu_i, u_i[gs] if G else 1.0)
+        d = -(info - np.where(pop, lb["mu_info"], lb["u_info"])) / (info * info)
+        if quantity == "prob":
+            z_m = np.where(pop, f[0], u_m[gs] if G else 0.0) + Xh @ f[4:4 + K]
+            z_s = np.sqrt(1.0 / info + (Xh * Xh) @ (1.0 / beta_i))
+            c = np.sqrt(2.0) * self.gh_x
+            sg = 1.0 / (1.0 + np.exp(-(z_m[:, None] + z_s[:, None] * c[None, :])))
+            dsg = (self.gh_w / np.sqrt(np.pi)) * sg * (1.0 - sg)
+            a, b = dsg.sum(axis=1), (dsg * c).sum(axis=1) / (2.0 * z_s)
+        else:
+            a, b = np.ones(M), np.zeros(M)
+        xt = -(Xh * Xh) * ((beta_i - lb["beta_info"]) / (beta_i * beta_i))[None, :]
+        cols = np.concatenate([np.tile(np.arange(4, Dg), (M, 1)), np.where(pop, 0, Dg + gh)[:, None],
+                               np.where(pop, 1, Dg + G + gh)[:, None]], axis=1)
+        vals = np.concatenate([a[:, None] * Xh, b[:, None] * xt, a[:, None], (b * d)[:, None]], axis=1)
+        rows = np.repeat(np.arange(M), 2 * K + 2)
+        return scipy.sparse.csr_matrix((vals.reshape(-1), (rows, cols.reshape(-1))), shape=(M, self.D))
 
     # ---- moments (for LinearResponseCovariances) ------------------------------------------------
     def moment_names(self):

@@ -46,6 +46,7 @@ class LinearResponseCovariances(object):
                     gmax, grad_tol))
         self.model.evaluate(opt_par_value, 2, "free")
         self._sinv = None
+        self._pred_blocks = None      # (cross, local covariances) of get_prediction_variances
 
     def _ensure_point(self):
         self.model.evaluate(self._opt0, 2, "free")
@@ -176,6 +177,26 @@ class LinearResponseCovariances(object):
              (np.concatenate([gi, gi, gi + G, gi + G]), np.concatenate([gi, gi + G, gi, gi + G]))), (2 * G, 2 * G))
         local_term = (jl1 @ Ls @ jl2.T).tocsr()
         return ArrowheadCovariance(w1, self._sinv, w2, local_term, symmetric=same)
+
+    def get_prediction_variances(self, X_new, groups_new):
+        """Predictions for new rows with their LRVB variances at the optimum: a ``GLMM.Prediction`` with
+        eta_mean, eta_var_mfvb, prob, prob_var_mfvb, prob_var_lr, eta_var_lr, where the LR variance of a
+        row is j H^{-1} j^T for j = its gradient with respect to the free parameters
+        (``model.prediction_jacobian``).  Always from the direct arrowhead pieces (S^{-1}, the beta x local
+        block of H^{-1} and the local covariances), whatever ``method`` is; one device pass over the rows
+        (csrc/predict.cu), nothing of size (M, D) or (M, Dg) is formed.  Covariances BETWEEN rows:
+        ``get_lr_covariance_factors(model.prediction_jacobian(...))``."""
+        model = self.model
+        if getattr(model, "local", None) is not None:
+            raise NotImplementedError("prediction of a sharded model: build a single-GPU LogisticGLMM of the "
+                                      "job and use its LinearResponseCovariances")
+        self._ensure_point()
+        if self._sinv is None:
+            self._sinv = model.global_covariance()
+        if self._pred_blocks is None:
+            self._pred_blocks = (model.prediction_cross(self._sinv), model.local_cov(self._sinv))
+        cross, lcov = self._pred_blocks
+        return model.predict_lr(self._sinv, cross, lcov, X_new, groups_new)
 
     MAX_DENSE = 1 << 26
 

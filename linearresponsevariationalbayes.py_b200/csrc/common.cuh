@@ -296,6 +296,7 @@ struct lrvb_glmm {
   double* T = nullptr;        // (G,2,Dg) L^-1 B for the Schur path
   int schur_grid = 0;
   double* schurpart = nullptr;
+  double* pred_B = nullptr;   // (3 Kp8, Kp4) scaled beta block of S^-1 for lrvb_glmm_predict_lr (predict.cu)
 };
 
 namespace lrvb {

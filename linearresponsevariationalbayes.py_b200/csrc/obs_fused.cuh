@@ -64,6 +64,7 @@ inline size_t obs_fused_smem(int K, int Q, int warps, int slots = kOfStages) {
 
 struct GHSumsF {
   double A, Am, As, Amm, Ams, Ass;
+  double App;   // sum what sigma^2 (ORDER >= 3: prediction, csrc/predict.cu)
 };
 
 // ---- branch-free fp64 kernels of the quadrature node ----------------------------------------
@@ -245,6 +246,7 @@ __device__ __forceinline__ void gh_nodes_f(double zm, double zs, const double* _
         s.Ams += wdc;
         s.Ass = fma(wdc, c[u], s.Ass);
       }
+      if (ORDER >= 3) s.App = fma(wsg, sg, s.App);
     }
   }
 }

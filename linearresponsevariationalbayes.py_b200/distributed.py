@@ -480,6 +480,12 @@ class ShardedLogisticGLMM(object):
         """LRVB covariances of this rank's groups' (u.mean, u.info), (G_local, 3)."""
         return self.local.local_cov(Sinv)
 
+    def _no_prediction(self, *args, **kwargs):
+        raise NotImplementedError("prediction of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                  "and use LogisticGLMM.predict / LinearResponseCovariances.get_prediction_variances")
+
+    predict = prediction_jacobian = _no_prediction
+
     def moment_jacobian(self, free):
         import scipy.sparse
         free = np.asarray(free, dtype=np.float64).reshape(-1)
