@@ -250,6 +250,19 @@ int lrvb_glmm_predict_cross(lrvb_glmm* h, const double* Sinv_dev, double* cross_
 int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
                          const double* X_dev, int32_t K, const int32_t* g_dev, const int64_t* order_dev, int64_t M,
                          double* out_dev, void* stream);
+/* Approximate leave-one-out cross-validation of the handle's own N training rows by the infinitesimal jackknife,
+ * at the cached Hessian (an order-2 evaluation in free coordinates, normally at the optimum; LRVB_ESTATE
+ * otherwise), from the same arrowhead pieces as lrvb_glmm_predict_lr.  For row n, with z = u_g + x.beta under q,
+ * Q_n = [j_m; j_v] H^-1 [j_m; j_v]^T (j_m, j_v = d E[z] / d free, d Var[z] / d free) and W_m, W_v = rows 0, 1 of
+ * lrvb_glmm_obs_weights (w_n dl_n/dz_m, w_n dl_n/dz_v of the same evaluation), dropping the row shifts its
+ * moments by (dz_m, dz_v) = -Q_n (W_m, W_v).  Output, in the handle's (group-sorted) row order:
+ *   out_dev (4, N) row-major = [lpd, lpd_loo, eta_mean_loo, eta_var_loo]
+ * with lpd = log E_q[p(y_n | z)] by the model's Gauss-Hermite rule (y = 0 as log E[sigma(-z)]), lpd_loo the
+ * same at the shifted moments, eta_*_loo = the shifted moments.  A row whose shifted variance is <= 0 gets NaN
+ * in lpd_loo and eta_var_loo.  y must be 0 or 1 (any y != 0 counts as 1).  No atomics: repeated calls are
+ * bitwise equal.  LRVB_EINVAL for NULL pointers; uses the scratch of lrvb_glmm_predict_lr. */
+int lrvb_glmm_loo(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
+                  double* out_dev, void* stream);
 
 /* ---- batched exponential-family terms (ExponentialFamilies.py) --------------------------
  * All pointers dev; M = number of factors. */

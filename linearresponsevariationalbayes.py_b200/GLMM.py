@@ -47,6 +47,15 @@ Prediction.__doc__ = """Per-row predictions for new observations (``LogisticGLMM
 prob = E_q[sigma(eta)] with their mean-field variances and, from the linear-response pass, their LRVB
 variances (None where not computed)."""
 
+ApproximateLOO = namedtuple("ApproximateLOO", ["lpd", "lpd_loo", "eta_mean_loo", "eta_var_loo", "elpd_loo",
+                                               "elpd_loo_se", "p_loo", "n_invalid"])
+ApproximateLOO.__doc__ = """Approximate leave-one-out cross-validation of the training rows by the infinitesimal
+jackknife (``LogisticGLMM.approximate_loo``, ``LinearResponseCovariances.get_approximate_loo``).  Per row (N,), in
+the caller's row order: lpd = log E_q[p(y_n | eta)], lpd_loo = the same with q moved to the IJ estimate of the fit
+without row n, and the moments eta_mean_loo, eta_var_loo of eta = u_g + x.beta there (NaN in lpd_loo and
+eta_var_loo where the shifted variance is <= 0).  Scalars: elpd_loo = sum lpd_loo, p_loo = sum lpd - elpd_loo,
+elpd_loo_se = sqrt(N) std(lpd_loo, ddof=1) (NaN when n_invalid > 0), n_invalid = rows with NaN."""
+
 
 class _DevView(object):
     """Zero-copy torch view of library-owned device memory (__cuda_array_interface__)."""
@@ -814,6 +823,36 @@ class LogisticGLMM(object):
                                                  nat.ptr(X), self.K, nat.ptr(g), nat.ptr(order), M, nat.ptr(out),
                                                  nat.stream_ptr()))
         return self._prediction_result(out, 6, (X_new, groups_new))
+
+    def _check_binary_y(self):
+        """Raises ValueError unless every training y is 0 or 1 (checked once: y is fixed with the model)."""
+        if not getattr(self, "_y_binary", False):
+            if self.N and bool(((self.y != 0) & (self.y != 1)).any()):
+                raise ValueError("approximate LOO needs a binary training y (0 or 1): a logistic GLMM has no "
+                                 "predictive density for other values")
+            self._y_binary = True
+
+    def approximate_loo(self, Sinv, cross, local_cov):
+        """Approximate leave-one-out cross-validation of the training rows by the infinitesimal jackknife at the
+        cached Hessian (normally the optimum), from the arrowhead pieces of ``predict_lr``: S^-1
+        (``global_covariance``), ``prediction_cross`` and ``local_cov``.  Dropping row n is the weight change
+        w_n -> 0; its first-order effect on the row's moments is (dz_m, dz_v) = -Q_n (w_n l_m, w_n l_v) with
+        Q_n = [j_m; j_v] H^-1 [j_m; j_v]^T, one device pass over the rows (csrc/predict.cu).  Returns an
+        ``ApproximateLOO`` with CUDA tensors in the caller's row order and Python scalars."""
+        torch = nat.require_cuda()
+        self._check_binary_y()
+        out = torch.empty(4, self.N, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_loo(self._h, nat.ptr(Sinv), nat.ptr(cross), nat.ptr(local_cov), nat.ptr(out),
+                                          nat.stream_ptr()))
+        if self.perm is not None:
+            res = torch.empty_like(out)
+            res.index_copy_(1, to_device(self.perm, torch.int64), out)
+            out = res
+        lpd, lpd_loo = out[0], out[1]
+        n_invalid = int(torch.isnan(out[3]).sum())
+        elpd = float(lpd_loo.sum())
+        se = float(lpd_loo.std(correction=1)) * np.sqrt(self.N) if self.N > 1 else float("nan")
+        return ApproximateLOO(lpd, lpd_loo, out[2], out[3], elpd, se, float(lpd.sum()) - elpd, n_invalid)
 
     def prediction_jacobian(self, free, X_new, groups_new, quantity="prob"):
         """d prob / d free (or d eta / d free) of new rows as scipy CSR (M, D): a x on beta.mean, b x~ on

@@ -198,6 +198,31 @@ class LinearResponseCovariances(object):
         cross, lcov = self._pred_blocks
         return model.predict_lr(self._sinv, cross, lcov, X_new, groups_new)
 
+    def get_approximate_loo(self):
+        """Approximate leave-one-out cross-validation of the training rows at the optimum by the infinitesimal
+        jackknife (Giordano et al., "A Swiss Army Infinitesimal Jackknife"): a ``GLMM.ApproximateLOO`` with the
+        pointwise lpd, lpd_loo, eta_mean_loo, eta_var_loo (caller's row order; numpy for a numpy optimum, CUDA
+        tensors for a CUDA one) and elpd_loo, elpd_loo_se, p_loo, n_invalid.  The same as dropping each row's
+        weight in ``WeightSensitivityLinearApproximation`` and pushing the shift of the optimum through the row's
+        moments, for all N rows in one device pass instead of N solves.  Always from the direct arrowhead
+        pieces, whatever ``method`` is (cached with ``get_prediction_variances``)."""
+        model = self.model
+        if getattr(model, "local", None) is not None:
+            raise NotImplementedError("approximate LOO of a sharded model: build a single-GPU LogisticGLMM of the "
+                                      "job and use its LinearResponseCovariances")
+        model._check_binary_y()
+        self._ensure_point()
+        if self._sinv is None:
+            self._sinv = model.global_covariance()
+        if self._pred_blocks is None:
+            self._pred_blocks = (model.prediction_cross(self._sinv), model.local_cov(self._sinv))
+        cross, lcov = self._pred_blocks
+        r = model.approximate_loo(self._sinv, cross, lcov)
+        if is_torch(self._opt0):
+            return r
+        return r._replace(**{f: getattr(r, f).cpu().numpy() for f in ("lpd", "lpd_loo", "eta_mean_loo",
+                                                                      "eta_var_loo")})
+
     MAX_DENSE = 1 << 26
 
     def get_lr_covariance_from_jacobians(self, moment_jacobian1, moment_jacobian2=None):

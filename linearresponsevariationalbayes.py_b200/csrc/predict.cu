@@ -14,6 +14,13 @@
 // (K x 3K, built by k_predict_pmat) followed by row dot products with [x | x^2 | x^2].  eta = z_m uses
 // a = 1, b = 0.  No per-row intermediate leaves the SM.
 //
+// Approximate leave-one-out (LOO) over the handle's own training rows (lrvb_glmm_loo, DESIGN.md 3c) runs the LR pass
+// with a = 1, b = 0 and a = 0, b = 1 at once: the three quadratic forms, the cross dot products and Sigma_g give
+//   Q_n = [j_m; j_v] H^-1 [j_m; j_v]^T,   j_m = d z_m / d free,  j_v = d z_v / d free,
+// and with W_m = w_n l_m, W_v = w_n l_v (rows 0, 1 of the handle's W, written by the last evaluation) the infinitesimal
+// jackknife moves the row's moments by (dz_m, dz_v) = -Q_n (W_m, W_v).  The epilogue evaluates log E_q[p(y_n | z)]
+// by the Gauss-Hermite rule before and after the shift (y = 0 as log E[sigma(-z)]: no cancellation when p -> 1).
+//
 // Every row's result depends on that row alone and is computed in the same order wherever the row sits
 // in a tile, so a permutation of the rows permutes the outputs bitwise.  Rows of one group read the same
 // C_g / Sigma_g, which stay in L1 when the rows are visited group by group: `order` (optional) is the
@@ -124,13 +131,16 @@ k_predict_cross(const double* __restrict__ Sinv, const double* __restrict__ B, c
 //   phase 1  lane = row: z_m, z_v, the four cross dot products, the quadrature, the MFVB outputs
 //   phase 2  (LR) the three quadratic forms of 32 rows on the DMMA units, then the LR variances
 // out: (4, M) [eta_mean, eta_var_mfvb, prob, prob_var_mfvb] or, LR, (6, M) + [prob_var_lr, eta_var_lr].
-template <bool LR, int KP8>
+// LOO (implies LR; training rows, order = NULL): phase 1 without its quadrature, then the epilogue above reading y and
+// W rows 0-1 (row stride ldw); out (4, M) [lpd, lpd_loo, eta_mean_loo, eta_var_loo].  The LOO arguments come last,
+// so the other instantiations keep their parameter layout.
+template <bool LR, int KP8, bool LOO = false>
 __global__ void __launch_bounds__(32 * kPrMaxWarps, 1)
 k_predict(const double* __restrict__ X, const int32_t* __restrict__ g, const int64_t* __restrict__ order, int64_t M,
           const double* __restrict__ vec, const double* __restrict__ freev,
           const double* __restrict__ gh, const double* __restrict__ Bt, const double* __restrict__ Sinv,
           const double* __restrict__ cross, const double* __restrict__ lcov, double* __restrict__ out, int K, int G,
-          int Q, lrvb_glmm_bounds bd) {
+          int Q, lrvb_glmm_bounds bd, const double* __restrict__ yv, const double* __restrict__ Wl, int64_t ldw) {
   extern __shared__ __align__(16) double sm[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
   const int S = pr_stride(K), Kp8 = KP8 ? KP8 : pr_kp8(K), Kp4 = pr_kp4(K), Dg = 4 + 2 * K;
@@ -235,11 +245,11 @@ k_predict(const double* __restrict__ X, const int32_t* __restrict__ g, const int
     }
     const double zs = sqrt(zv);
     GHSumsF s = {0, 0, 0, 0, 0, 0, 0};
-    gh_all_nodes_f<3, kOfUnroll>(zm, zs, ghc, ghw, Q, s);
+    if (!LOO) gh_all_nodes_f<3, kOfUnroll>(zm, zs, ghc, ghw, Q, s);
     const double p = s.Am;
     const double a = s.Amm, b = s.Ams * (0.5 / zs);
     const double nan = __longlong_as_double(0x7ff8000000000000ll);
-    if (valid) {
+    if (valid && !LOO) {
       out[o] = bad ? nan : zm;
       out[M + o] = bad ? nan : zv;
       out[2 * M + o] = bad ? nan : p;
@@ -312,9 +322,30 @@ k_predict(const double* __restrict__ X, const int32_t* __restrict__ g, const int
       const double quad = a * a * vm + 2.0 * a * b * vs + b * b * vq;
       const double crs = a * (cm0 * l0 + cm1 * l1) + b * (cs0 * l0 + cs1 * l1);
       const double sig = l0 * l0 * s00 + 2.0 * l0 * l1 * s01 + l1 * l1 * s11;
-      if (valid) {
+      if (valid && !LOO) {
         out[4 * M + o] = bad ? nan : quad + 2.0 * crs + sig;
         out[5 * M + o] = bad ? nan : vm + 2.0 * cm0 + s00;
+      }
+      if (LOO) {
+        // Q_n: the forms above with (a, b) = (1, 0), (1, 0) x (0, 1) and (0, 1)
+        const double qmm = vm + 2.0 * cm0 + s00;
+        const double qmv = vs + dg * cm1 + cs0 + dg * s01;
+        const double qvv = vq + 2.0 * dg * cs1 + dg * dg * s11;
+        const double wm = valid ? Wl[o] : 0.0, wv = valid ? Wl[ldw + o] : 0.0;
+        // w_n = 0: W_m = W_v = 0, the shift is exactly zero and both quadratures see the same (z_m, z_s)
+        const double zm1 = zm - fma(qmm, wm, qmv * wv);
+        const double zv1 = zv - fma(qmv, wm, qvv * wv);
+        const bool ok = zv1 > 0.0;    // outside the linearisation's range: NaN, nothing clamped
+        const double sgn = (valid && yv[o] == 0.0) ? -1.0 : 1.0;
+        GHSumsF s0 = {0, 0, 0, 0, 0, 0, 0}, s1 = {0, 0, 0, 0, 0, 0, 0};
+        gh_all_nodes_f<1, kOfUnroll>(sgn * zm, zs, ghc, ghw, Q, s0);
+        gh_all_nodes_f<1, kOfUnroll>(sgn * zm1, ok ? sqrt(zv1) : 1.0, ghc, ghw, Q, s1);
+        if (valid) {
+          out[o] = log(s0.Am);
+          out[M + o] = ok ? log(s1.Am) : nan;
+          out[2 * M + o] = zm1;
+          out[3 * M + o] = ok ? zv1 : nan;
+        }
       }
     }
     __syncwarp();   // every lane is done with this slot before the refill
@@ -324,7 +355,7 @@ k_predict(const double* __restrict__ X, const int32_t* __restrict__ g, const int
   asm volatile("cp.async.wait_group 0;\n" ::: "memory");
 }
 
-template <bool LR, int KP8>
+template <bool LR, int KP8, bool LOO = false>
 static int launch_predict(lrvb_glmm* h, const double* freev, const double* X, const int32_t* g, const int64_t* order, int64_t M,
                           const double* Sinv,
                           const double* cross, const double* lcov, double* out, cudaStream_t st) {
@@ -333,11 +364,11 @@ static int launch_predict(lrvb_glmm* h, const double* freev, const double* X, co
   const size_t smem = warps * pr_warp_bytes(K) + pr_fixed_bytes(K, Q, KP8);
   static size_t configured = 48 * 1024;   // per instantiation
   if (smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_predict<LR, KP8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    LRVB_CUDA(cudaFuncSetAttribute(k_predict<LR, KP8, LOO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = smem;
   }
   int per_sm = 0;
-  LRVB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_predict<LR, KP8>, 32 * warps, smem));
+  LRVB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_predict<LR, KP8, LOO>, 32 * warps, smem));
   if (per_sm < 1) per_sm = 1;
   const int64_t ntiles = (M + kPrRows - 1) / kPrRows;
   int64_t grid = (ntiles + warps - 1) / warps;
@@ -347,8 +378,9 @@ static int launch_predict(lrvb_glmm* h, const double* freev, const double* X, co
     k_predict_pmat<<<cdiv(nb, 256), 256, 0, st>>>(Sinv, h->vec, h->pred_B, K, h->bounds.beta_info);
     LRVB_CHECK_LAUNCH();
   }
-  k_predict<LR, KP8><<<(int)grid, 32 * warps, smem, st>>>(X, g, order, M, h->vec, freev, h->gh, h->pred_B, Sinv, cross, lcov, out, K,
-                                                    h->G, Q, h->bounds);
+  k_predict<LR, KP8, LOO><<<(int)grid, 32 * warps, smem, st>>>(X, g, order, M, h->vec, freev, h->gh, h->pred_B, Sinv, cross, lcov,
+                                                         out, K, h->G, Q, h->bounds, LOO ? h->y : nullptr,
+                                                         LOO ? h->W : nullptr, h->ldw);
   LRVB_CHECK_LAUNCH();
   return LRVB_OK;
 }
@@ -360,6 +392,19 @@ static int check_rows(lrvb_glmm* h, const char* who, const double* X, int32_t K,
   LRVB_REQUIRE(M >= 0, "%s: M = %lld negative", who, (long long)M);
   LRVB_REQUIRE(M == 0 || (X && g && out), "%s: NULL argument", who);
   LRVB_REQUIRE((((uintptr_t)X) & 15) == 0, "%s: X not 16-byte aligned", who);
+  return LRVB_OK;
+}
+
+// the (3 Kp8, Kp4) scratch of the LR pass, allocated in the handle on first use
+static int ensure_pred_B(lrvb_glmm* h, const char* who) {
+  if (h->pred_B) return LRVB_OK;
+  const size_t nb = 3 * (size_t)pr_kp8(h->K) * pr_kp4(h->K);
+  if (cudaMalloc(&h->pred_B, sizeof(double) * nb) != cudaSuccess) {
+    cudaGetLastError();
+    h->pred_B = nullptr;
+    set_error("%s: out of device memory (%zu bytes of scratch)", who, sizeof(double) * nb);
+    return LRVB_ECUDA;
+  }
   return LRVB_OK;
 }
 
@@ -408,15 +453,7 @@ int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cro
   }
   LRVB_REQUIRE(Sinv_dev && ((cross_dev && localcov_dev) || h->G == 0), "lrvb_glmm_predict_lr: NULL argument");
   if (M == 0) return LRVB_OK;
-  if (!h->pred_B) {
-    const size_t nb = 3 * (size_t)pr_kp8(h->K) * pr_kp4(h->K);
-    if (cudaMalloc(&h->pred_B, sizeof(double) * nb) != cudaSuccess) {
-      cudaGetLastError();
-      h->pred_B = nullptr;
-      set_error("lrvb_glmm_predict_lr: out of device memory (%zu bytes of scratch)", sizeof(double) * nb);
-      return LRVB_ECUDA;
-    }
-  }
+  LRVB_TRY(ensure_pred_B(h, "lrvb_glmm_predict_lr"));
   const cudaStream_t st = (cudaStream_t)stream;
 #define LRVB_PR_LR(KP) \
   case KP: return launch_predict<true, KP>(h, nullptr, X_dev, g_dev, order_dev, M, Sinv_dev, cross_dev, localcov_dev, out_dev, st);
@@ -425,6 +462,30 @@ int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cro
     default: return launch_predict<true, 0>(h, nullptr, X_dev, g_dev, order_dev, M, Sinv_dev, cross_dev, localcov_dev, out_dev, st);
   }
 #undef LRVB_PR_LR
+}
+
+int lrvb_glmm_loo(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
+                  double* out_dev, void* stream) {
+  LRVB_REQUIRE(h != nullptr, "lrvb_glmm_loo: NULL handle");
+  if (!h->hess_valid || h->vecmode) {
+    set_error("lrvb_glmm_loo: no Hessian in free coordinates cached (call lrvb_glmm_eval with order 2)");
+    return LRVB_ESTATE;
+  }
+  const int64_t N = h->N;
+  LRVB_REQUIRE(Sinv_dev && ((cross_dev && localcov_dev) || h->G == 0) && (out_dev || N == 0),
+               "lrvb_glmm_loo: NULL argument");
+  if (N == 0) return LRVB_OK;
+  LRVB_REQUIRE((((uintptr_t)h->X) & 15) == 0, "lrvb_glmm_loo: the training X is not 16-byte aligned");
+  LRVB_TRY(ensure_pred_B(h, "lrvb_glmm_loo"));
+  const cudaStream_t st = (cudaStream_t)stream;
+  // the training rows are group-sorted already: visited in place, order = NULL
+#define LRVB_PR_LOO(KP) \
+  case KP: return launch_predict<true, KP, true>(h, nullptr, h->X, h->g, nullptr, N, Sinv_dev, cross_dev, localcov_dev, out_dev, st);
+  switch (h->K <= kPrSmemK ? pr_kp8(h->K) : 0) {
+    LRVB_PR_LOO(8) LRVB_PR_LOO(16) LRVB_PR_LOO(24)
+    default: return launch_predict<true, 0, true>(h, nullptr, h->X, h->g, nullptr, N, Sinv_dev, cross_dev, localcov_dev, out_dev, st);
+  }
+#undef LRVB_PR_LOO
 }
 
 }  // extern "C"

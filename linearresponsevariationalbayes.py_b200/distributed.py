@@ -486,6 +486,10 @@ class ShardedLogisticGLMM(object):
 
     predict = prediction_jacobian = _no_prediction
 
+    def approximate_loo(self, *args, **kwargs):
+        raise NotImplementedError("approximate LOO of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                  "and use LinearResponseCovariances.get_approximate_loo")
+
     def moment_jacobian(self, free):
         import scipy.sparse
         free = np.asarray(free, dtype=np.float64).reshape(-1)
