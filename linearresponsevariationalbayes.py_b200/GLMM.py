@@ -14,7 +14,6 @@ accepts it in place of ``fun``.
                   + entropies(mu, beta, u, tau) + priors(mu, beta, tau) )
 """
 import ctypes
-import os
 import weakref
 from collections import namedtuple
 from dataclasses import dataclass
@@ -542,7 +541,7 @@ class LogisticGLMM(object):
         # small problems are launch-bound: the four launches of a full export are cheaper than the refill
         # plus its conditional fallback (and the host-side bookkeeping of the pending check)
         small = self.Dg * self.Dg + 4 * self.Dg * self.G < self._csr_refill_min
-        if pat is None or small or os.environ.get("LRVB_CSR_REFILL", "1") == "0":
+        if pat is None or small:
             pat, val = self._export_full()
             self._csr_pattern = pat
             return DeviceCSR(pat, val)

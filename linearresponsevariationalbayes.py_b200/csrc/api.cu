@@ -151,12 +151,10 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
   h->ldw = (N + 7) / 8 * 8;
   CREATE_TRY(dev_alloc(&h->W, 5 * (size_t)h->ldw));
 
-  // observation pass geometry (k_obs, K > 62: 64-row tiles; obs_nbuf = tile buffers, two when they fit;
-  // LRVB_OBS_NBUF=1 forces one)
+  // observation pass geometry (k_obs, K > 62: 64-row tiles; obs_nbuf = tile buffers, two when they fit)
   {
     const size_t tile = sizeof(double) * 64 * (size_t)K, extra = sizeof(double) * (2 * (size_t)(Q + 3) + 32 + 2);
     h->obs_nbuf = (2 * tile + extra <= 220 * 1024) ? 2 : 1;
-    if (getenv("LRVB_OBS_NBUF") && getenv("LRVB_OBS_NBUF")[0] == '1') h->obs_nbuf = 1;
     h->obs_smem = h->obs_nbuf * tile + extra;
     int64_t nt = (N + 63) / 64;
     h->obs_grid = (int)(nt < kNumSMs ? nt : kNumSMs);
@@ -177,9 +175,8 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
     int64_t nrec = tw;
     {
       // one-slot rings when they buy at least three more warps per SM (K >= ~36)
-      const char* e1 = getenv("LRVB_OBS_ONESLOT");
       const int w1 = obs_fused_warps(K, 1);
-      if (e1 ? (e1[0] != '0') : (w1 >= h->of_warps + 3)) {
+      if (w1 >= h->of_warps + 3) {
         int64_t g1 = (nst + w1 - 1) / w1;
         if (g1 > kNumSMs) g1 = kNumSMs;
         if (g1 < 1) g1 = 1;
@@ -192,24 +189,22 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
         if (h->obs_grid < h->of1_grid) h->obs_grid = h->of1_grid;
       }
     }
-    {
+    if (K <= kFuMaxK) {
       // order 2 in one pass (fused.cuh): teams of NQ quadrature warps + P DMMA warps, one CTA per SM; every
-      // Q warp owns a contiguous multiple-of-32 range of rows
-      const char* fe = getenv("LRVB_FUSED");
-      const FusedGeom fg = fused_geom((2 * K + 7) / 8);
-      const int nqw = fg.teams * fg.NQ;
+      // Q warp owns a contiguous multiple-of-32 range of rows.  Only for K <= 24, where quadrature and Gram
+      // need about the same pipe time and the one-pass kernel is ~10 % faster than the two kernels; for larger
+      // K the Gram dominates, the D warps of the one-pass kernel (128 registers, 4 warps per triangle) are
+      // slower than gram_mid's (255 registers, 2 warps) and the two-kernel path wins
+      // (profiles/r02_onepass_attempts.md).
+      const int nqw = kFuGeom.teams * kFuGeom.NQ;
       int64_t fgrid = (nst + nqw - 1) / nqw;
       if (fgrid > kNumSMs) fgrid = kNumSMs;
       if (fgrid < 1) fgrid = 1;
       const int64_t tt = fgrid * nqw;
-      // default: K <= 24, where quadrature and Gram need about the same pipe time and the one-pass kernel
-      // is ~10 % faster than the two kernels; for larger K the Gram dominates, the D warps of the one-pass
-      // kernel (128 registers, 4 warps per triangle) are slower than gram_mid's (255 registers, 2 warps) and
-      // the two-kernel path wins (profiles/r02_onepass_attempts.md).  LRVB_FUSED=1 / 0 forces / disables it.
-      h->fused2 = fe ? (fe[0] != '0') : ((2 * K + 7) / 8 <= 6);
+      h->fused2 = 1;
       h->fu_grid = (int)fgrid;
       h->fu_teams = nqw;
-      h->fu_warps = fg.warps;
+      h->fu_warps = kFuGeom.warps;
       h->fu_rows_per_team = ((nst + tt - 1) / tt) * kFuRows;
       if (tt > nrec) nrec = tt;
     }
@@ -234,27 +229,16 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
   // Gram geometry
   {
     size_t npart;
-    // K < 16: gram_small (register prefetch pays when a k-step is only a handful of DMMAs); from 16 on
-    // gram_mid's 16 warps without prefetch are 3-4 % faster (profiles/r01_gram_mid_sweep.log)
-    const char* gs_env = getenv("LRVB_GRAM_SMALL");
-    const int gs_max = gs_env ? (gs_env[0] == '0' ? 0 : 20) : 15;
-    if (K <= gs_max) {
-      // small K: every warp owns the whole packed upper triangle (gram_small.cuh), one CTA per SM
-      h->gram_small = 1;
-      h->gram_grid_x = kNumSMs;
-      h->gram_grid_y = 1;
-      npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
-    } else if (K <= kGmMaxK && !(getenv("LRVB_GRAM_MID") && getenv("LRVB_GRAM_MID")[0] == '0')) {
-      // 20 < K <= 52: still one warp = the whole packed triangle, 8 - 12 warps per SM (gram_mid.cuh)
+    if (h->fused2) {
+      // no Gram kernel: the one-pass kernel (fused.cuh) writes the packed partials, one slab per CTA
+      npart = (size_t)h->fu_grid * gram_small_shape(K).NT * 64;
+    } else if (K <= kGmMaxK) {
+      // 24 < K <= 104: one warp or a team of warps = the whole packed triangle (gram_mid.cuh)
       h->gram_mid = 1;
       h->gram_grid_x = kNumSMs;
       h->gram_grid_y = 1;
       npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
-    } else if (gram_wide_eligible(K) &&
-               (getenv("LRVB_GRAM_WIDE") ? getenv("LRVB_GRAM_WIDE")[0] != '0' : (K >= 176 && K <= 240))) {
-      // default range = where it beats the rectangle kernel (profiles/r02_gram_wide.md: 56 - 66 % against
-      // 49 - 55 % of the DMMA peak for K = 176 .. 240; below, the 4-tile blocks starve the warps and the
-      // staged bytes per DMMA grow; LRVB_GRAM_WIDE=1 forces it for every K >= 96 with K % 8 == 0)
+    } else if (gram_wide_eligible(K)) {
       // large K, no straddle tile: block-against-block jobs (16 - 25 tiles per warp), 8 warps per SM, only the
       // column blocks of a job group staged (gram_wide.cuh)
       const GwPlan pl = gram_wide_plan(K);

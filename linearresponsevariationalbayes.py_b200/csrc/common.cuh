@@ -231,7 +231,7 @@ struct lrvb_glmm {
   double* klpart = nullptr;   // (obs_grid) per-CTA partials of sum w*l
   double* gradpart = nullptr; // (obs_grid, 2, K) per-CTA partials of X^T l_m , S^T l_v
   // fused observation + group pass (K <= 62, obs_fused.cuh)
-  int gram_mid = 0;           // 20 < K <= 52: every warp owns the packed triangle (gram_mid.cuh)
+  int gram_mid = 0;           // 24 < K <= 104: a warp or team of warps owns the packed triangle (gram_mid.cuh)
   int obs_fused = 0, of_grid = 0, of_warps = 0;
   size_t of_smem = 0;
   int64_t of_rows_per_warp = 0;
@@ -241,7 +241,7 @@ struct lrvb_glmm {
   int of1_grid = 0, of1_warps = 0;
   size_t of1_smem = 0;
   int64_t of1_rows_per_warp = 0;
-  // order-2 evaluation in one pass (team.cuh): teams of warps do quadrature, group sums and Gram per stage
+  // order-2 evaluation in one pass (fused.cuh, K <= 24): teams of warps do quadrature, group sums and Gram per stage
   int fused2 = 0, fu_grid = 0, fu_teams = 0, fu_warps = 0;
   int64_t fu_rows_per_team = 0;
   int ev_gram = 0;            // the last timed evaluation ran a separate Gram kernel
@@ -255,9 +255,8 @@ struct lrvb_glmm {
   // Gram
   int gram_tn = 0, gram_grid_x = 0, gram_grid_y = 0, gram_jobs = 0;   // grid_y = job groups
   size_t gram_smem = 0;
-  int gram_small = 0;         // K <= 20: packed whole-triangle-per-warp kernel (gram_small.cuh)
   int group_overlap = 1;      // k_group on the side stream behind k_gram_wide (LRVB_GROUP_OVERLAP=0: serial)
-  int gram_wide = 0;          // K >= 96, K % 8 == 0: block jobs of 4-5 tiles, 8 warps x 255 registers (gram_wide.cuh);
+  int gram_wide = 0;          // K = 176 .. 240, K % 8 == 0: block jobs of 4-5 tiles, 8 warps x 255 registers (gram_wide.cuh);
                               // jobs = GwGroup[], gslots = GwCta[gram_grid_x]
   void* jobs = nullptr;            // device GbJob[gram_jobs]   (gram_big.cuh, K > 20)
   void* gslots = nullptr;          // device GbSlot[gram_grid_y * 16]

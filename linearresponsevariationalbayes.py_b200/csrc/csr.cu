@@ -366,8 +366,7 @@ __device__ __forceinline__ void csr_roles(const double* A, const double* B, cons
 // One launch per phase: blocks [0, nA) take the rows of A, the next nB blocks a chunk of B each,
 // the rest the local rows (block-uniform roles; only the B role uses the dynamic shared memory).
 // FILL = 0 count, 1 fill (and record the zero mask), 2 refill: data only with the cached offsets, the
-// zero mask compared with the recorded one.  run_if (nullable): the kernel is a no-op unless *run_if != 0
-// (the conditional full export behind a refill).
+// zero mask compared with the recorded one.
 template <int FILL>
 __global__ void __launch_bounds__(256)
 k_csr_pass(const double* __restrict__ A, const double* __restrict__ B, const double* __restrict__ L,
@@ -375,7 +374,7 @@ k_csr_pass(const double* __restrict__ A, const double* __restrict__ B, const dou
            int32_t* __restrict__ chunkcnt, const int32_t* __restrict__ chunkoff,
            const int32_t* __restrict__ coltot, int32_t* __restrict__ rowcnt,
            const int32_t* __restrict__ indptr, int32_t* __restrict__ indices, double* __restrict__ data,
-           uint32_t* __restrict__ mask, const MismatchFlag mismatch, const int* __restrict__ run_if) {
+           uint32_t* __restrict__ mask, const MismatchFlag mismatch) {
   const int bid = blockIdx.x;
   if constexpr (FILL == 2) {
   if (bid >= nA) {
@@ -398,7 +397,6 @@ k_csr_pass(const double* __restrict__ A, const double* __restrict__ B, const dou
   }
   }
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   csr_roles<FILL>(A, B, L, Dg, G, CG, nA, nB, cntA, chunkcnt, chunkoff, coltot, rowcnt, indptr, indices, data, mask,
                   mismatch);
 }
@@ -408,9 +406,8 @@ __device__ __forceinline__ void csr_colscan_body(int c, const int32_t* chunkcnt,
                                                  int nchunk, int ncol);
 __global__ void __launch_bounds__(256)
 k_csr_colscan(const int32_t* __restrict__ chunkcnt, int32_t* __restrict__ chunkoff,
-              int32_t* __restrict__ coltot, int nchunk, int ncol, const int* __restrict__ run_if) {
+              int32_t* __restrict__ coltot, int nchunk, int ncol) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   csr_colscan_body(blockIdx.x, chunkcnt, chunkoff, coltot, nchunk, ncol);
 }
 __device__ __forceinline__ void csr_colscan_body(int c, const int32_t* chunkcnt, int32_t* chunkoff, int32_t* coltot,
@@ -445,9 +442,8 @@ __device__ __forceinline__ void csr_colscan_body(int c, const int32_t* chunkcnt,
 // rowcnt[r] for the global rows
 __global__ void k_csr_global_rowcnt(const int32_t* __restrict__ cntA,
                                     const int32_t* __restrict__ coltot, int Dg,
-                                    int32_t* __restrict__ rowcnt, const int* __restrict__ run_if) {
+                                    int32_t* __restrict__ rowcnt) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r < Dg) rowcnt[r] = cntA[r] + coltot[r] + coltot[Dg + r];
 }
@@ -457,9 +453,8 @@ __device__ __forceinline__ void scan_sum_body(int vb, const int32_t* cnt, int64_
 __device__ __forceinline__ void scan_apply_body(int vb, int nblk, const int32_t* cnt, int64_t n, const int64_t* blk,
                                                 const int64_t* total, int32_t* indptr);
 __global__ void __launch_bounds__(256)
-k_scan_sum(const int32_t* __restrict__ cnt, int64_t n, int64_t* __restrict__ blk, const int* __restrict__ run_if) {
+k_scan_sum(const int32_t* __restrict__ cnt, int64_t n, int64_t* __restrict__ blk) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   scan_sum_body(blockIdx.x, cnt, n, blk);
 }
 __device__ __forceinline__ void scan_sum_body(int vb, const int32_t* cnt, int64_t n, int64_t* blk) {
@@ -475,9 +470,8 @@ __device__ __forceinline__ void scan_sum_body(int vb, const int32_t* cnt, int64_
 
 __device__ __forceinline__ void scan_top_body(int64_t* blk, int nblk, int64_t* total, int64_t* nnz_out);
 __global__ void k_scan_top(int64_t* __restrict__ blk, int nblk, int64_t* __restrict__ total,
-                           int64_t* __restrict__ nnz_out, const int* __restrict__ run_if) {
+                           int64_t* __restrict__ nnz_out) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   scan_top_body(blk, nblk, total, nnz_out);
 }
@@ -494,10 +488,8 @@ __device__ __forceinline__ void scan_top_body(int64_t* blk, int nblk, int64_t* t
 
 __global__ void __launch_bounds__(256)
 k_scan_apply(const int32_t* __restrict__ cnt, int64_t n, const int64_t* __restrict__ blk,
-             const int64_t* __restrict__ total, int32_t* __restrict__ indptr,
-             const int* __restrict__ run_if) {
+             const int64_t* __restrict__ total, int32_t* __restrict__ indptr) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   scan_apply_body(blockIdx.x, gridDim.x, cnt, n, blk, total, indptr);
 }
 __device__ __forceinline__ void scan_apply_body(int vb, int nblk, const int32_t* cnt, int64_t n, const int64_t* blk,
@@ -607,9 +599,8 @@ constexpr int64_t kIndptrOneCta = 262144;
 __global__ void __launch_bounds__(1024)
 k_csr_indptr_small(const int32_t* __restrict__ cntA, const int32_t* __restrict__ coltot, int Dg,
                    const int32_t* __restrict__ rowcnt, int64_t n, int32_t* __restrict__ indptr,
-                   int64_t* __restrict__ nnz_out, const int* __restrict__ run_if) {
+                   int64_t* __restrict__ nnz_out) {
   pdl_sync();
-  if (run_if && *run_if == 0) return;
   __shared__ int wsum[32];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   long long carry = 0;
@@ -727,7 +718,7 @@ static int csr_full_export(lrvb_glmm* h, int32_t* indptr_dev, int32_t* indices_d
   const size_t smem = sizeof(double) * (size_t)CG * (2 * Dg + 1);
 
   const int nA = cdiv(Dg, 8), nB = (G > 0) ? nchunk : 0, nL = (G > 0) ? cdiv(2 * (int64_t)G, 8) : 0;
-  if (run_if && !(getenv("LRVB_CSR_COOP") && getenv("LRVB_CSR_COOP")[0] == '0')) {
+  if (run_if) {
     // the conditional export behind a refill: one launch of co-resident CTAs (two per SM)
     int32_t* segb = chunkoff + (size_t)2 * Dg * nchunk;
     unsigned* bar = (unsigned*)(segb + (size_t)2 * Dg * nchunk);
@@ -740,14 +731,13 @@ static int csr_full_export(lrvb_glmm* h, int32_t* indptr_dev, int32_t* indices_d
     return LRVB_OK;
   }
   // ---- counts: rows of A, columns of B (per chunk) and local rows in one launch ----
-  int pass_grid = nA + nB + nL;
-  if (run_if && pass_grid > 4 * kNumSMs) pass_grid = 4 * kNumSMs;
+  const int pass_grid = nA + nB + nL;
   LRVB_CUDA(launch_pdl(k_csr_pass<0>, dim3(pass_grid), dim3(256), smem, st, h->A, h->B, h->L, Dg, G,
                        CG, nA, nB, cntA, chunkcnt, nullptr, nullptr, h->rowcnt, nullptr, nullptr, nullptr,
-                       (uint32_t*)nullptr, MismatchFlag{nullptr, nullptr}, run_if));
+                       (uint32_t*)nullptr, MismatchFlag{nullptr, nullptr}));
   LRVB_CHECK_LAUNCH();
   if (G > 0) {
-    LRVB_CUDA(launch_pdl(k_csr_colscan, dim3(2 * Dg), dim3(256), 0, st, chunkcnt, chunkoff, coltot, nchunk, 2 * Dg, run_if));
+    LRVB_CUDA(launch_pdl(k_csr_colscan, dim3(2 * Dg), dim3(256), 0, st, chunkcnt, chunkoff, coltot, nchunk, 2 * Dg));
     LRVB_CHECK_LAUNCH();
   } else {
     LRVB_CUDA(cudaMemsetAsync(coltot, 0, sizeof(int32_t) * 2 * Dg, st));
@@ -755,23 +745,23 @@ static int csr_full_export(lrvb_glmm* h, int32_t* indptr_dev, int32_t* indices_d
   // ---- indptr ----
   if (D <= kIndptrOneCta) {
     LRVB_CUDA(launch_pdl(k_csr_indptr_small, dim3(1), dim3(1024), 0, st, cntA, coltot, Dg, h->rowcnt, D,
-                         indptr_dev, (int64_t*)nnz_dev, run_if));
+                         indptr_dev, (int64_t*)nnz_dev));
     LRVB_CHECK_LAUNCH();
   } else {
-    LRVB_CUDA(launch_pdl(k_csr_global_rowcnt, dim3(cdiv(Dg, 256)), dim3(256), 0, st, cntA, coltot, Dg, h->rowcnt, run_if));
+    LRVB_CUDA(launch_pdl(k_csr_global_rowcnt, dim3(cdiv(Dg, 256)), dim3(256), 0, st, cntA, coltot, Dg, h->rowcnt));
     LRVB_CHECK_LAUNCH();
-    LRVB_CUDA(launch_pdl(k_scan_sum, dim3(nblk), dim3(256), 0, st, h->rowcnt, D, blk, run_if));
+    LRVB_CUDA(launch_pdl(k_scan_sum, dim3(nblk), dim3(256), 0, st, h->rowcnt, D, blk));
     LRVB_CHECK_LAUNCH();
-    LRVB_CUDA(launch_pdl(k_scan_top, dim3(1), dim3(32), 0, st, blk, nblk, blk + nblk, nnz_dev, run_if));
+    LRVB_CUDA(launch_pdl(k_scan_top, dim3(1), dim3(32), 0, st, blk, nblk, blk + nblk, nnz_dev));
     LRVB_CHECK_LAUNCH();
-    LRVB_CUDA(launch_pdl(k_scan_apply, dim3(nblk), dim3(256), 0, st, h->rowcnt, D, blk, blk + nblk, indptr_dev, run_if));
+    LRVB_CUDA(launch_pdl(k_scan_apply, dim3(nblk), dim3(256), 0, st, h->rowcnt, D, blk, blk + nblk, indptr_dev));
     LRVB_CHECK_LAUNCH();
   }
   // ---- fill: the same three roles, one launch; records the zero mask for later refills ----
   int32_t* segbase = chunkoff + (size_t)2 * Dg * nchunk;
   LRVB_CUDA(launch_pdl(k_csr_pass<1>, dim3(pass_grid), dim3(256), smem, st, h->A, h->B, h->L, Dg, G, CG,
                        nA, nB, cntA, segbase, chunkoff, coltot, nullptr, indptr_dev, indices_dev, data_dev,
-                       h->csrmask, MismatchFlag{nullptr, nullptr}, run_if));
+                       h->csrmask, MismatchFlag{nullptr, nullptr}));
   LRVB_CHECK_LAUNCH();
   h->csr_pattern_valid = 1;
   return LRVB_OK;
@@ -815,7 +805,7 @@ int lrvb_glmm_hessian_csr_refill(lrvb_glmm* h, const int32_t* indptr_dev, double
   const bool merged = G >= 32768;
   LRVB_CUDA(launch_pdl(k_csr_pass<2>, dim3(nA + nB + (merged ? 0 : nL)), dim3(256), smem, st, h->A, h->B, h->L, Dg, G, CG,
                        nA, nB, cntA, merged ? segbase : nullptr, chunkoff, coltot, nullptr, indptr_dev, (int32_t*)nullptr, data_dev,
-                       h->csrmask, MismatchFlag{(int*)mismatch_dev, (int*)mismatch_host_mapped}, (const int*)nullptr));
+                       h->csrmask, MismatchFlag{(int*)mismatch_dev, (int*)mismatch_host_mapped}));
   LRVB_CHECK_LAUNCH();
   return LRVB_OK;
 }

@@ -1,5 +1,5 @@
 // Order-2 evaluation in ONE pass over X: the per-observation quadrature + per-group sums of obs_fused.cuh
-// and the packed weighted Gram of gram_mid.cuh as one persistent, warp-specialised kernel (K <= 62), sm_100a.
+// and the packed weighted Gram of gram_mid.cuh as one persistent, warp-specialised kernel (K <= 24), sm_100a.
 //
 // Why: run back to back, the observation pass keeps the FP64 pipe ~50 % busy and the Gram kernel ~80 %
 // (DMMA), and each reads X from HBM.  What limits the observation pass is the DEPENDENT-issue latency of
@@ -44,28 +44,23 @@ constexpr int kFuRows = 32;          // rows per stage (= lanes of the Q warp = 
 #endif
 constexpr int kFuUnroll = LRVB_FUSED_UNROLL;   // quadrature nodes in flight per lane
 
+// K <= 24 (T2 <= 6), where quadrature and Gram need about the same pipe time
+constexpr int kFuMaxK = 24;
+
 struct FusedGeom {
   int teams, NQ, P, warps, slots;    // warps = CTA size / 32; slots = ring depth per Q warp
 };
-// T2 <= 6 (K <= 24; quadrature and Gram need about the same pipe time): 4 teams -- one per SM
-//   sub-partition -- of 3 Q warps + 1 D warp (15 / 21 accumulator tiles), 2-slot rings.
-// T2 7..8 (K 25..32): 4 teams of 1 Q + 3 D warps (10 - 12 tiles each).
-// T2 9..13 (K <= 52): 3 teams of 1 Q + 4 D = 15 (+1 idle) warps, three D warps per sub-partition.
-// T2 14..16 (K <= 62): 2 teams of 1 Q + 7 D = 16 warps (17 - 20 tiles per D warp).
-__host__ __device__ constexpr FusedGeom fused_geom(int T2) {
-  return T2 <= 6 ? FusedGeom{4, 3, 1, 16, 2} : T2 <= 8 ? FusedGeom{4, 1, 3, 16, 3}
-       : T2 <= 13 ? FusedGeom{2, 3, 4, 16, 2} : FusedGeom{2, 1, 7, 16, 3};
-}
+// 4 teams -- one per SM sub-partition -- of 3 Q warps + 1 D warp (15 / 21 accumulator tiles), 2-slot rings
+constexpr FusedGeom kFuGeom = {4, 3, 1, 16, 2};
 __host__ __device__ inline int fused_slot_elems(int K) { return kFuRows * K + 2 * kFuRows + kFuRows / 2 + 6 * kFuRows; }
 inline size_t fused_smem(int K, int Q, int T2) {
-  const FusedGeom g = fused_geom(T2);
-  const int nq = g.teams * g.NQ;
-  const size_t ring = sizeof(double) * (size_t)nq * g.slots * fused_slot_elems(K);
+  const int nq = kFuGeom.teams * kFuGeom.NQ;
+  const size_t ring = sizeof(double) * (size_t)nq * kFuGeom.slots * fused_slot_elems(K);
   const size_t red = sizeof(double) * (size_t)(T2 * (T2 + 1) / 2) * 64;
   const size_t body = ring > red ? ring : red;
   // + beta mean / var (2K), GH nodes (2Q), gradient partials (Q warps x 2K), KL partials (Q warps), barriers
   return body + sizeof(double) * (2 * (size_t)K + 2 * Q + (size_t)nq * 2 * K + nq) +
-         sizeof(unsigned long long) * (size_t)nq * g.slots * 3;
+         sizeof(unsigned long long) * (size_t)nq * kFuGeom.slots * 3;
 }
 
 struct FusedArgs {
@@ -616,14 +611,14 @@ k_fused_eval(const FusedArgs a) {
 // launch the instantiation for K; false when K / alignment is outside its range
 inline bool launch_fused_eval(const FusedArgs& a, int grid, int Q, cudaStream_t st) {
   const int K = a.K;
-  if (K < 1 || K > kOfMaxK || (a.ldw & 1) || (((uintptr_t)a.X) & 15)) return false;
+  if (K < 1 || K > kFuMaxK || (a.ldw & 1) || (((uintptr_t)a.X) & 15)) return false;
   const int T2 = (2 * K + 7) / 8, T0 = K / 8;
   const bool M = (K % 8) != 0;
   const int nch = (K + 1 + 31) / 32;
   const size_t smem = fused_smem(K, Q, T2);
 #define LRVB_FU(T2_, T0_, M_, NCH_)                                                                  \
   if (T2 == T2_ && T0 == T0_ && M == M_ && nch == NCH_) {                                            \
-    constexpr FusedGeom g = fused_geom(T2_);                                                         \
+    constexpr FusedGeom g = kFuGeom;                                                                 \
     static size_t configured = 48 * 1024;                                                            \
     if (smem > configured) {                                                                         \
       cudaFuncSetAttribute(k_fused_eval<T2_, T0_, M_, NCH_, g.teams, g.NQ, g.P, g.warps, g.slots>,   \
@@ -642,21 +637,6 @@ inline bool launch_fused_eval(const FusedArgs& a, int grid, int Q, cudaStream_t 
   LRVB_FU(5, 2, true, 1)
   LRVB_FU(6, 2, true, 1)
   LRVB_FU(6, 3, false, 1)
-  LRVB_FU(7, 3, true, 1)
-  LRVB_FU(8, 3, true, 1)
-  LRVB_FU(8, 3, true, 2)
-  LRVB_FU(8, 4, false, 2)
-  LRVB_FU(9, 4, true, 2)
-  LRVB_FU(10, 4, true, 2)
-  LRVB_FU(10, 5, false, 2)
-  LRVB_FU(11, 5, true, 2)
-  LRVB_FU(12, 5, true, 2)
-  LRVB_FU(12, 6, false, 2)
-  LRVB_FU(13, 6, true, 2)
-  LRVB_FU(14, 6, true, 2)
-  LRVB_FU(14, 7, false, 2)
-  LRVB_FU(15, 7, true, 2)
-  LRVB_FU(16, 7, true, 2)
 #undef LRVB_FU
   return false;
 }

@@ -584,9 +584,9 @@ int launch_wide_influence(lrvb_glmm* h, const double* v, double* out, cudaStream
   return LRVB_OK;
 }
 
-// Finish of the small-K packed Gram (gram_small.cuh): fixed-order sum of the per-CTA partials of
-// one packed tile, then the same chain rule as k_gram_finish.  Packed column p < K is x_p,
-// p >= K is s_{p-K}; only the upper triangle of the packed matrix was computed.
+// Finish of the packed Gram (layout of gram_small.cuh, written by the one-pass, mid and wide kernels):
+// fixed-order sum of the per-CTA partials of one packed tile, then the same chain rule as k_gram_finish.
+// Packed column p < K is x_p, p >= K is s_{p-K}; only the upper triangle of the packed matrix was computed.
 __device__ __forceinline__ void gram_small_finish_body(int bid, const double* __restrict__ part, const double* __restrict__ vec,
                     double* __restrict__ A, int K, int Dg, int NT, int n_cta, lrvb_glmm_bounds bd,
                     int vecmode) {
@@ -1114,7 +1114,7 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
   const bool one_pass = h->fused2 && order >= 2 && N > 0;
   h->ev_gram = 0;
   if (one_pass) {
-    // order 2, K <= 62: quadrature, per-group sums and the packed Gram in ONE pass over X (fused.cuh)
+    // order 2, K <= 24: quadrature, per-group sums and the packed Gram in ONE pass over X (fused.cuh)
     if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[0], st));
     FusedArgs fa;
     fa.X = h->X; fa.y = h->y; fa.g = h->g; fa.w = h->w; fa.vec = h->vec; fa.gh = h->gh; fa.gptr = h->gptr;
@@ -1198,12 +1198,7 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
     if (N > 0) {
       h->ev_gram = 1;
       if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[2], st));
-      if (h->gram_small) {
-        if (!launch_gram_small(h->X, h->W + 2 * h->ldw, h->grampart, N, h->ldw, K, h->gram_grid_x, st)) {
-          set_error("launch_eval: small-K Gram kernel rejected K = %d / alignment", K);
-          return LRVB_ESTATE;
-        }
-      } else if (h->gram_mid) {
+      if (h->gram_mid) {
         if (!launch_gram_mid(h->X, h->W + 2 * h->ldw, h->grampart, N, h->ldw, K, h->gram_grid_x, st)) {
           set_error("launch_eval: mid-K Gram kernel rejected K = %d / alignment", K);
           return LRVB_ESTATE;
@@ -1233,7 +1228,7 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
   {
     const int n_loc = h->loc_grid;
     int n_bor = 0, n_gf = 0, NT = 0;
-    const int packed_gram = (h->gram_small || h->gram_mid || h->gram_wide || one_pass) ? 1 : 0;   // partial layout (n_cta, NT, 64)
+    const int packed_gram = (h->gram_mid || h->gram_wide || one_pass) ? 1 : 0;   // partial layout (n_cta, NT, 64)
     const int packed_ctas = one_pass ? h->fu_grid : h->gram_grid_x;
     if (order >= 2) {
       if (G > 0) n_bor = cdiv(G, 8 * border_groups_per_warp(G));

@@ -395,7 +395,7 @@ k_gram_big(const double* __restrict__ X, const double* __restrict__ Wabc, int64_
 }
 
 // Sum the partials of one (job, tile) over the row chunks and the k-splits in a fixed order and
-// write the beta block of A in free coordinates (same chain rule as k_gram_small_finish).
+// write the beta block of A in free coordinates (same chain rule as gram_small_finish_body).
 __device__ __forceinline__ void gram_big_finish_body(int bid, const double* __restrict__ part, const GbJob* __restrict__ jobs,
                   const GbSlot* __restrict__ slots, const double* __restrict__ vec,
                   double* __restrict__ A, int K, int Dg, int n_groups, int n_chunk,

@@ -1,4 +1,4 @@
-// Weighted Grams of the beta block for 16 <= K <= 104 on the FP64 tensor cores (DMMA.8x8x4), sm_100a.
+// Weighted Grams of the beta block for 25 <= K <= 104 on the FP64 tensor cores (DMMA.8x8x4), sm_100a.
 //
 // Same packed formulation as gram_small.cuh (ONE weighted Gram of z = [x | s], upper triangle of
 // the T2 x T2 tile grid, tile classes pure-x / straddle / pure-s) and the same execution model:
@@ -27,7 +27,7 @@ namespace lrvb {
 
 // rows per stage: 32 (8 k-steps between two ring hand-overs) wherever three slots of them fit beside the
 // other teams' rings -- from T2 = 9 on (<= 6 teams per CTA); measured 0.7 - 3.5 % faster than 16 for K = 36 .. 104
-// (K = 50: 3.680 -> 3.654 ms at N = 10M); the 12 - 16 single-warp teams of T2 <= 8 stay at 16 rows
+// (K = 50: 3.680 -> 3.654 ms at N = 10M); the 12 single-warp teams of T2 <= 8 stay at 16 rows
 __host__ __device__ constexpr int gram_mid_rows(int T2) { return T2 >= 9 ? 32 : 16; }
 constexpr int kGmStages = 3;      // ring depth per team
 constexpr int kGmMaxK = 104;      // T2 = ceil(2K / 8) <= 26
@@ -38,12 +38,11 @@ constexpr int kGmMaxK = 104;      // T2 = ceil(2K / 8) <= 26
 struct GramMidGeom {
   int warps, P;
 };
-// T2 <= 8: 12-16 single-warp teams at <= 168 registers; 9..13: pairs of warps; 14..20: teams of four;
+// T2 <= 8: 12 single-warp teams at <= 168 registers; 9..13: pairs of warps; 14..20: teams of four;
 // 21..26: one team of eight (8 warps x 255 registers from T2 = 11 on).  Fewer, larger roles amortise the
 // operand fetch of a k-step over more DMMAs: as few warps per team as the 255-register budget allows
 __host__ __device__ constexpr GramMidGeom gram_mid_geom(int T2) {
-  return T2 <= 6 ? GramMidGeom{16, 1}
-       : T2 <= 8 ? GramMidGeom{12, 1}
+  return T2 <= 8 ? GramMidGeom{12, 1}
        : T2 <= 10 ? GramMidGeom{12, 2}
        : T2 <= 13 ? GramMidGeom{8, 2}
        : T2 <= 20 ? GramMidGeom{8, 4} : GramMidGeom{8, 8};
@@ -320,7 +319,8 @@ k_gram_mid(const double* __restrict__ X, const double* __restrict__ Wabc, double
   for (int e = threadIdx.x; e < NT * 64; e += blockDim.x) out[e] = red[e];
 }
 
-// launch the instantiation for K (20 < K <= 52); false when K / alignment is outside its range
+// launch the instantiation for K (24 < K <= 104; below, the one-pass kernel of fused.cuh computes the Gram);
+// false when K / alignment is outside its range
 inline bool launch_gram_mid(const double* X, const double* Wabc, double* part, int64_t N, int64_t ldw,
                             int K, int grid, cudaStream_t st) {
   if (K < 1 || K > kGmMaxK || (ldw & 1) || (((uintptr_t)X) & 15) || (((uintptr_t)Wabc) & 15)) return false;
@@ -339,15 +339,6 @@ inline bool launch_gram_mid(const double* X, const double* Wabc, double* part, i
     return launch_pdl(k_gram_mid<T2_, T0_, M_, g.warps, g.P>, dim3(grid), dim3(32 * g.warps), smem, st, X, \
                       Wabc, part, N, ldw, K) == cudaSuccess;                                        \
   }
-  LRVB_GM(1, 0, true)
-  LRVB_GM(2, 0, true)
-  LRVB_GM(2, 1, false)
-  LRVB_GM(3, 1, true)
-  LRVB_GM(4, 1, true)
-  LRVB_GM(4, 2, false)
-  LRVB_GM(5, 2, true)
-  LRVB_GM(6, 2, true)
-  LRVB_GM(6, 3, false)
   LRVB_GM(7, 3, true)
   LRVB_GM(8, 3, true)
   LRVB_GM(8, 4, false)

@@ -1,4 +1,4 @@
-// Weighted Grams of the beta block for K <= 20 on the FP64 tensor cores (DMMA.8x8x4), sm_100a.
+// Packed formulation of the weighted Grams of the beta block on the FP64 tensor cores (DMMA.8x8x4), sm_100a.
 //
 //   G_a = X^T diag(a) X      G_b = X^T diag(b) S      G_c = S^T diag(c) S        S = X * X
 //
@@ -17,47 +17,14 @@
 //                        A = z_i masked to its s columns, B = z_j * c
 //   straddle row, pure-s column:   A = z_i * (b | c by the class of A's column),  B = z_j
 //
-// Every warp streams its own kGsRows-row stages through a private shared-memory ring filled by
-// bulk async copies (TMA, one mbarrier per slot): no block barrier and no per-element copy
-// instructions in the main loop, and all warps of all CTAs do identical work, so the four FP64
-// pipes of an SM are evenly loaded.  The CTA's warps are summed in a fixed order at the end: one
-// partial per CTA.  Measured on B200 (tools/gram_bench.cu, N = 1M, K = 20): 82 us against 203 us
-// for the rectangle kernel it replaces; per-row slope 68 us/M against a pure-DMMA floor of 57.
+// This header keeps what the packed Gram kernels (gram_mid.cuh, gram_wide.cuh, fused.cuh) and the other
+// bulk-copy kernels share: the mbarrier / bulk async copy helpers and the shape of the packed tile grid.
+// Their partials use one layout: part (n_cta, NT, 64) with NT = T2 (T2+1) / 2, tile (i <= j) at slot
+// j (j+1)/2 + i, element (r, c) of a tile at r * 8 + c.
 #pragma once
 #include "common.cuh"
 
 namespace lrvb {
-
-#ifndef LRVB_GS_ROWS
-#define LRVB_GS_ROWS 32
-#endif
-#ifndef LRVB_GS_STAGES
-#define LRVB_GS_STAGES 2
-#endif
-constexpr int kGsRows = LRVB_GS_ROWS;      // rows per warp stage (k-steps of 4 observations)
-constexpr int kGsStages = LRVB_GS_STAGES;  // bulk-copy ring depth per warp
-#ifndef LRVB_GS_WARPS
-#define LRVB_GS_WARPS 12
-#endif
-#ifndef LRVB_GS_MINB
-#define LRVB_GS_MINB 1
-#endif
-#ifndef LRVB_GS_STAGGER
-#define LRVB_GS_STAGGER 1
-#endif
-constexpr int kGsWarps = LRVB_GS_WARPS;    // warps per CTA
-
-// One stage = kGsRows contiguous rows of X (a single 16-B aligned bulk copy whatever K is,
-// because a stage starts at a multiple of 8 rows) followed by the three weight rows.
-__host__ __device__ inline size_t gram_small_stage_elems(int K) {
-  return (size_t)kGsRows * K + 3 * kGsRows;
-}
-__host__ __device__ inline size_t gram_small_smem(int K, int NT) {
-  size_t ring = sizeof(double) * kGsWarps * kGsStages * gram_small_stage_elems(K) +
-                sizeof(unsigned long long) * kGsWarps * kGsStages;
-  size_t red = sizeof(double) * (size_t)kGsWarps * NT * 64;
-  return ring > red ? ring : red;
-}
 
 // ---- mbarrier + bulk async copy (TMA, SASS UBLKCP) ------------------------------------------
 __device__ __forceinline__ unsigned smem_u32(const void* p) {
@@ -113,227 +80,7 @@ __device__ __forceinline__ double vmul(double a, double b) {
   return v;
 }
 
-// part: (gridDim.x, NT, 64) with NT = T2 (T2+1) / 2, tile (i <= j) at slot j (j+1)/2 + i,
-// element (r, c) of a tile at r * 8 + c.  Wabc: rows a, b, c of the weight matrix, row stride
-// ldw (even, so every stage of a weight row is 16-B aligned).  X must be 16-B aligned.
-template <int T2, int T0, bool HAS_M>
-__global__ void __launch_bounds__(32 * kGsWarps, LRVB_GS_MINB)
-k_gram_small(const double* __restrict__ X, const double* __restrict__ Wabc,
-             double* __restrict__ part, int64_t N, int64_t ldw, int K) {
-  pdl_sync();
-  constexpr int TS = HAS_M ? T0 : -1;        // straddle tile
-  constexpr int TB = HAS_M ? T0 + 1 : T0;    // first pure-s tile
-  constexpr int NT = T2 * (T2 + 1) / 2;
-  extern __shared__ __align__(16) double sm[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int lr = lane & 3, lc = lane >> 2;
-  const int stage_elems = kGsRows * K + 3 * kGsRows;
-  double* ring = sm + (size_t)warp * kGsStages * stage_elems;
-  unsigned long long* bars =
-      reinterpret_cast<unsigned long long*>(sm + (size_t)kGsWarps * kGsStages * stage_elems) +
-      warp * kGsStages;
-  const unsigned ring_u = smem_u32(ring), bars_u = smem_u32(bars);
-  if (lane == 0) {
-#pragma unroll
-    for (int p = 0; p < kGsStages; ++p) mbar_init(bars_u + 8 * p, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-  }
-  __syncwarp();
-
-  // per-lane column of every packed tile: offset inside the staged x row, class, validity
-  int off[T2];
-  bool valid_last = true, cls1 = false, valid_m = true;
-#pragma unroll
-  for (int t = 0; t < T2; ++t) {
-    const int col = 8 * t + lc;
-    int o = col;
-    if (t >= TB || (t == TS && col >= K)) o = col - K;
-    const bool ok = col < 2 * K;
-    if (t == TS) { cls1 = col >= K; valid_m = ok; }
-    if (t == T2 - 1) valid_last = ok;
-    off[t] = (ok ? o : 0) + lr * K;
-  }
-
-  double acc[NT][2];
-#pragma unroll
-  for (int t = 0; t < NT; ++t) acc[t][0] = acc[t][1] = 0.0;
-  constexpr int KSTEPS = kGsRows / 4;
-
-  const int64_t nstage = (N + kGsRows - 1) / kGsRows;
-  const int64_t nfull = N / kGsRows;          // stages before nfull are complete
-  const int64_t tw = (int64_t)gridDim.x * kGsWarps;
-  const int64_t gw = (int64_t)blockIdx.x * kGsWarps + warp;
-  const unsigned xbytes = (unsigned)(kGsRows * K * sizeof(double));
-  const unsigned wbytes = (unsigned)(kGsRows * sizeof(double));
-
-  // complete stages arrive by four bulk copies (X rows, a, b, c) tracked by the slot's mbarrier;
-  // the ragged last stage is filled by the warp itself when it is consumed
-  auto issue = [&](int64_t s, int slot) {
-    if (s < nfull && lane < 4) {
-      const unsigned bar = bars_u + 8 * slot;
-      const unsigned dst = ring_u + (unsigned)(slot * stage_elems * sizeof(double));
-      const int64_t n0 = s * kGsRows;
-      if (lane == 0) {
-        mbar_arrive_expect_tx(bar, xbytes + 3 * wbytes);
-        bulk_g2s(dst, X + n0 * K, xbytes, bar);
-      } else {
-        bulk_g2s(dst + xbytes + (lane - 1) * wbytes, Wabc + (int64_t)(lane - 1) * ldw + n0, wbytes, bar);
-      }
-    }
-  };
-
-  // make stage s readable in `slot`: bulk stages complete on the slot's mbarrier, the ragged
-  // last stage is filled here by the warp itself
-  auto acquire = [&](int64_t s, int slot, unsigned ph) {
-    if (s < nfull) {
-      mbar_wait(bars_u + 8 * slot, ph);
-    } else {
-      double* xs = ring + (size_t)slot * stage_elems;
-      double* ws = xs + kGsRows * K;
-      const int64_t n0 = s * kGsRows;
-      const int rows = (int)(N - n0);
-      for (int e = lane; e < kGsRows * K; e += 32) xs[e] = (e < rows * K) ? X[n0 * K + e] : 0.0;
-      for (int e = lane; e < 3 * kGsRows; e += 32) {
-        const int f = e / kGsRows, r = e % kGsRows;
-        ws[e] = (r < rows) ? Wabc[(int64_t)f * ldw + n0 + r] : 0.0;
-      }
-      __syncwarp();
-    }
-  };
-
-#pragma unroll
-  for (int p = 0; p < kGsStages; ++p) issue(gw + p * tw, p);
-
-  // Software pipeline over the flat sequence of k-steps: the shared-memory loads of the next
-  // k-step (of the next stage at a stage boundary, after its mbarrier) are in flight while the
-  // FP64 pipe works on the current one; the DMULs of a k-step are issued as one group ahead of
-  // its DMMAs (volatile asm pins the order); a slot is refilled as soon as its last rows are in
-  // registers.
-  int slot = 0;
-  unsigned phase = 0;
-  int64_t s = gw;
-  // The refill of a consumed slot is the expensive part of a stage boundary.  The warps that
-  // share an SM sub-partition advance in lockstep (round-robin issue), so each of them postpones
-  // its refill by a different number of k-steps: while one warp issues copies the others feed
-  // the FP64 pipe.
-  const int refill_ks = (LRVB_GS_STAGGER ? (warp >> 2) : 0) % KSTEPS;
-  int pend_slot = -1;
-  int64_t pend_stage = 0;
-  double raw[T2], wv[3];
-  if (s < nstage) {
-    acquire(s, 0, 0);
-#pragma unroll
-    for (int t = 0; t < T2; ++t) raw[t] = lds_f64(ring_u + 8 * off[t]);
-#pragma unroll
-    for (int f = 0; f < 3; ++f) wv[f] = lds_f64(ring_u + 8 * (kGsRows * K + f * kGsRows + lr));
-  }
-  while (s < nstage) {
-    const int64_t sn = s + tw;
-    const int nslot = (slot + 1 == kGsStages) ? 0 : slot + 1;
-    const unsigned nphase = (nslot == 0) ? (phase ^ 1u) : phase;
-    const unsigned xs_u = ring_u + (unsigned)(slot * stage_elems * sizeof(double));
-    const unsigned ws_u = xs_u + 8 * (kGsRows * K + lr);
-#pragma unroll
-    for (int ks = 0; ks < KSTEPS; ++ks) {
-      double nraw[T2], nwv[3];
-      if (ks + 1 < KSTEPS) {
-#pragma unroll
-        for (int t = 0; t < T2; ++t) nraw[t] = lds_f64(xs_u + 8 * (off[t] + 4 * (ks + 1) * K));
-#pragma unroll
-        for (int f = 0; f < 3; ++f) nwv[f] = lds_f64(ws_u + 8 * (f * kGsRows + 4 * (ks + 1)));
-      } else if (sn < nstage) {
-        acquire(sn, nslot, nphase);
-        const unsigned nx_u = ring_u + (unsigned)(nslot * stage_elems * sizeof(double));
-#pragma unroll
-        for (int t = 0; t < T2; ++t) nraw[t] = lds_f64(nx_u + 8 * off[t]);
-#pragma unroll
-        for (int f = 0; f < 3; ++f) nwv[f] = lds_f64(nx_u + 8 * (kGsRows * K + f * kGsRows + lr));
-      } else {
-#pragma unroll
-        for (int t = 0; t < T2; ++t) nraw[t] = 0.0;
-        nwv[0] = nwv[1] = nwv[2] = 0.0;
-      }
-      const double wa = wv[0], wb = wv[1], wc = wv[2];
-      double z[T2], bw0[T2], bc[T2];
-#pragma unroll
-      for (int t = 0; t < T2; ++t) {
-        double x = raw[t];
-        if (t == TS) {
-          const double xx = vmul(x, x);
-          x = cls1 ? xx : x;
-          if (!valid_m) x = 0.0;
-        } else if (t >= TB) {
-          x = vmul(x, x);
-          if (t == T2 - 1 && !valid_last) x = 0.0;
-        }
-        z[t] = x;
-      }
-      double aw2 = 0.0;
-      if (HAS_M) aw2 = vmul(z[HAS_M ? TS : 0], cls1 ? wc : wb);
-#pragma unroll
-      for (int j = 0; j < T2; ++j) {
-        bw0[j] = bc[j] = 0.0;
-        if (T0 > 0 || j == TS) bw0[j] = vmul(z[j], (j < T0) ? wa : ((j == TS) ? (cls1 ? wb : wa) : wb));
-        if (j >= TB) bc[j] = vmul(z[j], wc);
-      }
-      const double zm0 = (HAS_M && !cls1) ? z[HAS_M ? TS : 0] : 0.0;
-      const double zm1 = (HAS_M && cls1) ? z[HAS_M ? TS : 0] : 0.0;
-      if (ks == refill_ks && pend_slot >= 0) {
-        // the previous slot's last rows were consumed a k-step (or more) ago: refill it
-        __syncwarp();
-        issue(pend_stage, pend_slot);
-        pend_slot = -1;
-      }
-#pragma unroll
-      for (int j = 0; j < T2; ++j) {
-        const int base = j * (j + 1) / 2;
-#pragma unroll
-        for (int i = 0; i < T0; ++i)
-          if (i <= j) dmma884(acc[base + i][0], acc[base + i][1], z[i], bw0[j]);
-        if (HAS_M && j == TS) {
-          dmma884(acc[base + j][0], acc[base + j][1], zm0, bw0[j]);
-          dmma884(acc[base + j][0], acc[base + j][1], zm1, aw2);   // s rows: (.|c s) columns
-        }
-        if (HAS_M && j > TS)
-          dmma884(acc[base + (HAS_M ? TS : 0)][0], acc[base + (HAS_M ? TS : 0)][1], aw2, z[j]);
-#pragma unroll
-        for (int i = TB; i < T2; ++i)
-          if (i <= j) dmma884(acc[base + i][0], acc[base + i][1], z[i], bc[j]);
-      }
-#pragma unroll
-      for (int t = 0; t < T2; ++t) raw[t] = nraw[t];
-#pragma unroll
-      for (int f = 0; f < 3; ++f) wv[f] = nwv[f];
-    }
-    pend_slot = slot;
-    pend_stage = s + (int64_t)kGsStages * tw;
-    s = sn;
-    slot = nslot;
-    phase = nphase;
-  }
-  __syncthreads();
-
-  // every warp parks its accumulators in shared memory, then the CTA sums them in a fixed
-  // order: one partial per CTA
-  double* red = sm;
-  const int e0 = (lane >> 2) * 8 + 2 * (lane & 3);
-#pragma unroll
-  for (int t = 0; t < NT; ++t) {
-    double* d = red + ((size_t)warp * NT + t) * 64 + e0;
-    d[0] = acc[t][0];
-    d[1] = acc[t][1];
-  }
-  __syncthreads();
-  double* out = part + (size_t)blockIdx.x * NT * 64;
-  for (int e = threadIdx.x; e < NT * 64; e += blockDim.x) {
-    double v = 0.0;
-#pragma unroll
-    for (int w = 0; w < kGsWarps; ++w) v += red[(size_t)w * NT * 64 + e];
-    out[e] = v;
-  }
-}
-
-// shape of the packed tile grid for a given K (K <= 20)
+// shape of the packed tile grid for a given K
 struct GramSmallShape {
   int T2, T0, has_m, NT;
 };
@@ -344,34 +91,6 @@ inline GramSmallShape gram_small_shape(int K) {
   s.has_m = (K % 8) != 0;
   s.NT = s.T2 * (s.T2 + 1) / 2;
   return s;
-}
-
-// launch the instantiation for K; returns false when K is outside the small-K range
-inline bool launch_gram_small(const double* X, const double* Wabc, double* part, int64_t N,
-                              int64_t ldw, int K, int grid, cudaStream_t st) {
-  const GramSmallShape s = gram_small_shape(K);
-  if (K > 20 || (ldw & 1) || (((uintptr_t)X) & 15) || (((uintptr_t)Wabc) & 15)) return false;
-  const size_t smem = gram_small_smem(K, s.NT);
-#define LRVB_GS(T2_, T0_, M_)                                                                 \
-  if (s.T2 == T2_ && s.T0 == T0_ && s.has_m == (M_ ? 1 : 0)) {                                \
-    static size_t configured = 48 * 1024;                                                    \
-    if (smem > configured) {                                                                 \
-      cudaFuncSetAttribute(k_gram_small<T2_, T0_, M_>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                           (int)smem);                                                       \
-      configured = smem;                                                                     \
-    }                                                                                        \
-    return launch_pdl(k_gram_small<T2_, T0_, M_>, dim3(grid), dim3(32 * kGsWarps), smem, st, X, Wabc, \
-                      part, N, ldw, K) == cudaSuccess;                                         \
-  }
-  LRVB_GS(1, 0, true)
-  LRVB_GS(2, 0, true)
-  LRVB_GS(2, 1, false)
-  LRVB_GS(3, 1, true)
-  LRVB_GS(4, 1, true)
-  LRVB_GS(4, 2, false)
-  LRVB_GS(5, 2, true)
-#undef LRVB_GS
-  return false;
 }
 
 }  // namespace lrvb

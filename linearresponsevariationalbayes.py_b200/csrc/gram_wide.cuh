@@ -1,5 +1,5 @@
-// Weighted Grams of the beta block for LARGE K (K >= 96, K % 8 == 0; default K = 176 .. 240; BASELINE configs[3]:
-// K = 200) on the FP64 tensor cores (DMMA.8x8x4), sm_100a.
+// Weighted Grams of the beta block for LARGE K (K % 8 == 0, K = 176 .. 240; BASELINE configs[3]: K = 200) on the
+// FP64 tensor cores (DMMA.8x8x4), sm_100a.  The planner covers every K >= 96 with K % 8 == 0.
 //
 // Same packed formulation as gram_small / gram_mid / gram_big: one weighted Gram of z_n = [x_n | s_n]
 // (2K columns, T2 = K/4 tiles of 8), upper triangle only; with K % 8 == 0 no tile straddles the x | s
@@ -75,7 +75,9 @@ struct GwPlan {
 inline size_t gram_wide_smem(int ZS, int TN) {
   return sizeof(double) * kGwBuffers * (size_t)TN * (ZS + 3) + 64;
 }
-inline bool gram_wide_eligible(int K) { return K >= 96 && K % 8 == 0 && K <= kMaxK; }
+// where it beats the rectangle kernel (profiles/r02_gram_wide.md: 56 - 66 % against 49 - 55 % of the DMMA peak
+// for K = 176 .. 240; below, the 4-tile blocks starve the warps and the staged bytes per DMMA grow)
+inline bool gram_wide_eligible(int K) { return K >= 176 && K <= 240 && K % 8 == 0; }
 
 inline GwPlan gram_wide_plan(int K) {
   GwPlan pl;

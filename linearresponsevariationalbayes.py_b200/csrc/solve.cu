@@ -610,62 +610,10 @@ k_spd_inverse_reg(double* __restrict__ S, int n, int* __restrict__ info) {
   if (tid == 0) *info = bad;
 }
 
-// ---- in-place inverse of a small SPD matrix (Gauss-Jordan sweeps, one CTA) ---------------------
-// No pivoting is needed for SPD input; a non-positive pivot aborts with info = its index + 1.
-__global__ void __launch_bounds__(1024)
-k_spd_inverse(double* __restrict__ S, int n, int* __restrict__ info, int use_smem) {
-  pdl_sync();
-  extern __shared__ double sm[];
-  double* row = sm;        // n   scaled pivot row
-  double* col = sm + n;    // n   pivot column
-  double* M = use_smem ? sm + 2 * n : S;
-  const int tid = threadIdx.x, nt = blockDim.x;
-  if (use_smem)
-    for (int i = tid; i < n * n; i += nt) M[i] = S[i];
-  __syncthreads();
-  // thread -> (row stripe i0 + k TI, column lane jj): no integer division in the sweep, the pivot
-  // column entry of a row stays in a register; every thread sees the same pivot, so the
-  // "not positive definite" exit is uniform and needs no shared flag (two barriers per pivot)
-  const int TJ = 8, TI = nt / TJ;
-  const int i0 = tid / TJ, jj = tid - i0 * TJ;
-  int bad = 0;
-  for (int k = 0; k < n; ++k) {
-    const double d = M[(size_t)k * n + k];
-    if (!(d > 0.0)) {
-      bad = k + 1;
-      break;
-    }
-    const double pinv = 1.0 / d;
-    for (int j = tid; j < n; j += nt) {
-      row[j] = M[(size_t)k * n + j] * pinv;
-      col[j] = M[(size_t)j * n + k];
-    }
-    __syncthreads();
-    for (int i = i0; i < n; i += TI) {
-      double* mi = M + (size_t)i * n;
-      if (i == k) {
-        for (int j = jj; j < n; j += TJ) mi[j] = (j == k) ? pinv : row[j];
-      } else {
-        const double ci = col[i];
-        for (int j = jj; j < n; j += TJ) mi[j] = (j == k) ? -ci * pinv : fma(-ci, row[j], mi[j]);
-      }
-    }
-    __syncthreads();
-  }
-  if (use_smem && !bad)
-    for (int i = tid; i < n * n; i += nt) S[i] = M[i];
-  if (tid == 0) *info = bad;
-}
-
-// ---- 128 < n <= 234: symmetric sweeps on the packed lower triangle in shared memory ---------------
-// The full n x n matrix no longer fits in shared memory beyond n = 167, its lower triangle does up
-// to n = 234 (K = 115).  The sweep operator keeps the matrix symmetric at every step:
-//   SWP(k):  A_kk <- -1 / A_kk,   A_ik <- A_ik / A_kk,   A_ij <- A_ij - A_ik A_jk / A_kk   (i, j != k)
-// and after all n sweeps A = -S^-1.  Two barriers per pivot, every element touched once per pivot.
 // ---- SPD inverse on many CTAs: blocked Gauss-Jordan sweeps (n > kSpdBlockedMin) ------------------------
 // (profiles/r02_spd_inverse_blocked.log)
-// The one-CTA kernels above are bound by one SM (its registers up to n = 128, its shared memory up to 234,
-// global memory beyond: 5.5 ms at n = 264, ~20 ms at n = 404 = the LRVB covariance of K = 200).  Here the
+// A one-CTA inverse is bound by one SM (its registers up to n = 128, its shared memory up to 234, global
+// memory beyond: 5.5 ms at n = 264, ~20 ms at n = 404 = the LRVB covariance of K = 200).  Here the
 // matrix is cut into 32 x 32 tiles and pivot block kb is swept by ONE launch of T x T CTAs, out of place
 // (X -> Y, two buffers in turn; the matrix is at most 2 MB, so it lives in the L2):
 //     Y_kk = P^-1        Y_kj = P^-1 X_kj        Y_ik = -X_ik P^-1        Y_ij = X_ij - X_ik P^-1 X_kj
@@ -777,55 +725,6 @@ k_spd_gj_finish(const double* Z, double* S, int n) {
   const double v = 0.5 * (Z[(size_t)i * n + j] + Z[(size_t)j * n + i]);
   S[(size_t)i * n + j] = v;
   S[(size_t)j * n + i] = v;
-}
-
-constexpr int kSpdPackedMax = 234;
-// One SM's shared-memory bandwidth bounds this kernel (every element is read and written once per
-// pivot: ~n^2 / 2 * 24 B at 128 B / clock); rows are striped over groups of 8 lanes so that the pivot
-// column entry of a row is fetched once per row (a flat element-per-thread mapping, perfectly balanced,
-// measured 15 % slower because it fetches two column entries per element).
-__global__ void __launch_bounds__(1024)
-k_spd_inverse_packed(double* __restrict__ S, int n, int* __restrict__ info) {
-  pdl_sync();
-  extern __shared__ double sm[];
-  double* __restrict__ col = sm;            // n   pivot column A_ik (all i)
-  double* __restrict__ A = sm + n;          // n (n + 1) / 2, row-major lower triangle: (i, j <= i) at i (i + 1) / 2 + j
-  const int tid = threadIdx.x, nt = blockDim.x;
-  for (int i = tid >> 3; i < n; i += nt >> 3)
-    for (int j = tid & 7; j <= i; j += 8) A[i * (i + 1) / 2 + j] = S[(size_t)i * n + j];
-  __syncthreads();
-  const int TJ = 8, TI = nt / TJ;
-  const int i0 = tid / TJ, jj = tid - i0 * TJ;
-  int bad = 0;
-  for (int k = 0; k < n; ++k) {
-    const double d = A[k * (k + 1) / 2 + k];
-    if (!(d > 0.0)) {          // uniform: every thread reads the same pivot
-      bad = k + 1;
-      break;
-    }
-    for (int i = tid; i < n; i += nt) col[i] = (i >= k) ? A[i * (i + 1) / 2 + k] : A[k * (k + 1) / 2 + i];
-    __syncthreads();
-    const double pinv = 1.0 / d;
-    for (int i = i0; i < n; i += TI) {
-      double* __restrict__ ai = A + i * (i + 1) / 2;
-      const double ci = col[i] * pinv;
-      if (i == k) {
-        for (int j = jj; j <= i; j += TJ) ai[j] = (j == k) ? -pinv : col[j] * pinv;
-      } else {
-#pragma unroll 4
-        for (int j = jj; j <= i; j += TJ) ai[j] = (j == k) ? ci : fma(-ci, col[j], ai[j]);
-      }
-    }
-    __syncthreads();
-  }
-  if (!bad)
-    for (int i = tid >> 3; i < n; i += nt >> 3)
-      for (int j = tid & 7; j <= i; j += 8) {
-        const double v = -A[i * (i + 1) / 2 + j];
-        S[(size_t)i * n + j] = v;
-        S[(size_t)j * n + i] = v;
-      }
-  if (tid == 0) *info = bad;
 }
 
 // ---- direct solve by block elimination -----------------------------------------------------------
@@ -1222,7 +1121,7 @@ int lrvb_spd_inverse(double* S_dev, int32_t n, int32_t* info_host, void* stream)
   // memory at every synchronisation)
   int* dinfo = nullptr;
   double* scratch = nullptr;        // second matrix buffer of the blocked sweeps: 8 per device, round-robin
-  const bool blocked = n > kSpdBlockedMin && !(getenv("LRVB_SPD_BLOCKED") && getenv("LRVB_SPD_BLOCKED")[0] == '0');
+  const bool blocked = n > kSpdBlockedMin;
   {
     static std::mutex mu;
     static int* words[64] = {nullptr};          // per device: 64 ints
@@ -1241,12 +1140,6 @@ int lrvb_spd_inverse(double* S_dev, int32_t n, int32_t* info_host, void* stream)
       scratch = bufs[dev] + (size_t)(slot & 7u) * nmax * nmax;
     }
   }
-  size_t smem = sizeof(double) * (2 * (size_t)n + (size_t)n * n);
-  int use_smem = 1;
-  if (smem > 200 * 1024) {
-    use_smem = 0;
-    smem = sizeof(double) * 2 * (size_t)n;
-  }
   if (blocked) {
     const int T = (n + 31) / 32;
     LRVB_CUDA(cudaMemsetAsync(dinfo, 0, sizeof(int), st));
@@ -1258,7 +1151,7 @@ int lrvb_spd_inverse(double* S_dev, int32_t n, int32_t* info_host, void* stream)
     }
     LRVB_CUDA(launch_pdl(k_spd_gj_finish, dim3((n + 15) / 16, (n + 15) / 16), dim3(256), 0, st, (const double*)cur,
                          S_dev, (int)n));
-  } else if (n <= 128) {
+  } else {
     const int threads = 8 * ((n + 3) / 4 * 4);     // whole warps: 4 rows of 8 lanes each
     const int nq = (n + 7) / 8;
     cudaError_t le;
@@ -1270,13 +1163,6 @@ int lrvb_spd_inverse(double* S_dev, int32_t n, int32_t* info_host, void* stream)
     else LRVB_SPD(16);
 #undef LRVB_SPD
     LRVB_CUDA(le);
-  } else if (n <= kSpdPackedMax && !(getenv("LRVB_SPD_PACKED") && getenv("LRVB_SPD_PACKED")[0] == '0')) {
-    const size_t psm = sizeof(double) * ((size_t)n + (size_t)n * (n + 1) / 2);
-    cudaFuncSetAttribute(k_spd_inverse_packed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm);
-    LRVB_CUDA(launch_pdl(k_spd_inverse_packed, dim3(1), dim3(1024), psm, st, S_dev, (int)n, dinfo));
-  } else {
-    cudaFuncSetAttribute(k_spd_inverse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    LRVB_CUDA(launch_pdl(k_spd_inverse, dim3(1), dim3(1024), smem, st, S_dev, n, dinfo, use_smem));
   }
   cudaError_t e = cudaGetLastError();
   if (e == cudaSuccess) e = cudaMemcpyAsync(info_host, dinfo, sizeof(int), cudaMemcpyDeviceToHost, st);

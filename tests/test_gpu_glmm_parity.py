@@ -57,11 +57,13 @@ CASES = {
     "k77_team8": dict(N=1101, K=77, G=11, Q=4, seed=36),
     "k104_team8_ring_wrap": dict(N=30011, K=104, G=30, Q=4, seed=37),
     "k72_team4_ring_wrap": dict(N=40009, K=72, G=40, Q=4, seed=46, weights=True),
-    # k_gram_wide (K >= 112, K % 8 == 0): blocks of 5,5,4 tiles (mixed 5x4 / 4x5 / 4x4 jobs), of 5 only, of 4
-    # only (K = 128); ragged last stage; enough rows that every CTA's 3-slot ring wraps
-    "k112_wide": dict(N=2503, K=112, G=20, Q=4, seed=38, weights=True),
-    "k120_wide": dict(N=1999, K=120, G=20, Q=4, seed=39),
-    "k128_wide_ring_wrap": dict(N=40013, K=128, G=40, Q=4, seed=40),
+    # k_gram_wide (K = 176 .. 240, K % 8 == 0): blocks of 5,5,4,4,4 tiles (K = 176: mixed 5x4 / 4x5 / 4x4 jobs),
+    # of 5 only (K = 200, 240); ragged last stage; enough rows that every CTA's 3-slot ring wraps:
+    # gram_wide_plan(192) deals 7 job groups of 28 - 60-row stages to 19 - 24 CTAs each, at most 19 CTAs x 60
+    # rows = 1140 rows per round of stages, so N = 12007 gives every CTA >= 10 stages
+    "k176_wide": dict(N=2503, K=176, G=20, Q=4, seed=38, weights=True),
+    "k240_wide": dict(N=2003, K=240, G=20, Q=4, seed=39),
+    "k192_wide_ring_wrap": dict(N=12007, K=192, G=40, Q=4, seed=40),
     "k200_wide_ragged": dict(N=3010, K=200, G=30, Q=4, seed=41, ragged=True, weights=True),
     "k184_wide_default": dict(N=2400, K=184, G=24, Q=4, seed=42),
     # wide-model observation kernel (K > 62): node slots with unequal node counts (Q = 6: 2, 2, 1, 1), an empty
@@ -76,17 +78,7 @@ CASES = {
 def setup(request, vb):
     case = make_case(**CASES[request.param])
     oracle = make_oracle(case)
-    # the "_wide" cases force k_gram_wide (default only for K = 176 .. 240) so that its mixed block sizes are
-    # covered; the switch is read when the handle is created
-    import os
-    forced = "_wide" in request.param
-    if forced:
-        os.environ["LRVB_GRAM_WIDE"] = "1"
-    try:
-        model = make_model(vb, case)
-    finally:
-        if forced:
-            os.environ.pop("LRVB_GRAM_WIDE", None)
+    model = make_model(vb, case)
     obj = vb.Objective(model.glmm_par, model)
     return case, oracle, model, obj
 

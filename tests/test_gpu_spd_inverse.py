@@ -1,10 +1,10 @@
 """lrvb_spd_inverse (the role of cho_solve(cho_factor(H), .) in ModelSensitivity.py:594-602) against
-numpy.linalg.inv for every kernel variant: register-resident (n <= 104), blocked multi-CTA sweeps (n > 104,
-ragged and full tiles up to the largest n the library accepts), and the one-CTA kernels they replace
-(LRVB_SPD_BLOCKED=0).  Tolerance: 1e-9 relative to the largest entry (the covariance tolerance of the north
-star); `info` = first non-positive leading minor, as a Cholesky factorisation reports it."""
+numpy.linalg.inv for both kernels: register-resident (n <= 104) and blocked multi-CTA sweeps (n > 104, ragged
+and full tiles up to the largest n the library accepts).  Tolerance: 1e-9 relative to the largest entry (the
+covariance tolerance of the north star).  The blocked sweeps are also held to 1e-10 of a Gauss-Jordan inverse
+in extended precision (np.longdouble, a 64-bit mantissa on x86-64), whose residual |R S - I| stays near 1e-17
+on these matrices.  `info` = first non-positive leading minor, as a Cholesky factorisation reports it."""
 import ctypes
-import os
 
 import numpy as np
 import pytest
@@ -43,15 +43,28 @@ def test_inverse_matches_numpy(n):
         assert np.abs(got - got.T).max() <= 1e-13 * np.abs(want).max()
 
 
+def _inverse_longdouble(S):
+    """In-place Gauss-Jordan sweeps without pivoting (S is SPD) in np.longdouble."""
+    M = S.astype(np.longdouble)
+    for k in range(M.shape[0]):
+        p = 1 / M[k, k]
+        r = M[k] * p
+        c = M[:, k].copy()
+        M -= np.outer(c, r)
+        M[k] = r
+        M[:, k] = -c * p
+        M[k, k] = p
+    return M
+
+
 @pytest.mark.parametrize("n", [128, 204, 404])
-def test_blocked_equals_one_cta_kernels(n, monkeypatch):
+def test_blocked_matches_longdouble_reference(n):
     S = _spd(n, 3 * n)
     S = 0.5 * (S + S.T)
-    a, ia = _inverse(S)
-    monkeypatch.setenv("LRVB_SPD_BLOCKED", "0")
-    b, ib = _inverse(S)
-    assert ia == 0 and ib == 0
-    assert np.abs(a - b).max() <= 1e-10 * np.abs(b).max()
+    got, info = _inverse(S)
+    assert info == 0
+    ref = _inverse_longdouble(S)
+    assert np.abs(got - ref).max() <= 1e-10 * np.abs(ref).max()
 
 
 @pytest.mark.parametrize("n,k", [(40, 17), (100, 1), (130, 33), (130, 70), (300, 290), (404, 129)])

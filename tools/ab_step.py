@@ -1,4 +1,4 @@
-"""Quick device-step timing of one workload (A/B of library builds / env switches): prints ms per step,
+"""Quick device-step timing of one workload (A/B of library builds): prints ms per step,
 per-kernel times, and checks the result against a reference build if LRVB_AB_REF is set."""
 import os, sys, ctypes
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -39,6 +39,6 @@ for i in range(8):
         ev.append(ms3[0]); ob.append(ms3[1]); gr.append(ms3[2])
 A, B, L = model.blocks()
 chk = float(A.abs().sum() + B.abs().sum() + L.abs().sum() + model.kl_tensor().abs() + model.grad_tensor().abs().sum())
-print("%s lib=%s FUSED=%s WARPS=%s: step %.4f ms (min %.4f) eval %.4f obs/onepass %.4f gram %.4f  checksum %.15e" % (
-    sys.argv[1] if len(sys.argv) > 1 else "c2", os.path.basename(nat.LIB_PATH), os.environ.get("LRVB_FUSED", "1"),
-    os.environ.get("LRVB_TEAM_WARPS", "auto"), np.mean(ts), np.min(ts), np.mean(ev), np.mean(ob), np.mean(gr), chk))
+print("%s lib=%s: step %.4f ms (min %.4f) eval %.4f obs/onepass %.4f gram %.4f  checksum %.15e" % (
+    sys.argv[1] if len(sys.argv) > 1 else "c2", os.path.basename(nat.LIB_PATH), np.mean(ts), np.min(ts), np.mean(ev),
+    np.mean(ob), np.mean(gr), chk))
