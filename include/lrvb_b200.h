@@ -263,6 +263,21 @@ int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cro
  * bitwise equal.  LRVB_EINVAL for NULL pointers; uses the scratch of lrvb_glmm_predict_lr. */
 int lrvb_glmm_loo(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
                   double* out_dev, void* stream);
+/* Approximate leave-one-group-out cross-validation and group influence by the infinitesimal jackknife, at the cached
+ * Hessian (an order-2 evaluation in free coordinates, normally at the optimum; LRVB_ESTATE otherwise).  Dropping
+ * group g (w_n -> 0 on its rows) shifts the globals by delta_g = -S^-1 (v_glob - B_g^T L_g^-1 v_loc), v = the group's
+ * data gradient from W rows 0, 1 (lrvb_glmm_obs_weights).  Sinv_dev = S^-1 (Dg,Dg), Pinv_dev = the inverse of its
+ * (K,K) block on E[beta].  Output:
+ *   delta_dev     (G, Dg) row-major: delta_g
+ *   group_out_dev (2, G)  row-major: [cook_g = delta_beta,g^T P^-1 delta_beta,g / K, elpd_logo_group]
+ *   row_out_dev   (3, N)  row-major, the handle's (group-sorted) row order: [lpd_logo, eta_mean_logo, eta_var_logo]
+ * with the globals at theta + delta_g mapped exactly to constrained values, q(u_g) at its optimum without the group's
+ * rows (mean E[mu]', info max(E[tau]', lb_u)), eta = u_g + x.beta under that q and lpd_logo = log E_q[p(y_n | eta)]
+ * by the model's Gauss-Hermite rule (y = 0 as log E[sigma(-eta)]).  An empty group gets delta = 0, cook = 0 and
+ * elpd_logo_group = 0.  No atomics: repeated calls are bitwise equal.  LRVB_EINVAL for NULL pointers; allocates a
+ * (G, Dg) scratch in the handle on first use. */
+int lrvb_glmm_logo(lrvb_glmm* h, const double* Sinv_dev, const double* Pinv_dev, double* delta_dev,
+                   double* group_out_dev, double* row_out_dev, void* stream);
 
 /* ---- batched exponential-family terms (ExponentialFamilies.py) --------------------------
  * All pointers dev; M = number of factors. */

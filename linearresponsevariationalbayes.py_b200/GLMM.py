@@ -55,6 +55,18 @@ without row n, and the moments eta_mean_loo, eta_var_loo of eta = u_g + x.beta t
 eta_var_loo where the shifted variance is <= 0).  Scalars: elpd_loo = sum lpd_loo, p_loo = sum lpd - elpd_loo,
 elpd_loo_se = sqrt(N) std(lpd_loo, ddof=1) (NaN when n_invalid > 0), n_invalid = rows with NaN."""
 
+ApproximateLOGO = namedtuple("ApproximateLOGO", ["lpd_logo", "eta_mean_logo", "eta_var_logo", "elpd_logo_group",
+                                                 "cooks_distance", "delta_global", "elpd_logo", "elpd_logo_se"])
+ApproximateLOGO.__doc__ = """Approximate leave-one-group-out cross-validation and group influence by the infinitesimal
+jackknife (``LogisticGLMM.approximate_logo``, ``LinearResponseCovariances.get_approximate_logo``).  Per row (N,), in
+the caller's row order: lpd_logo = log E_q[p(y_n | eta)] with the globals at the IJ estimate of the fit without the
+row's group and q(u_g) at its optimum without the group's rows (mean E[mu], info max(E[tau], lb)), and the moments
+eta_mean_logo, eta_var_logo of eta = u_g + x.beta there.  Per group (G,): elpd_logo_group = the sum of lpd_logo over
+the group's rows, cooks_distance = delta_beta^T P^-1 delta_beta / K (P = the LRVB covariance of E[beta]) and
+delta_global (G, Dg) = the IJ shift of the global free parameters.  Scalars: elpd_logo = sum lpd_logo, elpd_logo_se =
+sqrt(G') std(elpd_logo_group over the G' non-empty groups, ddof=1) (NaN when G' < 2).  An empty group has zero
+delta_global, cooks_distance and elpd_logo_group."""
+
 
 class _DevView(object):
     """Zero-copy torch view of library-owned device memory (__cuda_array_interface__)."""
@@ -852,6 +864,30 @@ class LogisticGLMM(object):
         elpd = float(lpd_loo.sum())
         se = float(lpd_loo.std(correction=1)) * np.sqrt(self.N) if self.N > 1 else float("nan")
         return ApproximateLOO(lpd, lpd_loo, out[2], out[3], elpd, se, float(lpd.sum()) - elpd, n_invalid)
+
+    def approximate_logo(self, Sinv):
+        """Approximate leave-one-group-out cross-validation and group influence by the infinitesimal jackknife at the
+        cached Hessian (normally the optimum), given S^-1 (``global_covariance``).  Dropping group g is w_n -> 0 on
+        its rows; the globals move by delta_g = -S^-1 (v_glob - B_g^T L_g^-1 v_loc) (v = the group's data gradient),
+        all groups in three device passes (csrc/logo.cu).  Returns an ``ApproximateLOGO`` with CUDA tensors (rows in
+        the caller's order) and Python scalars."""
+        torch = nat.require_cuda()
+        self._check_binary_y()
+        Pinv = self.spd_inverse_(Sinv[4:4 + self.K, 4:4 + self.K].clone())
+        delta = torch.empty(self.G, self.Dg, dtype=torch.float64, device=self.device)
+        grp = torch.empty(2, self.G, dtype=torch.float64, device=self.device)
+        out = torch.empty(3, self.N, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_logo(self._h, nat.ptr(Sinv), nat.ptr(Pinv), nat.ptr(delta), nat.ptr(grp),
+                                           nat.ptr(out), nat.stream_ptr()))
+        if self.perm is not None:
+            res = torch.empty_like(out)
+            res.index_copy_(1, to_device(self.perm, torch.int64), out)
+            out = res
+        if getattr(self, "_group_nonempty", None) is None:
+            self._group_nonempty = torch.bincount(self.g.to(torch.int64), minlength=self.G) > 0
+        fold = grp[1][self._group_nonempty]
+        se = float(fold.std(correction=1)) * np.sqrt(fold.numel()) if fold.numel() > 1 else float("nan")
+        return ApproximateLOGO(out[0], out[1], out[2], grp[1], grp[0], delta, float(out[0].sum()), se)
 
     def prediction_jacobian(self, free, X_new, groups_new, quantity="prob"):
         """d prob / d free (or d eta / d free) of new rows as scipy CSR (M, D): a x on beta.mean, b x~ on

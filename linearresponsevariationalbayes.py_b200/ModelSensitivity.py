@@ -223,6 +223,28 @@ class LinearResponseCovariances(object):
         return r._replace(**{f: getattr(r, f).cpu().numpy() for f in ("lpd", "lpd_loo", "eta_mean_loo",
                                                                       "eta_var_loo")})
 
+    def get_approximate_logo(self):
+        """Approximate leave-one-group-out cross-validation and group influence at the optimum by the infinitesimal
+        jackknife: a ``GLMM.ApproximateLOGO`` with the pointwise lpd_logo, eta_mean_logo, eta_var_logo (caller's row
+        order), the per-group elpd_logo_group, cooks_distance and delta_global (G, Dg), and elpd_logo, elpd_logo_se;
+        numpy for a numpy optimum, CUDA tensors for a CUDA one.  delta_global[g] is the global block of
+        ``WeightSensitivityLinearApproximation.get_dinput_dhyper_times`` with the weights of group g's rows dropped,
+        for all groups at once.  Always from S^-1, whatever ``method`` is (cached with ``get_prediction_variances``)."""
+        model = self.model
+        if getattr(model, "local", None) is not None:
+            raise NotImplementedError("approximate LOGO of a sharded model: build a single-GPU LogisticGLMM of the "
+                                      "job and use its LinearResponseCovariances")
+        model._check_binary_y()
+        self._ensure_point()
+        if self._sinv is None:
+            self._sinv = model.global_covariance()
+        r = model.approximate_logo(self._sinv)
+        if is_torch(self._opt0):
+            return r
+        return r._replace(**{f: getattr(r, f).cpu().numpy() for f in ("lpd_logo", "eta_mean_logo", "eta_var_logo",
+                                                                      "elpd_logo_group", "cooks_distance",
+                                                                      "delta_global")})
+
     MAX_DENSE = 1 << 26
 
     def get_lr_covariance_from_jacobians(self, moment_jacobian1, moment_jacobian2=None):

@@ -296,6 +296,7 @@ struct lrvb_glmm {
   int schur_grid = 0;
   double* schurpart = nullptr;
   double* pred_B = nullptr;   // (3 Kp8, Kp4) scaled beta block of S^-1 for lrvb_glmm_predict_lr (predict.cu)
+  double* logo_V = nullptr;   // (G, Dg) per-group gradients of lrvb_glmm_logo, then its (G, K) Cook's products (logo.cu)
 };
 
 namespace lrvb {

@@ -490,6 +490,10 @@ class ShardedLogisticGLMM(object):
         raise NotImplementedError("approximate LOO of a sharded model: build a single-GPU LogisticGLMM of the job "
                                   "and use LinearResponseCovariances.get_approximate_loo")
 
+    def approximate_logo(self, *args, **kwargs):
+        raise NotImplementedError("approximate LOGO of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                  "and use LinearResponseCovariances.get_approximate_logo")
+
     def moment_jacobian(self, free):
         import scipy.sparse
         free = np.asarray(free, dtype=np.float64).reshape(-1)
