@@ -1,16 +1,9 @@
 // C-ABI entry points: handle life-cycle and evaluation (see include/lrvb_b200.h).
 #include <stdarg.h>
 #include <string.h>
-#include <stdlib.h>
 #include <new>
 #include <vector>
 #include "common.cuh"
-#include "gram_small.cuh"
-#include "obs_fused.cuh"
-#include "gram_mid.cuh"
-#include "gram_big.cuh"
-#include "gram_wide.cuh"
-#include "fused.cuh"
 
 namespace lrvb {
 
@@ -36,18 +29,6 @@ __global__ void k_gptr(const int32_t* __restrict__ g, int32_t* __restrict__ gptr
   if (n > 0 && n < N && cur < prev) { atomicOr(flags, 2); return; }
   for (int gg = prev + 1; gg <= cur; ++gg) gptr[gg] = (int32_t)n;
 }
-
-template <typename T>
-static int dev_alloc(T** p, size_t n) {
-  *p = nullptr;
-  if (n == 0) n = 1;
-  LRVB_CUDA(cudaMalloc((void**)p, n * sizeof(T)));
-  return LRVB_OK;
-}
-
-// kernels defined in glmm_eval.cu whose attributes must be raised for > 48 KB dynamic smem
-void configure_kernels(size_t obs_smem, size_t gram_smem);
-void configure_obs_fused(size_t smem);
 
 }  // namespace lrvb
 
@@ -151,135 +132,7 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
   h->ldw = (N + 7) / 8 * 8;
   CREATE_TRY(dev_alloc(&h->W, 5 * (size_t)h->ldw));
 
-  // observation pass geometry (k_obs, K > 62: 64-row tiles; obs_nbuf = tile buffers, two when they fit)
-  {
-    const size_t tile = sizeof(double) * 64 * (size_t)K, extra = sizeof(double) * (2 * (size_t)(Q + 3) + 32 + 2);
-    h->obs_nbuf = (2 * tile + extra <= 220 * 1024) ? 2 : 1;
-    h->obs_smem = h->obs_nbuf * tile + extra;
-    int64_t nt = (N + 63) / 64;
-    h->obs_grid = (int)(nt < kNumSMs ? nt : kNumSMs);
-    if (h->obs_grid < 1) h->obs_grid = 1;
-  }
-  if (K <= kOfMaxK) {
-    // fused observation + group pass: every warp owns a contiguous multiple-of-32 range of rows
-    h->obs_fused = 1;
-    h->of_warps = obs_fused_warps(K);
-    const int64_t nst = (N + kOfRows - 1) / kOfRows;
-    int64_t grid = (nst + h->of_warps - 1) / h->of_warps;
-    if (grid > kNumSMs) grid = kNumSMs;
-    if (grid < 1) grid = 1;
-    h->of_grid = (int)grid;
-    const int64_t tw = grid * h->of_warps;
-    h->of_rows_per_warp = ((nst + tw - 1) / tw) * kOfRows;
-    h->of_smem = obs_fused_smem(K, Q, h->of_warps);
-    int64_t nrec = tw;
-    {
-      // one-slot rings when they buy at least three more warps per SM (K >= ~36)
-      const int w1 = obs_fused_warps(K, 1);
-      if (w1 >= h->of_warps + 3) {
-        int64_t g1 = (nst + w1 - 1) / w1;
-        if (g1 > kNumSMs) g1 = kNumSMs;
-        if (g1 < 1) g1 = 1;
-        const int64_t tw1 = g1 * w1;
-        h->of1_grid = (int)g1;
-        h->of1_warps = w1;
-        h->of1_rows_per_warp = ((nst + tw1 - 1) / tw1) * kOfRows;
-        h->of1_smem = obs_fused_smem(K, Q, w1, 1);
-        if (tw1 > nrec) nrec = tw1;
-        if (h->obs_grid < h->of1_grid) h->obs_grid = h->of1_grid;
-      }
-    }
-    if (K <= kFuMaxK) {
-      // order 2 in one pass (fused.cuh): teams of NQ quadrature warps + P DMMA warps, one CTA per SM; every
-      // Q warp owns a contiguous multiple-of-32 range of rows.  Only for K <= 24, where quadrature and Gram
-      // need about the same pipe time and the one-pass kernel is ~10 % faster than the two kernels; for larger
-      // K the Gram dominates, the D warps of the one-pass kernel (128 registers, 4 warps per triangle) are
-      // slower than gram_mid's (255 registers, 2 warps) and the two-kernel path wins
-      // (profiles/r02_onepass_attempts.md).
-      const int nqw = kFuGeom.teams * kFuGeom.NQ;
-      int64_t fgrid = (nst + nqw - 1) / nqw;
-      if (fgrid > kNumSMs) fgrid = kNumSMs;
-      if (fgrid < 1) fgrid = 1;
-      const int64_t tt = fgrid * nqw;
-      h->fused2 = 1;
-      h->fu_grid = (int)fgrid;
-      h->fu_teams = nqw;
-      h->fu_warps = kFuGeom.warps;
-      h->fu_rows_per_team = ((nst + tt - 1) / tt) * kFuRows;
-      if (tt > nrec) nrec = tt;
-    }
-    CREATE_TRY(dev_alloc(&h->bval, (size_t)nrec * 2 * (5 + 4 * (size_t)K)));
-    configure_obs_fused(h->of_smem > h->of1_smem ? h->of_smem : h->of1_smem);
-    if (h->obs_grid < h->of_grid) h->obs_grid = h->of_grid;
-    if (h->obs_grid < h->fu_grid) h->obs_grid = h->fu_grid;     // klpart / gradpart are sized by obs_grid
-  }
-  CREATE_TRY(dev_alloc(&h->klpart, (size_t)h->obs_grid));
-  CREATE_TRY(dev_alloc(&h->gradpart, (size_t)h->obs_grid * 2 * K));
-
-  CREATE_TRY(dev_alloc(&h->gsc, (size_t)G * 5));
-  CREATE_TRY(dev_alloc(&h->BR, (size_t)G * 4 * K));
-  h->loc_grid = cdiv(G, 256);
-  if (h->loc_grid > 2 * kNumSMs) h->loc_grid = 2 * kNumSMs;
-  if (h->loc_grid < 1) h->loc_grid = 1;
-  CREATE_TRY(dev_alloc(&h->locpart, (size_t)h->loc_grid * 4));
-  CREATE_TRY(dev_alloc(&h->fin_counter, 1));
-  CREATE_TRY(dev_alloc(&h->fin_pre, 8 + 2 * (size_t)K));
-  CREATE_CUDA(cudaMemsetAsync(h->fin_counter, 0, sizeof(unsigned int), st));
-
-  // Gram geometry
-  {
-    size_t npart;
-    if (h->fused2) {
-      // no Gram kernel: the one-pass kernel (fused.cuh) writes the packed partials, one slab per CTA
-      npart = (size_t)h->fu_grid * gram_small_shape(K).NT * 64;
-    } else if (K <= kGmMaxK) {
-      // 24 < K <= 104: one warp or a team of warps = the whole packed triangle (gram_mid.cuh)
-      h->gram_mid = 1;
-      h->gram_grid_x = kNumSMs;
-      h->gram_grid_y = 1;
-      npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
-    } else if (gram_wide_eligible(K)) {
-      // large K, no straddle tile: block-against-block jobs (16 - 25 tiles per warp), 8 warps per SM, only the
-      // column blocks of a job group staged (gram_wide.cuh)
-      const GwPlan pl = gram_wide_plan(K);
-      h->gram_wide = 1;
-      if (getenv("LRVB_GROUP_OVERLAP") && getenv("LRVB_GROUP_OVERLAP")[0] == '0') h->group_overlap = 0;
-      h->gram_grid_x = (int)pl.ctas.size();
-      h->gram_grid_y = (int)pl.groups.size();
-      h->gram_smem = pl.smem;
-      CREATE_TRY(dev_alloc((char**)&h->jobs, sizeof(GwGroup) * pl.groups.size()));
-      CREATE_TRY(dev_alloc((char**)&h->gslots, sizeof(GwCta) * pl.ctas.size()));
-      CREATE_CUDA(cudaMemcpyAsync(h->jobs, pl.groups.data(), sizeof(GwGroup) * pl.groups.size(),
-                                  cudaMemcpyHostToDevice, st));
-      CREATE_CUDA(cudaMemcpyAsync(h->gslots, pl.ctas.data(), sizeof(GwCta) * pl.ctas.size(),
-                                  cudaMemcpyHostToDevice, st));
-      CREATE_CUDA(cudaStreamSynchronize(st));   // pl goes out of scope
-      npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
-    } else {
-      // rectangles of the packed triangle dealt to 16-warp CTAs (gram_big.cuh)
-      const GbPlan pl = gram_big_plan(K);
-      h->gram_jobs = (int)pl.jobs.size();
-      h->gram_grid_y = pl.n_groups;
-      h->gram_tn = pl.TN;
-      h->gram_smem = pl.smem;
-      int64_t nst = (N + pl.TN - 1) / pl.TN;
-      int64_t nchunk = (kNumSMs * kGbCtasPerSM) / pl.n_groups;
-      if (nchunk > nst) nchunk = nst;
-      if (nchunk < 1) nchunk = 1;
-      h->gram_grid_x = (int)nchunk * pl.n_groups;
-      CREATE_TRY(dev_alloc((char**)&h->jobs, sizeof(GbJob) * pl.jobs.size()));
-      CREATE_TRY(dev_alloc((char**)&h->gslots, sizeof(GbSlot) * pl.slots.size()));
-      CREATE_CUDA(cudaMemcpyAsync(h->jobs, pl.jobs.data(), sizeof(GbJob) * pl.jobs.size(),
-                                  cudaMemcpyHostToDevice, st));
-      CREATE_CUDA(cudaMemcpyAsync(h->gslots, pl.slots.data(), sizeof(GbSlot) * pl.slots.size(),
-                                  cudaMemcpyHostToDevice, st));
-      CREATE_CUDA(cudaStreamSynchronize(st));   // pl goes out of scope
-      npart = (size_t)nchunk * pl.n_groups * kGbWarps * 16 * 64;
-    }
-    CREATE_TRY(dev_alloc(&h->grampart, npart));
-    CREATE_CUDA(cudaMemsetAsync(h->grampart, 0, sizeof(double) * npart, st));
-  }
-  configure_kernels(h->obs_smem, h->gram_smem);
+  CREATE_TRY(plan_eval(h, st));
 
   CREATE_TRY(dev_alloc(&h->B, (size_t)G * 2 * Dg));
   CREATE_TRY(dev_alloc(&h->L, (size_t)G * 3));

@@ -54,6 +54,26 @@ constexpr int kRT = 4;        // Schur warp job = kRT x kRT output tiles of 8x8 
 
 static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
+template <typename T>
+static int dev_alloc(T** p, size_t n) {
+  *p = nullptr;
+  if (n == 0) n = 1;
+  LRVB_CUDA(cudaMalloc((void**)p, n * sizeof(T)));
+  return LRVB_OK;
+}
+
+// Let `kernel` use `bytes` of dynamic shared memory on the current device.  The limit is an attribute of the
+// kernel on a device, shared by every handle there, so it is only ever raised: lowering it to one handle's
+// need would make another handle's launches fail.
+template <typename... KArgs>
+static int raise_smem_limit(void (*kernel)(KArgs...), size_t bytes) {
+  cudaFuncAttributes fa;
+  LRVB_CUDA(cudaFuncGetAttributes(&fa, kernel));
+  if (bytes > (size_t)fa.maxDynamicSharedSizeBytes)
+    LRVB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  return LRVB_OK;
+}
+
 // ---- fp64 special functions the CUDA math library lacks -------------------------------
 // digamma / trigamma / tetragamma for x > 0: upward recurrence to x >= 16, then the
 // asymptotic (Bernoulli) series; truncation < 1e-17 relative there.
@@ -206,6 +226,8 @@ __device__ __forceinline__ void tile_load_async(double* dst, const double* src, 
 }
 #endif  // __CUDACC__
 
+struct FusedArgs;   // fused.cuh
+
 }  // namespace lrvb
 
 // ---- the model handle --------------------------------------------------------------------
@@ -237,13 +259,15 @@ struct lrvb_glmm {
   int64_t of_rows_per_warp = 0;
   double* bval = nullptr;     // (of_grid * of_warps, 2, 5 + 4K) head / tail pieces of straddling groups
   double* wc_scratch = nullptr;   // (2, ldw) l_m, l_v of a weight-cross-Hessian pass for K > 62 (allocated on first use)
-  // one-slot variant of the fused observation pass for the evaluation (larger K: more warps per SM)
+  // one-slot variant of the fused observation pass, which the evaluation runs (more warps per SM than two slots)
   int of1_grid = 0, of1_warps = 0;
   size_t of1_smem = 0;
   int64_t of1_rows_per_warp = 0;
   // order-2 evaluation in one pass (fused.cuh, K <= 24): teams of warps do quadrature, group sums and Gram per stage
   int fused2 = 0, fu_grid = 0, fu_teams = 0, fu_warps = 0;
   int64_t fu_rows_per_team = 0;
+  size_t fu_smem = 0;
+  void (*fu_kernel)(lrvb::FusedArgs) = nullptr;   // the instantiation for K
   int ev_gram = 0;            // the last timed evaluation ran a separate Gram kernel
   // group pass
   double* gsc = nullptr;      // (G, 5) per-group sums of l_m, l_v, a, b, c
@@ -255,6 +279,9 @@ struct lrvb_glmm {
   // Gram
   int gram_tn = 0, gram_grid_x = 0, gram_grid_y = 0, gram_jobs = 0;   // grid_y = job groups
   size_t gram_smem = 0;
+  // gram_mid: the instantiation for K and its CTA size
+  void (*gm_kernel)(const double*, const double*, double*, int64_t, int64_t, int) = nullptr;
+  int gm_warps = 0;
   int group_overlap = 1;      // k_group on the side stream behind k_gram_wide (LRVB_GROUP_OVERLAP=0: serial)
   int gram_wide = 0;          // K = 176 .. 240, K % 8 == 0: block jobs of 4-5 tiles, 8 warps x 255 registers (gram_wide.cuh);
                               // jobs = GwGroup[], gslots = GwCta[gram_grid_x]
@@ -300,7 +327,9 @@ struct lrvb_glmm {
 };
 
 namespace lrvb {
-// kernels.cu entry points used by api.cu (all enqueue on `st`)
+// glmm_eval.cu entry points used by api.cu (all enqueue on `st`)
+// Plan the evaluation of a new handle: kernels, launch geometries, their scratch buffers and shared-memory limits.
+int plan_eval(lrvb_glmm* h, cudaStream_t st);
 int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_global,
                 double* grad_local, cudaStream_t st);
 }  // namespace lrvb

@@ -661,6 +661,12 @@ static int ensure_csr_scratch(lrvb_glmm* h) {
   const int nblk = cdiv(D, kScanChunk);
   const int CG = csr_chunk_groups(Dg);
   const int nchunk = cdiv(G, CG) > 0 ? cdiv(G, CG) : 1;
+  // raised first: once h->rowcnt is set, this function returns at its first line
+  const size_t smem = sizeof(double) * (size_t)CG * (2 * Dg + 1);
+  LRVB_TRY(raise_smem_limit(k_csr_pass<0>, smem));
+  LRVB_TRY(raise_smem_limit(k_csr_pass<1>, smem));
+  LRVB_TRY(raise_smem_limit(k_csr_pass<2>, csr_refill_smem(Dg, CG)));
+  LRVB_TRY(raise_smem_limit(k_csr_export_coop, smem));
   h->csr_cg = CG;
   h->csr_nchunk = nchunk;
   LRVB_CUDA(cudaMalloc((void**)&h->rowcnt, sizeof(int32_t) * (size_t)(D + 1)));
@@ -671,11 +677,6 @@ static int ensure_csr_scratch(lrvb_glmm* h) {
   // zero mask of the last full export: A (Dg x WA) | B (2G x WA) | L (G) words
   const size_t WA = ((size_t)Dg + 31) / 32;
   LRVB_CUDA(cudaMalloc((void**)&h->csrmask, sizeof(uint32_t) * ((size_t)(Dg + 2 * (size_t)G) * WA + (size_t)G + 1)));
-  const size_t smem = sizeof(double) * (size_t)CG * (2 * Dg + 1);
-  cudaFuncSetAttribute(k_csr_pass<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  cudaFuncSetAttribute(k_csr_pass<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  cudaFuncSetAttribute(k_csr_pass<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csr_refill_smem(Dg, CG));
-  cudaFuncSetAttribute(k_csr_export_coop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   // the grid-barrier words of the one-launch export (the four spare words behind the scan scratch)
   LRVB_CUDA(cudaMemset(h->csrwork + (size_t)3 * Dg + (size_t)6 * Dg * nchunk, 0, sizeof(int32_t) * 4));
   return LRVB_OK;

@@ -608,25 +608,16 @@ k_fused_eval(const FusedArgs a) {
   }
 }
 
-// launch the instantiation for K; false when K / alignment is outside its range
-inline bool launch_fused_eval(const FusedArgs& a, int grid, int Q, cudaStream_t st) {
-  const int K = a.K;
-  if (K < 1 || K > kFuMaxK || (a.ldw & 1) || (((uintptr_t)a.X) & 15)) return false;
+// the instantiation for K (K <= kFuMaxK), launched with 32 * kFuGeom.warps threads and fused_smem bytes; null
+// outside that range
+inline auto fused_eval_kernel(int K) -> void (*)(FusedArgs) {
   const int T2 = (2 * K + 7) / 8, T0 = K / 8;
   const bool M = (K % 8) != 0;
   const int nch = (K + 1 + 31) / 32;
-  const size_t smem = fused_smem(K, Q, T2);
 #define LRVB_FU(T2_, T0_, M_, NCH_)                                                                  \
   if (T2 == T2_ && T0 == T0_ && M == M_ && nch == NCH_) {                                            \
-    constexpr FusedGeom g = kFuGeom;                                                                 \
-    static size_t configured = 48 * 1024;                                                            \
-    if (smem > configured) {                                                                         \
-      cudaFuncSetAttribute(k_fused_eval<T2_, T0_, M_, NCH_, g.teams, g.NQ, g.P, g.warps, g.slots>,   \
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                  \
-      configured = smem;                                                                             \
-    }                                                                                                \
-    return launch_pdl(k_fused_eval<T2_, T0_, M_, NCH_, g.teams, g.NQ, g.P, g.warps, g.slots>, dim3(grid), \
-                      dim3(32 * g.warps), smem, st, a) == cudaSuccess;                               \
+    return k_fused_eval<T2_, T0_, M_, NCH_, kFuGeom.teams, kFuGeom.NQ, kFuGeom.P, kFuGeom.warps,       \
+                        kFuGeom.slots>;                                                              \
   }
   LRVB_FU(1, 0, true, 1)
   LRVB_FU(2, 0, true, 1)
@@ -638,7 +629,7 @@ inline bool launch_fused_eval(const FusedArgs& a, int grid, int Q, cudaStream_t 
   LRVB_FU(6, 2, true, 1)
   LRVB_FU(6, 3, false, 1)
 #undef LRVB_FU
-  return false;
+  return nullptr;
 }
 
 }  // namespace lrvb

@@ -8,12 +8,17 @@
 //
 // Pipeline of one evaluation (all on one stream, no atomics, fixed reduction orders so the
 // result is bitwise reproducible for a given launch geometry):
-//   k_prep         free -> constrained vector
-//   k_obs          per-observation pass: z_mean/z_var, Gauss-Hermite softplus / sigma / sigma',
-//                  analytic l, dl, d2l; per-CTA partials of KL and of X^T l_m, S^T l_v
-//   k_group        per-group segmented sums (observations are group-sorted): scalars + borders
-//   k_gram         X^T diag(a) X, X^T diag(b) S, S^T diag(c) S on the FP64 tensor cores (DMMA)
-//   k_local/k_border/k_gram_finish/k_global   chain rule to free coordinates, non-data terms
+//   k_prep          free -> constrained vector
+//   observation pass: z_mean/z_var, Gauss-Hermite softplus / sigma / sigma', analytic l, dl, d2l; per-CTA
+//                   partials of KL and of X^T l_m, S^T l_v; per-group segmented sums (observations are
+//                   group-sorted): scalars + borders
+//     K <= 24, order 2   k_fused_eval (fused.cuh) also computes the Gram: one pass over X
+//     K <= 62            k_obs_fused (obs_fused.cuh), one-slot rings
+//     K > 62             k_obs, then k_group
+//   Gram            X^T diag(a) X, X^T diag(b) S, S^T diag(c) S on the FP64 tensor cores (DMMA), order 2:
+//                   k_gram_mid (K <= 104), k_gram_wide (gram_wide_eligible), k_gram_big (the rest)
+//   k_finish, k_global_post   straddling-group fix-up, chain rule to free coordinates, non-data terms
+#include <stdlib.h>
 #include "common.cuh"
 #include "gram_small.cuh"
 #include "obs_fused.cuh"
@@ -67,35 +72,6 @@ __global__ void k_prep(const double* __restrict__ free_v, double* __restrict__ v
     aux[8 + (i - 4 - K)] = -1.0 / (v * v);
   } else if (i >= 4 + 2 * K + G) {
     aux[8 + K + (i - 4 - 2 * K - G)] = 1.0 / (v * v);
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// Gauss-Hermite node: softplus(t), sigma(t), sigma'(t) from ONE exp (SURVEY.md section 7).
-// Modeling.py:48 evaluates log1p(exp(t)) unstabilised; this is the same function to <= 1 ulp
-// on the finite range and stays finite beyond it.
-struct GHSums {
-  double A, Am, As, Amm, Ams, Ass;
-};
-
-template <int ORDER>
-__device__ __forceinline__ void gh_node(double t, double c, double wq, GHSums& s) {
-  const double e = exp(-fabs(t));
-  const double sp = fmax(t, 0.0) + log1p(e);
-  s.A = fma(wq, sp, s.A);
-  if (ORDER >= 1) {
-    const double r = 1.0 / (1.0 + e);
-    const double sg = (t >= 0.0) ? r : e * r;
-    const double wsg = wq * sg;
-    s.Am += wsg;
-    s.As = fma(wsg, c, s.As);
-    if (ORDER >= 2) {
-      const double wd = wq * (e * r * r);
-      const double wdc = wd * c;
-      s.Amm += wd;
-      s.Ams += wdc;
-      s.Ass = fma(wdc, c, s.Ass);
-    }
   }
 }
 
@@ -555,29 +531,53 @@ k_group(const double* __restrict__ X, const double* __restrict__ W,
   }
 }
 
-// Launchers for sensitivity.cu (K > 62): the data terms of the gradient with dw as the weights -- k_obs<1>
-// writing l_m, l_v into a scratch W (the cached evaluation's W stays intact) + k_group<1> on it -- and the
-// influence pass.
-int launch_wide_weight_pass(lrvb_glmm* h, const double* dw, double* scratchW, cudaStream_t st) {
+// The data terms of the gradient with dw as the weights, for lrvb_glmm_weight_cross_matvec (sensitivity.cu):
+// the per-CTA partials of X^T l_m, S^T l_v go to gradpart (*n_gp of them), the per-group sums to gsc and BR.  The
+// cached evaluation's W (lrvb_glmm_obs_weights) stays intact.  K <= 62: the two-slot fused observation pass,
+// which writes no W, then k_obs_fixup<1>; K > 62: k_obs<1>, writing l_m, l_v into a scratch block, then k_group<1>.
+int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t st) {
   const int K = h->K, G = h->G, Q = h->Q;
-  if (h->N > 0) {
-    k_obs<1><<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, scratchW, h->klpart,
-                                                    h->gradpart, h->N, h->ldw, K, G, Q, h->obs_nbuf);
+  const int64_t N = h->N;
+  *n_gp = 0;
+  if (h->obs_fused) {
+    if (N > 0) {
+      auto kern = (K + 1 + 31) / 32 == 1 ? k_obs_fused<1, 1> : k_obs_fused<1, 2>;
+      LRVB_TRY(raise_smem_limit(kern, h->of_smem));
+      kern<<<h->of_grid, 32 * h->of_warps, h->of_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, h->gptr, nullptr,
+                                                             h->ldw, h->klpart, h->gradpart, h->gsc, h->BR, h->bval,
+                                                             N, K, G, Q, h->of_rows_per_warp);
+      LRVB_CHECK_LAUNCH();
+      *n_gp = h->of_grid;
+    }
+    if (G > 0) {
+      k_obs_fixup<1><<<cdiv(G, 8), 256, 0, st>>>(h->gptr, h->bval, h->gsc, h->BR, K, G,
+                                                 h->of_rows_per_warp > 0 ? h->of_rows_per_warp : 32);
+      LRVB_CHECK_LAUNCH();
+    }
+    return LRVB_OK;
+  }
+  if (N > 0) {
+    if (!h->wc_scratch && cudaMalloc(&h->wc_scratch, sizeof(double) * 2 * (size_t)h->ldw) != cudaSuccess) {
+      cudaGetLastError();
+      set_error("lrvb_glmm_weight_cross_matvec: out of device memory (%zu bytes of scratch)",
+                sizeof(double) * 2 * (size_t)h->ldw);
+      return LRVB_ECUDA;
+    }
+    k_obs<1><<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, h->wc_scratch, h->klpart,
+                                                    h->gradpart, N, h->ldw, K, G, Q, h->obs_nbuf);
     LRVB_CHECK_LAUNCH();
+    *n_gp = h->obs_grid;
   }
   if (G > 0) {
     const int ggrid = (int)((G + 7) / 8 < 148 * 8 ? (G + 7) / 8 : 148 * 8);
-    k_group<1><<<ggrid, 256, 0, st>>>(h->X, scratchW, h->gptr, h->gsc, h->BR, h->ldw, K, G);
+    k_group<1><<<ggrid, 256, 0, st>>>(h->X, h->wc_scratch, h->gptr, h->gsc, h->BR, h->ldw, K, G);
     LRVB_CHECK_LAUNCH();
   }
   return LRVB_OK;
 }
+// The influence pass for K > 62 (lrvb_glmm_weight_cross_rmatvec) on the k_obs tile walk
 int launch_wide_influence(lrvb_glmm* h, const double* v, double* out, cudaStream_t st) {
-  static size_t configured = 48 * 1024;
-  if (h->obs_smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_obs_influence_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->obs_smem));
-    configured = h->obs_smem;
-  }
+  LRVB_TRY(raise_smem_limit(k_obs_influence_wide, h->obs_smem));
   k_obs_influence_wide<<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, h->vec, h->gh, v, out, h->N, h->K,
                                                              h->G, h->Q, h->obs_nbuf, h->bounds, h->vecmode);
   LRVB_CHECK_LAUNCH();
@@ -1095,6 +1095,160 @@ k_global_post(const double* __restrict__ vec, const double* locpart, int K, int 
 }
 
 // ------------------------------------------------------------------------------------------
+int plan_eval(lrvb_glmm* h, cudaStream_t st) {
+  const int K = h->K, G = h->G, Q = h->Q;
+  const int64_t N = h->N;
+  // observation pass geometry (k_obs, K > 62: 64-row tiles; obs_nbuf = tile buffers, two when they fit)
+  {
+    const size_t tile = sizeof(double) * 64 * (size_t)K, extra = sizeof(double) * (2 * (size_t)(Q + 3) + 32 + 2);
+    h->obs_nbuf = (2 * tile + extra <= 220 * 1024) ? 2 : 1;
+    h->obs_smem = h->obs_nbuf * tile + extra;
+    int64_t nt = (N + 63) / 64;
+    h->obs_grid = (int)(nt < kNumSMs ? nt : kNumSMs);
+    if (h->obs_grid < 1) h->obs_grid = 1;
+  }
+  if (K <= kOfMaxK) {
+    // fused observation + group pass: every warp owns a contiguous multiple-of-32 range of rows.  The two-slot
+    // geometry (of_*) serves the weight-cross pass (launch_weight_pass) and the influence pass (k_obs_influence).
+    h->obs_fused = 1;
+    h->of_warps = obs_fused_warps(K);
+    const int64_t nst = (N + kOfRows - 1) / kOfRows;
+    int64_t grid = (nst + h->of_warps - 1) / h->of_warps;
+    if (grid > kNumSMs) grid = kNumSMs;
+    if (grid < 1) grid = 1;
+    h->of_grid = (int)grid;
+    const int64_t tw = grid * h->of_warps;
+    h->of_rows_per_warp = ((nst + tw - 1) / tw) * kOfRows;
+    h->of_smem = obs_fused_smem(K, Q, h->of_warps);
+    int64_t nrec = tw;
+    {
+      // the evaluation runs one-slot rings: they fit 16 down to 12 warps per SM where two slots fit 12 down to 6
+      const int w1 = obs_fused_warps(K, 1);
+      int64_t g1 = (nst + w1 - 1) / w1;
+      if (g1 > kNumSMs) g1 = kNumSMs;
+      if (g1 < 1) g1 = 1;
+      const int64_t tw1 = g1 * w1;
+      h->of1_grid = (int)g1;
+      h->of1_warps = w1;
+      h->of1_rows_per_warp = ((nst + tw1 - 1) / tw1) * kOfRows;
+      h->of1_smem = obs_fused_smem(K, Q, w1, 1);
+      if (tw1 > nrec) nrec = tw1;
+      if (h->obs_grid < h->of1_grid) h->obs_grid = h->of1_grid;
+      if ((K + 1 + 31) / 32 == 1) {
+        LRVB_TRY(raise_smem_limit(k_obs_fused<0, 1, 1>, h->of1_smem));
+        LRVB_TRY(raise_smem_limit(k_obs_fused<1, 1, 1>, h->of1_smem));
+        LRVB_TRY(raise_smem_limit(k_obs_fused<2, 1, 1>, h->of1_smem));
+      } else {
+        LRVB_TRY(raise_smem_limit(k_obs_fused<0, 2, 1>, h->of1_smem));
+        LRVB_TRY(raise_smem_limit(k_obs_fused<1, 2, 1>, h->of1_smem));
+        LRVB_TRY(raise_smem_limit(k_obs_fused<2, 2, 1>, h->of1_smem));
+      }
+    }
+    if (K <= kFuMaxK) {
+      // order 2 in one pass (fused.cuh): teams of NQ quadrature warps + P DMMA warps, one CTA per SM; every
+      // Q warp owns a contiguous multiple-of-32 range of rows.  Only for K <= 24, where quadrature and Gram
+      // need about the same pipe time and the one-pass kernel is ~10 % faster than the two kernels; for larger
+      // K the Gram dominates, the D warps of the one-pass kernel (128 registers, 4 warps per triangle) are
+      // slower than gram_mid's (255 registers, 2 warps) and the two-kernel path wins
+      // (profiles/r02_onepass_attempts.md).
+      const int nqw = kFuGeom.teams * kFuGeom.NQ;
+      int64_t fgrid = (nst + nqw - 1) / nqw;
+      if (fgrid > kNumSMs) fgrid = kNumSMs;
+      if (fgrid < 1) fgrid = 1;
+      const int64_t tt = fgrid * nqw;
+      h->fused2 = 1;
+      h->fu_grid = (int)fgrid;
+      h->fu_teams = nqw;
+      h->fu_warps = kFuGeom.warps;
+      h->fu_rows_per_team = ((nst + tt - 1) / tt) * kFuRows;
+      h->fu_kernel = fused_eval_kernel(K);
+      h->fu_smem = fused_smem(K, Q, gram_small_shape(K).T2);
+      LRVB_TRY(raise_smem_limit(h->fu_kernel, h->fu_smem));
+      if (tt > nrec) nrec = tt;
+    }
+    LRVB_TRY(dev_alloc(&h->bval, (size_t)nrec * 2 * (5 + 4 * (size_t)K)));
+    if (h->obs_grid < h->of_grid) h->obs_grid = h->of_grid;
+    if (h->obs_grid < h->fu_grid) h->obs_grid = h->fu_grid;     // klpart / gradpart are sized by obs_grid
+  } else {
+    LRVB_TRY(raise_smem_limit(k_obs<0>, h->obs_smem));
+    LRVB_TRY(raise_smem_limit(k_obs<1>, h->obs_smem));
+    LRVB_TRY(raise_smem_limit(k_obs<2>, h->obs_smem));
+  }
+  LRVB_TRY(dev_alloc(&h->klpart, (size_t)h->obs_grid));
+  LRVB_TRY(dev_alloc(&h->gradpart, (size_t)h->obs_grid * 2 * K));
+
+  LRVB_TRY(dev_alloc(&h->gsc, (size_t)G * 5));
+  LRVB_TRY(dev_alloc(&h->BR, (size_t)G * 4 * K));
+  h->loc_grid = cdiv(G, 256);
+  if (h->loc_grid > 2 * kNumSMs) h->loc_grid = 2 * kNumSMs;
+  if (h->loc_grid < 1) h->loc_grid = 1;
+  LRVB_TRY(dev_alloc(&h->locpart, (size_t)h->loc_grid * 4));
+  LRVB_TRY(dev_alloc(&h->fin_counter, 1));
+  LRVB_TRY(dev_alloc(&h->fin_pre, 8 + 2 * (size_t)K));
+  LRVB_CUDA(cudaMemsetAsync(h->fin_counter, 0, sizeof(unsigned int), st));
+
+  // Gram geometry
+  size_t npart;
+  if (h->fused2) {
+    // no Gram kernel: the one-pass kernel (fused.cuh) writes the packed partials, one slab per CTA
+    npart = (size_t)h->fu_grid * gram_small_shape(K).NT * 64;
+  } else if (K <= kGmMaxK) {
+    // 24 < K <= 104: one warp or a team of warps = the whole packed triangle (gram_mid.cuh)
+    const GramMidKernel gk = gram_mid_kernel(K);
+    h->gram_mid = 1;
+    h->gm_kernel = gk.fn;
+    h->gm_warps = gk.warps;
+    h->gram_smem = gram_mid_smem(K, gram_small_shape(K).T2);
+    LRVB_TRY(raise_smem_limit(h->gm_kernel, h->gram_smem));
+    h->gram_grid_x = kNumSMs;
+    h->gram_grid_y = 1;
+    npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
+  } else if (gram_wide_eligible(K)) {
+    // large K, no straddle tile: block-against-block jobs (16 - 25 tiles per warp), 8 warps per SM, only the
+    // column blocks of a job group staged (gram_wide.cuh)
+    const GwPlan pl = gram_wide_plan(K);
+    h->gram_wide = 1;
+    if (getenv("LRVB_GROUP_OVERLAP") && getenv("LRVB_GROUP_OVERLAP")[0] == '0') h->group_overlap = 0;
+    h->gram_grid_x = (int)pl.ctas.size();
+    h->gram_grid_y = (int)pl.groups.size();
+    h->gram_smem = pl.smem;
+    LRVB_TRY(raise_smem_limit(k_gram_wide, h->gram_smem));
+    LRVB_TRY(dev_alloc((char**)&h->jobs, sizeof(GwGroup) * pl.groups.size()));
+    LRVB_TRY(dev_alloc((char**)&h->gslots, sizeof(GwCta) * pl.ctas.size()));
+    LRVB_CUDA(cudaMemcpyAsync(h->jobs, pl.groups.data(), sizeof(GwGroup) * pl.groups.size(),
+                              cudaMemcpyHostToDevice, st));
+    LRVB_CUDA(cudaMemcpyAsync(h->gslots, pl.ctas.data(), sizeof(GwCta) * pl.ctas.size(),
+                              cudaMemcpyHostToDevice, st));
+    LRVB_CUDA(cudaStreamSynchronize(st));   // pl goes out of scope
+    npart = (size_t)h->gram_grid_x * gram_small_shape(K).NT * 64;
+  } else {
+    // rectangles of the packed triangle dealt to 16-warp CTAs (gram_big.cuh)
+    const GbPlan pl = gram_big_plan(K);
+    h->gram_jobs = (int)pl.jobs.size();
+    h->gram_grid_y = pl.n_groups;
+    h->gram_tn = pl.TN;
+    h->gram_smem = pl.smem;
+    LRVB_TRY(raise_smem_limit(k_gram_big, h->gram_smem));
+    int64_t nst = (N + pl.TN - 1) / pl.TN;
+    int64_t nchunk = (kNumSMs * kGbCtasPerSM) / pl.n_groups;
+    if (nchunk > nst) nchunk = nst;
+    if (nchunk < 1) nchunk = 1;
+    h->gram_grid_x = (int)nchunk * pl.n_groups;
+    LRVB_TRY(dev_alloc((char**)&h->jobs, sizeof(GbJob) * pl.jobs.size()));
+    LRVB_TRY(dev_alloc((char**)&h->gslots, sizeof(GbSlot) * pl.slots.size()));
+    LRVB_CUDA(cudaMemcpyAsync(h->jobs, pl.jobs.data(), sizeof(GbJob) * pl.jobs.size(),
+                              cudaMemcpyHostToDevice, st));
+    LRVB_CUDA(cudaMemcpyAsync(h->gslots, pl.slots.data(), sizeof(GbSlot) * pl.slots.size(),
+                              cudaMemcpyHostToDevice, st));
+    LRVB_CUDA(cudaStreamSynchronize(st));   // pl goes out of scope
+    npart = (size_t)nchunk * pl.n_groups * kGbWarps * 16 * 64;
+  }
+  LRVB_TRY(dev_alloc(&h->grampart, npart));
+  LRVB_CUDA(cudaMemsetAsync(h->grampart, 0, sizeof(double) * npart, st));
+  return LRVB_OK;
+}
+
+// ------------------------------------------------------------------------------------------
 int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_global,
                 double* grad_local, cudaStream_t st) {
   const int K = h->K, G = h->G, Q = h->Q, Dg = h->Dg;
@@ -1121,10 +1275,7 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
     fa.W = h->W; fa.ldw = h->ldw; fa.klpart = h->klpart; fa.gradpart = h->gradpart; fa.gsc = h->gsc; fa.BR = h->BR;
     fa.bval = h->bval; fa.grampart = h->grampart; fa.N = N; fa.K = K; fa.G = G; fa.Q = Q;
     fa.rows_per_q = h->fu_rows_per_team;
-    if (!launch_fused_eval(fa, h->fu_grid, Q, st)) {
-      set_error("launch_eval: one-pass kernel rejected K = %d / alignment", K);
-      return LRVB_ESTATE;
-    }
+    LRVB_CUDA(launch_pdl(h->fu_kernel, dim3(h->fu_grid), dim3(32 * h->fu_warps), h->fu_smem, st, fa));
     LRVB_CHECK_LAUNCH();
     if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[1], st));
     n_obs_cta = h->fu_grid;
@@ -1135,16 +1286,9 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
       if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[0], st));
       const int nch = (K + 1 + 31) / 32;
 #define LRVB_OF(O, C)                                                                          \
-  do {                                                                                         \
-    if (h->of1_warps > 0)                                                                      \
-      LRVB_CUDA(launch_pdl(k_obs_fused<O, C, 1>, dim3(h->of1_grid), dim3(32 * h->of1_warps), h->of1_smem, st, \
-          h->X, h->y, h->g, h->w, h->vec, h->gh, h->gptr, h->W, h->ldw, h->klpart, h->gradpart,    \
-          h->gsc, h->BR, h->bval, N, K, G, Q, h->of1_rows_per_warp));                          \
-    else                                                                                       \
-      LRVB_CUDA(launch_pdl(k_obs_fused<O, C>, dim3(h->of_grid), dim3(32 * h->of_warps), h->of_smem, st, \
-          h->X, h->y, h->g, h->w, h->vec, h->gh, h->gptr, h->W, h->ldw, h->klpart, h->gradpart,    \
-          h->gsc, h->BR, h->bval, N, K, G, Q, h->of_rows_per_warp));                           \
-  } while (0)
+  LRVB_CUDA(launch_pdl(k_obs_fused<O, C, 1>, dim3(h->of1_grid), dim3(32 * h->of1_warps), h->of1_smem, st, \
+                       h->X, h->y, h->g, h->w, h->vec, h->gh, h->gptr, h->W, h->ldw, h->klpart, h->gradpart, \
+                       h->gsc, h->BR, h->bval, N, K, G, Q, h->of1_rows_per_warp))
       if (nch == 1) {
         if (order == 0) LRVB_OF(0, 1);
         else if (order == 1) LRVB_OF(1, 1);
@@ -1157,11 +1301,8 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
 #undef LRVB_OF
       LRVB_CHECK_LAUNCH();
       if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[1], st));
-      n_obs_cta = h->of1_warps > 0 ? h->of1_grid : h->of_grid;
-    }
-    if (N > 0) {
-      const int64_t rpw = h->of1_warps > 0 ? h->of1_rows_per_warp : h->of_rows_per_warp;
-      fix_rpw = rpw > 0 ? rpw : 32;
+      n_obs_cta = h->of1_grid;
+      fix_rpw = h->of1_rows_per_warp > 0 ? h->of1_rows_per_warp : 32;
     }
   } else {
   if (N > 0) {
@@ -1199,10 +1340,8 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
       h->ev_gram = 1;
       if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[2], st));
       if (h->gram_mid) {
-        if (!launch_gram_mid(h->X, h->W + 2 * h->ldw, h->grampart, N, h->ldw, K, h->gram_grid_x, st)) {
-          set_error("launch_eval: mid-K Gram kernel rejected K = %d / alignment", K);
-          return LRVB_ESTATE;
-        }
+        LRVB_CUDA(launch_pdl(h->gm_kernel, dim3(h->gram_grid_x), dim3(32 * h->gm_warps), h->gram_smem, st,
+                             h->X, h->W + 2 * h->ldw, h->grampart, N, h->ldw, K));
       } else if (h->gram_wide) {
         LRVB_CUDA(launch_pdl(k_gram_wide, dim3(h->gram_grid_x), dim3(32 * kGwWarps), h->gram_smem, st,
             h->X, h->W + 2 * h->ldw, h->ldw, (const GwGroup*)h->jobs, (const GwCta*)h->gslots,
@@ -1287,32 +1426,3 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
 }
 
 }  // namespace lrvb
-
-namespace lrvb {
-void configure_obs_fused(size_t smem) {
-  const int v = (int)smem;
-  cudaFuncSetAttribute(k_obs_fused<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<0, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<0, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<2, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<0, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<1, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaFuncSetAttribute(k_obs_fused<2, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, v);
-  cudaGetLastError();
-}
-void configure_kernels(size_t obs_smem, size_t gram_smem) {
-  const int o = (int)obs_smem, gsm = (int)gram_smem;
-  cudaFuncSetAttribute(k_obs<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, o);
-  cudaFuncSetAttribute(k_obs<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, o);
-  cudaFuncSetAttribute(k_obs<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, o);
-  if (gsm > 0) cudaFuncSetAttribute(k_gram_big, cudaFuncAttributeMaxDynamicSharedMemorySize, gsm);
-  if (gsm > 0) cudaFuncSetAttribute(k_gram_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, gsm);
-  cudaGetLastError();
-}
-}  // namespace lrvb
-

@@ -319,25 +319,19 @@ k_gram_mid(const double* __restrict__ X, const double* __restrict__ Wabc, double
   for (int e = threadIdx.x; e < NT * 64; e += blockDim.x) out[e] = red[e];
 }
 
-// launch the instantiation for K (24 < K <= 104; below, the one-pass kernel of fused.cuh computes the Gram);
-// false when K / alignment is outside its range
-inline bool launch_gram_mid(const double* X, const double* Wabc, double* part, int64_t N, int64_t ldw,
-                            int K, int grid, cudaStream_t st) {
-  if (K < 1 || K > kGmMaxK || (ldw & 1) || (((uintptr_t)X) & 15) || (((uintptr_t)Wabc) & 15)) return false;
+// the instantiation for K (24 < K <= 104; below, the one-pass kernel of fused.cuh computes the Gram) and its CTA
+// size in warps; a null kernel outside that range
+struct GramMidKernel {
+  void (*fn)(const double*, const double*, double*, int64_t, int64_t, int);
+  int warps;
+};
+inline GramMidKernel gram_mid_kernel(int K) {
   const int T2 = (2 * K + 7) / 8, T0 = K / 8;
   const bool M = (K % 8) != 0;
-  const size_t smem = gram_mid_smem(K, T2);
 #define LRVB_GM(T2_, T0_, M_)                                                                       \
   if (T2 == T2_ && T0 == T0_ && M == M_) {                                                          \
     constexpr GramMidGeom g = gram_mid_geom(T2_);                                                   \
-    static size_t configured = 48 * 1024;                                                           \
-    if (smem > configured) {                                                                        \
-      cudaFuncSetAttribute(k_gram_mid<T2_, T0_, M_, g.warps, g.P>,                                  \
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                 \
-      configured = smem;                                                                            \
-    }                                                                                               \
-    return launch_pdl(k_gram_mid<T2_, T0_, M_, g.warps, g.P>, dim3(grid), dim3(32 * g.warps), smem, st, X, \
-                      Wabc, part, N, ldw, K) == cudaSuccess;                                        \
+    return {k_gram_mid<T2_, T0_, M_, g.warps, g.P>, g.warps};                                        \
   }
   LRVB_GM(7, 3, true)
   LRVB_GM(8, 3, true)
@@ -370,7 +364,7 @@ inline bool launch_gram_mid(const double* X, const double* Wabc, double* part, i
   LRVB_GM(26, 12, true)
   LRVB_GM(26, 13, false)
 #undef LRVB_GM
-  return false;
+  return {nullptr, 0};
 }
 
 }  // namespace lrvb

@@ -279,11 +279,7 @@ int lrvb_glmm_logo(lrvb_glmm* h, const double* Sinv_dev, const double* Pinv_dev,
   LRVB_TRY(launch_gemm(h->logo_V, Dg, Sinv_dev, Dg, delta_dev, Dg, G, Dg, Dg, -1.0, st));
   LRVB_TRY(launch_gemm(delta_dev + 4, Dg, Pinv_dev, K, h->logo_V, K, G, K, K, 1.0, st));
   const size_t smem = sizeof(double) * (2 * (size_t)Q + kLgWarps * logo_warp_doubles(K));
-  static size_t configured = 48 * 1024;
-  if (smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_logo_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
+  LRVB_TRY(raise_smem_limit(k_logo_rows, smem));
   k_logo_rows<<<cdiv(G, kLgWarps), 32 * kLgWarps, smem, st>>>(h->X, h->y, h->gptr, h->vec, delta_dev, h->logo_V, h->gh,
                                                               group_out_dev, row_out_dev, N, K, G, Q, h->bounds);
   LRVB_CHECK_LAUNCH();

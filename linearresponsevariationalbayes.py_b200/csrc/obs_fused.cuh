@@ -44,7 +44,9 @@ __host__ __device__ inline int obs_fused_warp_elems(int K, int slots = kOfStages
 }
 // One-slot variant (SLOTS = 1): from K ~ 36 on a two-slot ring leaves room for fewer than 10 warps per SM
 // (7 at K = 50) and the pass is latency-bound; with ONE slot per warp -- the next stage is requested when
-// the current one is finished, the other warps cover the copy -- up to 14 warps fit.
+// the current one is finished, the other warps cover the copy -- up to 14 warps fit.  It fits at least three
+// more warps than two slots for every K <= 62, so the evaluation always runs it; the weight-cross pass
+// (launch_weight_pass) and the influence pass (k_obs_influence) keep two slots.
 constexpr int kOfMaxWarps1 = 16;
 inline int obs_fused_warps(int K, int slots = kOfStages) {
   // all of the 227 KB a CTA may own (one CTA per SM): per warp its ring, weights, gradient partials (2K), KL

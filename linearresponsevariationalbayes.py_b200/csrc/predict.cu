@@ -362,11 +362,7 @@ static int launch_predict(lrvb_glmm* h, const double* freev, const double* X, co
   const int K = h->K, Q = h->Q;
   const int warps = pr_warps(K, Q, KP8);
   const size_t smem = warps * pr_warp_bytes(K) + pr_fixed_bytes(K, Q, KP8);
-  static size_t configured = 48 * 1024;   // per instantiation
-  if (smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_predict<LR, KP8, LOO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
+  LRVB_TRY(raise_smem_limit(k_predict<LR, KP8, LOO>, smem));
   int per_sm = 0;
   LRVB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_predict<LR, KP8, LOO>, 32 * warps, smem));
   if (per_sm < 1) per_sm = 1;
@@ -431,11 +427,7 @@ int lrvb_glmm_predict_cross(lrvb_glmm* h, const double* Sinv_dev, double* cross_
   }
   if (h->G == 0) return LRVB_OK;
   const size_t smem = sizeof(double) * 4 * 2 * (size_t)h->Dg;
-  static size_t configured = 48 * 1024;
-  if (smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_predict_cross, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
+  LRVB_TRY(raise_smem_limit(k_predict_cross, smem));
   int grid = cdiv(h->G, 4);
   if (grid > 8 * kNumSMs) grid = 8 * kNumSMs;
   k_predict_cross<<<grid, 128, smem, (cudaStream_t)stream>>>(Sinv_dev, h->B, h->L, cross_dev, h->K, h->G);

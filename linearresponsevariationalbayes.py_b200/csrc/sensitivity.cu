@@ -15,8 +15,8 @@
 
 namespace lrvb {
 
-// K > 62 (glmm_eval.cu): k_obs<1> + k_group<1> with dw as the weights; the influence pass on the k_obs tile walk
-int launch_wide_weight_pass(lrvb_glmm* h, const double* dw, double* scratchW, cudaStream_t st);
+// glmm_eval.cu: the observation and group passes with dw as the weights; the influence pass for K > 62
+int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t st);
 int launch_wide_influence(lrvb_glmm* h, const double* v, double* out, cudaStream_t st);
 
 // out = C dw from the sums of the fused pass run with weights dw (gradpart: X^T l_m, S^T l_v per
@@ -192,54 +192,10 @@ int lrvb_glmm_weight_cross_matvec(lrvb_glmm* h, const double* dw_dev, double* ou
     return LRVB_ESTATE;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  const int K = h->K, G = h->G, Q = h->Q;
-  const int64_t N = h->N;
   int n_gp = 0;
-  if (!h->obs_fused) {
-    // K > 62: the wide-model observation kernel + k_group with dw as the weights; l_m, l_v go to a scratch
-    // block so that the cached evaluation's W (lrvb_glmm_obs_weights) stays intact
-    if (!h->wc_scratch && N > 0) {
-      if (cudaMalloc(&h->wc_scratch, sizeof(double) * 2 * (size_t)h->ldw) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("lrvb_glmm_weight_cross_matvec: out of device memory (%zu bytes of scratch)",
-                  sizeof(double) * 2 * (size_t)h->ldw);
-        return LRVB_ECUDA;
-      }
-    }
-    LRVB_TRY(launch_wide_weight_pass(h, dw_dev, h->wc_scratch, st));
-    k_wc_finish<<<cdiv(h->D, 256), 256, 0, st>>>(h->vec, h->gradpart, N > 0 ? h->obs_grid : 0, h->gsc, out_dev, K, G,
-                                                 h->bounds, h->vecmode);
-    LRVB_CHECK_LAUNCH();
-    return LRVB_OK;
-  }
-  {
-    // this translation unit has its own instantiations of the fused kernel: raise their limits too
-    static size_t configured = 48 * 1024;
-    if (h->of_smem > configured) {
-      LRVB_CUDA(cudaFuncSetAttribute(k_obs_fused<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->of_smem));
-      LRVB_CUDA(cudaFuncSetAttribute(k_obs_fused<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->of_smem));
-      configured = h->of_smem;
-    }
-  }
-  if (N > 0) {
-    if ((K + 1 + 31) / 32 == 1)
-      k_obs_fused<1, 1><<<h->of_grid, 32 * h->of_warps, h->of_smem, st>>>(
-          h->X, h->y, h->g, dw_dev, h->vec, h->gh, h->gptr, nullptr, h->ldw, h->klpart, h->gradpart,
-          h->gsc, h->BR, h->bval, N, K, G, Q, h->of_rows_per_warp);
-    else
-      k_obs_fused<1, 2><<<h->of_grid, 32 * h->of_warps, h->of_smem, st>>>(
-          h->X, h->y, h->g, dw_dev, h->vec, h->gh, h->gptr, nullptr, h->ldw, h->klpart, h->gradpart,
-          h->gsc, h->BR, h->bval, N, K, G, Q, h->of_rows_per_warp);
-    LRVB_CHECK_LAUNCH();
-    n_gp = h->of_grid;
-  }
-  if (G > 0) {
-    k_obs_fixup<1><<<cdiv(G, 8), 256, 0, st>>>(h->gptr, h->bval, h->gsc, h->BR, K, G,
-                                               h->of_rows_per_warp > 0 ? h->of_rows_per_warp : 32);
-    LRVB_CHECK_LAUNCH();
-  }
-  k_wc_finish<<<cdiv(h->D, 256), 256, 0, st>>>(h->vec, h->gradpart, n_gp, h->gsc, out_dev, K, G,
-                                               h->bounds, h->vecmode);
+  LRVB_TRY(launch_weight_pass(h, dw_dev, &n_gp, st));
+  k_wc_finish<<<cdiv(h->D, 256), 256, 0, st>>>(h->vec, h->gradpart, n_gp, h->gsc, out_dev, h->K, h->G, h->bounds,
+                                               h->vecmode);
   LRVB_CHECK_LAUNCH();
   return LRVB_OK;
 }
@@ -254,11 +210,7 @@ int lrvb_glmm_weight_cross_rmatvec(lrvb_glmm* h, const double* v_dev, double* ou
   if (h->N == 0) return LRVB_OK;
   if (!h->obs_fused) return launch_wide_influence(h, v_dev, out_dev, (cudaStream_t)stream);
   const size_t smem = h->of_smem + sizeof(double) * (2 * (size_t)h->K + 2);
-  static size_t configured = 48 * 1024;
-  if (smem > configured) {
-    LRVB_CUDA(cudaFuncSetAttribute(k_obs_influence, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
+  LRVB_TRY(raise_smem_limit(k_obs_influence, smem));
   k_obs_influence<<<h->of_grid, 32 * h->of_warps, smem, (cudaStream_t)stream>>>(
       h->X, h->y, h->g, h->vec, h->gh, v_dev, out_dev, h->N, h->K, h->G, h->Q, h->of_rows_per_warp,
       h->bounds, h->vecmode);
