@@ -278,6 +278,12 @@ int lrvb_glmm_loo(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev,
  * (G, Dg) scratch in the handle on first use. */
 int lrvb_glmm_logo(lrvb_glmm* h, const double* Sinv_dev, const double* Pinv_dev, double* delta_dev,
                    double* group_out_dev, double* row_out_dev, void* stream);
+/* The third derivative of the KL along a_dev (D), at the point of the last evaluation (free coordinates;
+ * LRVB_ESTATE otherwise): t_dev (D) = D^3 KL[a, a, .] and q_dev (N) = a^T (grad^2 l_n) a, the unweighted per-row
+ * quadratic form, in the handle's (group-sorted) row order.  With a = H^-1 c it gives how the LRVB variance
+ * c^T H^-1 c moves with the observation weights: d/dw_n = q_n - grad l_n . (H^-1 t).  No atomics: repeated calls are
+ * bitwise equal.  LRVB_EINVAL for NULL pointers; allocates a (2N + 5G + O(K)) scratch in the handle on first use. */
+int lrvb_glmm_third_contract(lrvb_glmm* h, const double* a_dev, double* t_dev, double* q_dev, void* stream);
 
 /* ---- batched exponential-family terms (ExponentialFamilies.py) --------------------------
  * All pointers dev; M = number of factors. */

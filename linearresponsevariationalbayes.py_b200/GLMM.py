@@ -67,6 +67,21 @@ delta_global (G, Dg) = the IJ shift of the global free parameters.  Scalars: elp
 sqrt(G') std(elpd_logo_group over the G' non-empty groups, ddof=1) (NaN when G' < 2).  An empty group has zero
 delta_global, cooks_distance and elpd_logo_group."""
 
+DropResult = namedtuple("DropResult", ["n_drop", "fraction", "dropped", "predicted_estimate", "predicted_sd"])
+DropResult.__doc__ = """One target of ``LinearResponseCovariances.get_approximate_max_influence``: the fewest units (rows or
+groups) whose removal the first-order prediction says is enough to reach the target, n_drop (None if no such set
+within max_fraction), fraction = n_drop over the units of non-zero weight, dropped = their indices (caller's row order
+or group ids, most influential first), and the predicted estimate and sd_lr without them (None with n_drop)."""
+
+ApproximateMaxInfluence = namedtuple("ApproximateMaxInfluence", ["estimate", "sd_lr", "z", "mean_shift", "sd_shift",
+                                                                 "targets"])
+ApproximateMaxInfluence.__doc__ = """The approximate maximum influence perturbation (AMIP) of phi = c^T E[beta]
+(``LinearResponseCovariances.get_approximate_max_influence``).  Scalars: estimate = phi, sd_lr = its LRVB standard
+deviation sqrt(c^T H^-1 c), z = the normal quantile of the interval phi +/- z sd_lr.  Per unit (rows in the caller's
+order, or groups by id): mean_shift and sd_shift, the first-order changes of phi and sd_lr when the unit is dropped
+(its weights set to 0).  targets: dict of ``DropResult`` for "sign" (phi crosses 0), "significance" (the interval
+bound nearest 0 crosses it) and "significant_opposite" (the far bound crosses 0)."""
+
 
 class _DevView(object):
     """Zero-copy torch view of library-owned device memory (__cuda_array_interface__)."""
@@ -639,6 +654,25 @@ class LogisticGLMM(object):
             res.index_copy_(0, to_device(self.perm, torch.int64), out)
             return res
         return out
+
+    def third_derivative_contraction(self, a):
+        """(t (D,), q (N,)) at the point and in the free coordinates of the last evaluation: t = D^3 KL[a, a, .], the
+        derivative of a^T H a, and q_n = a^T (grad^2 l_n) a, the unweighted quadratic form of every row's
+        log-likelihood term (caller's row order); CUDA tensors.  One pass over the rows plus one over the groups
+        (csrc/amip.cu).  With a = H^-1 c, d (c^T H^-1 c) / d w_n = q_n + (C^T H^-1 t)_n (``weight_cross_rmatvec``)."""
+        torch = nat.require_cuda()
+        ad = to_device(a).reshape(-1).contiguous()
+        if ad.numel() != self.D:
+            raise ValueError("Wrong size for parameter {}.  Expected {}, got {}".format(
+                self.glmm_par.name, self.D, ad.numel()))
+        t = torch.empty(self.D, dtype=torch.float64, device=self.device)
+        q = torch.empty(self.N, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_third_contract(self._h, nat.ptr(ad), nat.ptr(t), nat.ptr(q), nat.stream_ptr()))
+        if self.perm is not None:
+            res = torch.empty_like(q)
+            res.index_copy_(0, to_device(self.perm, torch.int64), q)
+            q = res
+        return t, q
 
     # names shared with distributed.ShardedLogisticGLMM (where they add the all-reduce)
     def hvp(self, v):

@@ -15,7 +15,8 @@ device conjugate gradient -- the dense ``cho_factor`` of the reference is O(D^3)
 import numpy as np
 import scipy.sparse
 
-from ._tensors import is_torch
+from .GLMM import ApproximateMaxInfluence, DropResult
+from ._tensors import is_torch, to_device
 
 
 class LinearResponseCovariances(object):
@@ -244,6 +245,113 @@ class LinearResponseCovariances(object):
         return r._replace(**{f: getattr(r, f).cpu().numpy() for f in ("lpd_logo", "eta_mean_logo", "eta_var_logo",
                                                                       "elpd_logo_group", "cooks_distance",
                                                                       "delta_global")})
+
+    def get_approximate_max_influence(self, c, unit="row", level=0.95, max_fraction=0.1):
+        """The approximate maximum influence perturbation (AMIP, Broderick, Giordano and Meager) of the contrast
+        phi = c^T E[beta] at the optimum: how few rows (unit="row") or whole groups (unit="group") must be dropped to
+        change its sign, its significance at ``level``, or to make it significant with the opposite sign.  ``c`` is a
+        length-K vector or an integer k (e_k).  Returns a ``GLMM.ApproximateMaxInfluence``; per-unit fields are numpy
+        for a numpy optimum and CUDA tensors for a CUDA one.
+
+        With a = H^-1 chat (chat = c on the beta.mean block), b = H^-1 t and t = D^3 KL[a, a, .]
+        (``model.third_derivative_contraction``), dropping unit u (w_n -> 0 on its rows) moves phi and
+        sd_lr^2 = chat^T H^-1 chat to first order by sum_{n in u} w_n (C^T a)_n and -sum_{n in u} w_n (q_n + (C^T b)_n)
+        (C = d^2 KL / d theta d w, ``weight_cross_rmatvec``).  Each target is a linear statistic -- s phi,
+        s phi - z sd_lr, s phi + z sd_lr with s = sign(phi) -- and its search sorts the units of non-zero weight by
+        their push toward zero (ties by index) and takes the shortest prefix that carries the statistic across zero,
+        of at most floor(max_fraction * units) units.  Always from the direct arrowhead pieces, whatever ``method``
+        is."""
+        import scipy.special
+        import torch
+        model = self.model
+        if getattr(model, "local", None) is not None:
+            raise NotImplementedError("approximate maximum influence of a sharded model: build a single-GPU "
+                                      "LogisticGLMM of the job and use its LinearResponseCovariances")
+        if unit not in ("row", "group"):
+            raise ValueError("unit must be 'row' or 'group', got %r" % (unit,))
+        level, max_fraction = float(level), float(max_fraction)
+        if not 0.0 < level < 1.0:
+            raise ValueError("level must lie in (0, 1), got %r" % (level,))
+        if not 0.0 < max_fraction <= 1.0:
+            raise ValueError("max_fraction must lie in (0, 1], got %r" % (max_fraction,))
+        chat = self._contrast(c)
+        self._ensure_point()
+        if self._sinv is None:
+            self._sinv = model.global_covariance()
+        dev = model.device
+        ch = torch.from_numpy(chat).to(dev)
+
+        def solve(rhs):
+            return model.solve_finish(self._sinv, model.solve_reduce_rhs(rhs), rhs)
+
+        a = solve(ch)
+        x = self._opt0.detach().to(dev, torch.float64) if is_torch(self._opt0) else \
+            torch.from_numpy(np.asarray(self._opt0, dtype=np.float64)).to(dev)
+        t, q = model.third_derivative_contraction(a)
+        b = solve(t)
+        ca, cb = model.weight_cross_rmatvec(a), model.weight_cross_rmatvec(b)
+        w = torch.ones(model.N, dtype=torch.float64, device=dev) if model.w is None else model.w
+        perm = None if model.perm is None else to_device(model.perm, torch.int64)
+        if perm is not None:                     # caller's row order
+            w = torch.empty_like(w).index_copy_(0, perm, w)
+        est, var = float(torch.dot(ch, x.reshape(-1))), float(torch.dot(ch, a))
+        if not var > 0.0:
+            raise np.linalg.LinAlgError("the LRVB variance of the contrast is {} (not positive)".format(var))
+        sd = float(np.sqrt(var))
+        mean_shift = w * ca
+        sd_shift = -w * (q + cb) / (2.0 * sd)
+        keep = w != 0
+        if unit == "group":
+            # the model's rows are group-sorted: fixed-order segment sums, no atomics
+            counts = torch.bincount(model.g.to(torch.int64), minlength=model.G)
+            srt = (lambda v: v) if perm is None else (lambda v: v.index_select(0, perm))
+            gsum = lambda v: torch.segment_reduce(srt(v), "sum", lengths=counts, initial=0.0)   # noqa: E731
+            mean_shift, sd_shift = gsum(mean_shift), gsum(sd_shift)
+            keep = gsum(keep.to(torch.float64)) > 0
+        z = float(scipy.special.ndtri(0.5 + 0.5 * level))
+        s = 1.0 if est >= 0 else -1.0
+        linear = dict(sign=(s * est, s * mean_shift),
+                      significance=(s * est - z * sd, s * mean_shift - z * sd_shift),
+                      significant_opposite=(s * est + z * sd, s * mean_shift + z * sd_shift))
+        elig = torch.nonzero(keep).reshape(-1)
+        nmax = int(np.floor(max_fraction * elig.numel() + 1e-9))
+        host = not is_torch(self._opt0)
+        targets = {}
+        for name, (stat, push) in linear.items():
+            side = 1.0 if stat >= 0 else -1.0
+            key, order = torch.sort(side * push.index_select(0, elig), stable=True)
+            hit = torch.nonzero(side * stat + torch.cumsum(key[:nmax], 0) < 0).reshape(-1)
+            if hit.numel() == 0:
+                drop = elig[:0]
+                targets[name] = DropResult(None, None, drop.cpu().numpy() if host else drop, None, None)
+                continue
+            n = int(hit[0]) + 1
+            drop = elig.index_select(0, order[:n])
+            targets[name] = DropResult(n, n / elig.numel(), drop.cpu().numpy() if host else drop,
+                                       est + float(mean_shift.index_select(0, drop).sum()),
+                                       sd + float(sd_shift.index_select(0, drop).sum()))
+        if host:
+            mean_shift, sd_shift = mean_shift.cpu().numpy(), sd_shift.cpu().numpy()
+        return ApproximateMaxInfluence(est, sd, z, mean_shift, sd_shift, targets)
+
+    def _contrast(self, c):
+        """c (length K, numpy / list / torch) or an integer k -> chat (D,) numpy with c on the beta.mean block."""
+        K, D = self.model.K, self.model.D
+        chat = np.zeros(D)
+        if isinstance(c, (int, np.integer)) and not isinstance(c, (bool, np.bool_)):
+            if not 0 <= int(c) < K:
+                raise ValueError("coefficient index must lie in [0, {}), got {}".format(K, int(c)))
+            chat[4 + int(c)] = 1.0
+            return chat
+        v = c.detach().cpu().numpy() if is_torch(c) else np.asarray(c)
+        if v.ndim != 1 or v.shape[0] != K or not np.issubdtype(v.dtype, np.number) or \
+                np.issubdtype(v.dtype, np.complexfloating):
+            raise ValueError("c must be an integer in [0, {0}) or a real vector of length {0}".format(K))
+        v = v.astype(np.float64)
+        if not np.all(np.isfinite(v)) or not np.any(v != 0):
+            raise ValueError("c must be finite and not all zero")
+        chat[4:4 + K] = v
+        return chat
 
     MAX_DENSE = 1 << 26
 

@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "lib", "liblrvb_b200.so")
 SOURCES = ["api.cu", "glmm_eval.cu", "solve.cu", "csr.cu", "ef.cu", "sensitivity.cu", "p2p.cu", "packing.cu",
-           "predict.cu", "logo.cu"]
+           "predict.cu", "logo.cu", "amip.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xptxas", "-v",

@@ -135,6 +135,39 @@ __host__ __device__ inline PsiLg digamma_lgamma_pos(double x, bool want_lg) {
   return o;
 }
 
+// psi', psi'' and psi''' for x > 0, branch-free like digamma_lgamma_pos (the third derivative of the gamma entropy
+// and of E log tau, amip.cu): shift by eight (psi^(n)(x) = psi^(n)(x+8) + (-1)^(n+1) n! sum_{k<8} (x+k)^-(n+1)),
+// then the asymptotic series at y = x + 8 >= 8 through the Bernoulli number B_20: the first omitted term is
+// below 1e-16 (psi'), 3e-15 (psi''), 3e-14 (psi''') relative.
+struct Psi123 {
+  double p1, p2, p3;
+};
+__host__ __device__ inline Psi123 polygamma123_pos(double x) {
+  double s2 = 0.0, s3 = 0.0, s4 = 0.0;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    const double r = 1.0 / (x + (double)k), rr = r * r;
+    s2 += rr;
+    s3 = fma(rr, r, s3);
+    s4 = fma(rr, rr, s4);
+  }
+  const double y = x + 8.0, r = 1.0 / y, r2 = r * r;
+  const double b1 = 1.0 / 6.0 + r2 * (-1.0 / 30.0 + r2 * (1.0 / 42.0 + r2 * (-1.0 / 30.0 + r2 * (5.0 / 66.0 +
+                    r2 * (-691.0 / 2730.0 + r2 * (7.0 / 6.0 + r2 * (-3617.0 / 510.0 + r2 * (43867.0 / 798.0 +
+                    r2 * (-174611.0 / 330.0)))))))));
+  const double b2 = 0.5 + r2 * (-1.0 / 6.0 + r2 * (1.0 / 6.0 + r2 * (-3.0 / 10.0 + r2 * (5.0 / 6.0 +
+                    r2 * (-691.0 / 210.0 + r2 * (35.0 / 2.0 + r2 * (-3617.0 / 30.0 + r2 * (43867.0 / 42.0 +
+                    r2 * (-1222277.0 / 110.0)))))))));
+  const double b3 = 2.0 + r2 * (-1.0 + r2 * (4.0 / 3.0 + r2 * (-3.0 + r2 * (10.0 +
+                    r2 * (-691.0 / 15.0 + r2 * (280.0 + r2 * (-10851.0 / 5.0 + r2 * (438670.0 / 21.0 +
+                    r2 * (-1222277.0 / 5.0)))))))));
+  Psi123 o;
+  o.p1 = r + 0.5 * r2 + r * r2 * b1 + s2;
+  o.p2 = -r2 - r * r2 - r2 * r2 * b2 - 2.0 * s3;
+  o.p3 = 2.0 * r * r2 + 3.0 * r2 * r2 + r * r2 * r2 * b3 + 6.0 * s4;
+  return o;
+}
+
 #ifdef __CUDACC__
 // ---- programmatic dependent launch (PDL) ------------------------------------------------------
 // Every kernel of the evaluation / CSR chain starts with pdl_sync(): it lets the NEXT kernel of the
@@ -324,6 +357,7 @@ struct lrvb_glmm {
   double* schurpart = nullptr;
   double* pred_B = nullptr;   // (3 Kp8, Kp4) scaled beta block of S^-1 for lrvb_glmm_predict_lr (predict.cu)
   double* logo_V = nullptr;   // (G, Dg) per-group gradients of lrvb_glmm_logo, then its (G, K) Cook's products (logo.cu)
+  double* amip_work = nullptr;   // row coefficients, per-CTA and per-group partials of lrvb_glmm_third_contract (amip.cu)
 };
 
 namespace lrvb {

@@ -494,6 +494,10 @@ class ShardedLogisticGLMM(object):
         raise NotImplementedError("approximate LOGO of a sharded model: build a single-GPU LogisticGLMM of the job "
                                   "and use LinearResponseCovariances.get_approximate_logo")
 
+    def third_derivative_contraction(self, *args, **kwargs):
+        raise NotImplementedError("the third derivative of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                  "and use LinearResponseCovariances.get_approximate_max_influence")
+
     def moment_jacobian(self, free):
         import scipy.sparse
         free = np.asarray(free, dtype=np.float64).reshape(-1)
