@@ -54,6 +54,15 @@ constexpr int kRT = 4;        // Schur warp job = kRT x kRT output tiles of 8x8 
 
 static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
+// Shared memory of k_obs (the observation pass for K > 62, glmm_eval.cu): nbuf 64-row tiles of X, the Q
+// quadrature nodes and weights (each padded to whole node slots of 4), 32 reduction values and 2 spare.
+inline size_t obs_smem(int K, int Q, int nbuf) {
+  return sizeof(double) * ((size_t)nbuf * 64 * K + 2 * (size_t)(Q + 3) + 32 + 2);
+}
+// Tile buffers of k_obs: two (tile t + 1 in flight while tile t is computed) when they fit in 220 KB, else one
+// (from K = 220 on, and at K = 219 for Q > 44).
+inline int obs_tile_buffers(int K, int Q) { return obs_smem(K, Q, 2) <= 220 * 1024 ? 2 : 1; }
+
 template <typename T>
 static int dev_alloc(T** p, size_t n) {
   *p = nullptr;

@@ -613,7 +613,7 @@ k_fused_eval(const FusedArgs a) {
 inline auto fused_eval_kernel(int K) -> void (*)(FusedArgs) {
   const int T2 = (2 * K + 7) / 8, T0 = K / 8;
   const bool M = (K % 8) != 0;
-  const int nch = (K + 1 + 31) / 32;
+  const int nch = obs_fused_chunks(K);
 #define LRVB_FU(T2_, T0_, M_, NCH_)                                                                  \
   if (T2 == T2_ && T0 == T0_ && M == M_ && nch == NCH_) {                                            \
     return k_fused_eval<T2_, T0_, M_, NCH_, kFuGeom.teams, kFuGeom.NQ, kFuGeom.P, kFuGeom.warps,       \

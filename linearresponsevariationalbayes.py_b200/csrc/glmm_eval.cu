@@ -77,7 +77,8 @@ __global__ void k_prep(const double* __restrict__ free_v, double* __restrict__ v
 
 // Observation pass for K > 62 (the fused kernels of obs_fused.cuh / fused.cuh cover K <= 62).  A CTA of 8
 // warps walks 64-row tiles of X, double-buffered in shared memory (TMA bulk copies on an mbarrier per buffer, cp.async
-// for odd K; tile t + 1 is in flight while tile t is computed; one buffer when two do not fit, K > 214).  Per tile every warp owns 8 rows:
+// for odd K; tile t + 1 is in flight while tile t is computed; one buffer when two do not fit, obs_tile_buffers).
+// Per tile every warp owns 8 rows:
 //   A. z_mean / z_var dot products with lane = column (coalesced, conflict-free), then ONE transposing
 //      butterfly (16 exchanges instead of 16 x 5) that leaves row rr's two sums in lanes 4 rr .. 4 rr + 3;
 //   B. quadrature with lane = (row, node slot): the 4 lanes of a row split the Q nodes (branch-free exp /
@@ -541,7 +542,7 @@ int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t s
   *n_gp = 0;
   if (h->obs_fused) {
     if (N > 0) {
-      auto kern = (K + 1 + 31) / 32 == 1 ? k_obs_fused<1, 1> : k_obs_fused<1, 2>;
+      auto kern = obs_fused_chunks(K) == 1 ? k_obs_fused<1, 1> : k_obs_fused<1, 2>;
       LRVB_TRY(raise_smem_limit(kern, h->of_smem));
       kern<<<h->of_grid, 32 * h->of_warps, h->of_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, h->gptr, nullptr,
                                                              h->ldw, h->klpart, h->gradpart, h->gsc, h->BR, h->bval,
@@ -1100,9 +1101,8 @@ int plan_eval(lrvb_glmm* h, cudaStream_t st) {
   const int64_t N = h->N;
   // observation pass geometry (k_obs, K > 62: 64-row tiles; obs_nbuf = tile buffers, two when they fit)
   {
-    const size_t tile = sizeof(double) * 64 * (size_t)K, extra = sizeof(double) * (2 * (size_t)(Q + 3) + 32 + 2);
-    h->obs_nbuf = (2 * tile + extra <= 220 * 1024) ? 2 : 1;
-    h->obs_smem = h->obs_nbuf * tile + extra;
+    h->obs_nbuf = obs_tile_buffers(K, Q);
+    h->obs_smem = obs_smem(K, Q, h->obs_nbuf);
     int64_t nt = (N + 63) / 64;
     h->obs_grid = (int)(nt < kNumSMs ? nt : kNumSMs);
     if (h->obs_grid < 1) h->obs_grid = 1;
@@ -1134,7 +1134,7 @@ int plan_eval(lrvb_glmm* h, cudaStream_t st) {
       h->of1_smem = obs_fused_smem(K, Q, w1, 1);
       if (tw1 > nrec) nrec = tw1;
       if (h->obs_grid < h->of1_grid) h->obs_grid = h->of1_grid;
-      if ((K + 1 + 31) / 32 == 1) {
+      if (obs_fused_chunks(K) == 1) {
         LRVB_TRY(raise_smem_limit(k_obs_fused<0, 1, 1>, h->of1_smem));
         LRVB_TRY(raise_smem_limit(k_obs_fused<1, 1, 1>, h->of1_smem));
         LRVB_TRY(raise_smem_limit(k_obs_fused<2, 1, 1>, h->of1_smem));
@@ -1284,7 +1284,7 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
     // K <= 62: observation pass and per-group sums in one kernel (obs_fused.cuh)
     if (N > 0) {
       if (h->timing) LRVB_CUDA(cudaEventRecord(h->ev[0], st));
-      const int nch = (K + 1 + 31) / 32;
+      const int nch = obs_fused_chunks(K);
 #define LRVB_OF(O, C)                                                                          \
   LRVB_CUDA(launch_pdl(k_obs_fused<O, C, 1>, dim3(h->of1_grid), dim3(32 * h->of1_warps), h->of1_smem, st, \
                        h->X, h->y, h->g, h->w, h->vec, h->gh, h->gptr, h->W, h->ldw, h->klpart, h->gradpart, \

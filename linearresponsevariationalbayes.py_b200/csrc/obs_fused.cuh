@@ -35,6 +35,8 @@ constexpr int kOfStages = 2;
 constexpr int kOfMaxWarps = LRVB_OF_WARPS;
 constexpr int kOfUnroll = LRVB_OF_UNROLL;   // quadrature nodes in flight per lane
 constexpr int kOfMaxK = 62;      // K + 1 columns in at most two 32-lane chunks
+// 32-lane column chunks of the K + 1 columns (the NCH template argument of the fused kernels)
+__host__ __device__ constexpr int obs_fused_chunks(int K) { return (K + 1 + 31) / 32; }
 
 // doubles per stage: X rows | y | w | g (int32, 16 doubles)
 __host__ __device__ inline int obs_fused_stage_elems(int K) { return kOfRows * K + 2 * kOfRows + kOfRows / 2; }

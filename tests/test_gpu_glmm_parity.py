@@ -51,10 +51,10 @@ CASES = {
     "k52_team": dict(N=1999, K=52, G=20, Q=4, seed=31),
     "k50_team_ring_wrap": dict(N=70003, K=50, G=70, Q=4, seed=32, weights=True),
     "k28_ring_wrap": dict(N=120011, K=28, G=120, Q=4, seed=33),
-    # teams of four (T2 14..18) and eight (T2 19..26) warps with tile-range roles
+    # teams of four (T2 14..20) and eight (T2 21..26) warps with tile-range roles (gram_mid_geom)
     "k56_team4": dict(N=1503, K=56, G=15, Q=4, seed=34),
     "k72_team4": dict(N=1200, K=72, G=12, Q=4, seed=35, weights=True),
-    "k77_team8": dict(N=1101, K=77, G=11, Q=4, seed=36),
+    "k77_team4_straddle": dict(N=1101, K=77, G=11, Q=4, seed=36),
     "k104_team8_ring_wrap": dict(N=30011, K=104, G=30, Q=4, seed=37),
     "k72_team4_ring_wrap": dict(N=40009, K=72, G=40, Q=4, seed=46, weights=True),
     # k_gram_wide (K = 176 .. 240, K % 8 == 0): blocks of 5,5,4,4,4 tiles (K = 176: mixed 5x4 / 4x5 / 4x4 jobs),
@@ -71,6 +71,49 @@ CASES = {
     "k80_q6": dict(N=1003, K=80, G=10, Q=6, seed=43, weights=True),
     "k65_q3": dict(N=700, K=65, G=7, Q=3, seed=44),
     "k96_q13": dict(N=1500, K=96, G=15, Q=13, seed=45, ragged=True),
+    # Every compiled kernel instantiation, k_gram_big plan and Gauss-Hermite edge below has a case;
+    # test_host_api.py::test_dispatch_cases_reach_every_kernel_class checks that against tools/dispatch_table.cu.
+    # k_fused_eval (T2 = 4, T0 = 1, straddle tile) with Q = 7: the quadrature loops of both fused kernels
+    # (4 nodes at a time, then 2, then 1) all run
+    "k13_fused_straddle_q7": dict(N=2000, K=13, G=20, Q=7, seed=47, weights=True),
+    # a single node (Q = 1) and the most nodes (Q = kMaxQ = 64) through k_fused_eval and k_obs_fused
+    "k15_fused_q1": dict(N=1501, K=15, G=15, Q=1, seed=48, ragged=True),
+    "k24_fused_q64": dict(N=2400, K=24, G=24, Q=64, seed=49),
+    # k_gram_mid teams of two / four with a straddle tile, and 64 = 8 T0 without one; two-chunk k_obs_fused
+    # at Q = 64 and Q = 1, k_obs at Q = 1 (three of its four node slots empty)
+    "k53_team2_q64": dict(N=1600, K=53, G=16, Q=64, seed=50),
+    "k58_team4_straddle_q1": dict(N=1700, K=58, G=17, Q=1, seed=51, weights=True),
+    "k64_team4_q1": dict(N=1800, K=64, G=18, Q=1, seed=52),
+    "k75_team4_straddle_q7": dict(N=1500, K=75, G=15, Q=7, seed=53, ragged=True),
+    # k_gram_mid teams of eight: every tile grid T2 = 21 .. 26 with a straddle tile, and T2 = 22 without one
+    "k82_team8_straddle": dict(N=1200, K=82, G=12, Q=4, seed=54),
+    "k87_team8_straddle": dict(N=1301, K=87, G=13, Q=5, seed=55, weights=True),
+    "k88_team8": dict(N=1400, K=88, G=14, Q=8, seed=56),
+    "k90_team8_straddle": dict(N=1203, K=90, G=12, Q=3, seed=57),
+    "k95_team8_straddle_ragged": dict(N=1500, K=95, G=15, Q=6, seed=58, ragged=True),
+    "k99_team8_straddle_q16": dict(N=1100, K=99, G=11, Q=16, seed=59),
+    # one team of eight per CTA: 148 teams x 32 rows x 3 slots = 14,208 rows fill every ring once, N = 30011
+    # gives every team 6 - 7 stages, so each ring wraps; odd K (rows not bulk-copied)
+    "k101_team8_straddle_ring_wrap": dict(N=30011, K=101, G=30, Q=4, seed=60, weights=True),
+    # k_gram_big plans (n_groups / rows per stage TN / straddle tile), one case per plan of gram_big_plan.
+    # TN = 32 (K = 105 .. 128): gram_big_plan(105) has 3 job groups, so 148 / 3 = 49 row chunks of 32-row
+    # stages; 49 x 32 = 1568 rows per round of stages, and N = 10007 (313 stages) gives every chunk 6 - 7
+    # stages, so each 3-slot ring wraps; odd K (rows loaded by the warps, not by TMA)
+    "k105_big_g3_tn32_straddle_ring_wrap": dict(N=10007, K=105, G=20, Q=4, seed=61),
+    "k112_big_g2_tn32": dict(N=1200, K=112, G=12, Q=8, seed=62),
+    "k120_big_g3_tn32": dict(N=1300, K=120, G=13, Q=4, seed=63, weights=True),
+    "k139_big_g4_straddle": dict(N=1401, K=139, G=14, Q=4, seed=64),
+    "k144_big_g4": dict(N=1200, K=144, G=12, Q=5, seed=65, ragged=True),
+    "k168_big_g5": dict(N=1100, K=168, G=11, Q=4, seed=66),
+    "k171_big_g5_straddle": dict(N=1100, K=171, G=11, Q=4, seed=67, weights=True),
+    "k186_big_g6_straddle": dict(N=1200, K=186, G=12, Q=4, seed=68),
+    "k201_big_g7_straddle": dict(N=1003, K=201, G=10, Q=6, seed=69),
+    # K = 219 is the last K where k_obs keeps two tile buffers at Q = 8; at Q = 64 it has one
+    "k219_big_g8_straddle_q64_one_buffer": dict(N=1100, K=219, G=11, Q=64, seed=70),
+    "k235_big_g9_straddle_q1": dict(N=1000, K=235, G=10, Q=1, seed=71, ragged=True),
+    "k250_big_g10_straddle": dict(N=1000, K=250, G=10, Q=4, seed=72),
+    # K = kMaxK, Q = kMaxQ: 9 job groups without a straddle tile, k_obs with one tile buffer
+    "k256_big_g9_q64": dict(N=1200, K=256, G=12, Q=64, seed=73, weights=True),
 }
 
 
@@ -114,10 +157,11 @@ def test_hessian_csr_bit_exact_pattern_and_values(setup):
 
 def test_structural_nnz_formula(setup):
     case, oracle, model, obj = setup
-    # SURVEY A.3: nnz = 4K^2 + 14 + G(8K + 14) when every group is non-empty and no X column
-    # is identically zero
+    # SURVEY A.3: nnz = 4K^2 + 14 + G(8K + 14) when every group is non-empty, no X column
+    # is identically zero and Q > 1 (the single node of Q = 1 sits at 0, which makes the x-s and s-s
+    # blocks exactly zero; test_hessian_csr_bit_exact_pattern_and_values checks that pattern)
     counts = np.bincount(case["g"], minlength=case["G"])
-    if (counts > 0).all():
+    if (counts > 0).all() and case["gh_x"].size > 1:
         K, G = case["K"], case["G"]
         H = obj.fun_free_hessian(case["free"])
         assert H.nnz == 4 * K * K + 14 + G * (8 * K + 14)

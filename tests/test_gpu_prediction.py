@@ -34,8 +34,9 @@ def _oracle_predict(case, x, X, g):
     return po.predict(x, X, g, case["K"], case["G"], case["gh_x"], case["gh_w"], _bounds(case))
 
 
-@pytest.mark.parametrize("K", [1, 5, 20, 50, 130, 200, 256])
-@pytest.mark.parametrize("Q,bounds", [(4, 0.0), (8, 0.1)])
+# K = 9 .. 16 round the row stride up to 16 columns (pr_kp8); Q = 1 and Q = kMaxQ = 64 are the node-count edges
+@pytest.mark.parametrize("K", [1, 5, 9, 12, 13, 16, 20, 50, 130, 200, 256])
+@pytest.mark.parametrize("Q,bounds", [(4, 0.0), (8, 0.1), (1, 0.0), (64, 0.1)])
 def test_predict_matches_oracle(vb, K, Q, bounds):
     case = make_case(N=1500, K=K, G=40, Q=Q, seed=500 + K + Q, shuffle=True, bounds=bounds, empty_groups=3)
     model = make_model(vb, case)
@@ -70,6 +71,9 @@ def _optimum(vb, case):
     ("k50", dict(N=6000, K=50, G=60, Q=8, seed=3001)),
     ("k130", dict(N=4000, K=130, G=20, Q=4, seed=23)),
     ("k200", dict(N=12_000, K=200, G=30, Q=8, seed=4001)),
+    # the LR pass with Bt staged for KP8 = 16: K padded to 4 (12) short of KP8, and K = KP8
+    ("k12", dict(N=3000, K=12, G=30, Q=8, seed=1201)),
+    ("k16", dict(N=3000, K=16, G=30, Q=4, seed=1601)),
 ])
 def test_lr_variances_at_the_optimum(vb, name, kw):
     case = make_case(**kw)

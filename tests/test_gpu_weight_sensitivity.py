@@ -17,6 +17,11 @@ CASES = {
     "k80_wide": dict(N=903, K=80, G=10, Q=6, seed=34, weights=True, bounds=0.05),
     "k200_wide_ragged": dict(N=777, K=200, G=9, Q=8, seed=35, ragged=True),
     "k65_odd": dict(N=300, K=65, G=5, Q=5, seed=36),
+    # the last K of the fused two-slot pass and the first of k_obs<1> + k_group<1> / k_obs_influence_wide
+    "k62_fused_two_slot": dict(N=400, K=62, G=6, Q=8, seed=37, weights=True),
+    "k63_obs_group": dict(N=400, K=63, G=6, Q=8, seed=38),
+    # k_obs with one tile buffer (K >= 220) and the most quadrature nodes
+    "k226_one_buffer_q64": dict(N=600, K=226, G=6, Q=64, seed=39, ragged=True),
 }
 
 

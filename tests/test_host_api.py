@@ -289,3 +289,96 @@ def test_gram_wide_plan_covers_every_packed_tile_once(tmp_path):
     assert out.returncode == 0, out.stdout[-2000:]
     assert "plan ok" in out.stdout
     assert "K=200 T2=50 groups= 7 ctas=148 live=1275" in out.stdout
+
+
+def _k_ranges(ks):
+    """[53, 54, 55, 64] -> '53..55, 64'"""
+    ks, out = sorted(ks), []
+    lo = hi = ks[0]
+    for k in ks[1:] + [None]:
+        if k == hi + 1:
+            hi = k
+            continue
+        out.append(str(lo) if lo == hi else "%d..%d" % (lo, hi))
+        lo = hi = k
+    return ", ".join(out)
+
+
+def test_dispatch_cases_reach_every_kernel_class(tmp_path):
+    """The parity cases (CASES of test_gpu_glmm_parity.py) run every kernel an evaluation can pick: every
+    compiled instantiation of k_fused_eval and k_gram_mid, every k_gram_big plan (job groups, rows per stage,
+    straddle tile) and K = kMaxK, both column-chunk counts of k_obs_fused, k_obs with a single tile buffer
+    beside k_gram_wide and beside k_gram_big, Q = 1 and Q = kMaxQ on each observation kernel, and a Q that
+    runs all three node loops (U at a time, 2, 1) of both fused kernels.  What each K runs comes from
+    tools/dispatch_table.cu, which calls the planner's own functions; host-only, it launches nothing."""
+    import shutil
+    import subprocess
+    from test_gpu_glmm_parity import CASES
+    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
+    if not os.path.exists(nvcc):
+        pytest.skip("nvcc not available")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    exe = str(tmp_path / "dispatch")
+    subprocess.run([nvcc, "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-o", exe,
+                    os.path.join(root, "tools", "dispatch_table.cu")], check=True, capture_output=True)
+    out = subprocess.run([exe], capture_output=True, text=True)
+    assert out.returncode == 0, out.stdout[-2000:]
+    lines = out.stdout.splitlines()
+    consts = {k: int(v) for k, v in (t.split("=") for t in lines[-1].split())}
+    table = {}
+    for line in lines[:-1]:
+        row = dict(t.split("=") for t in line.split())
+        table[int(row.pop("K"))] = row
+    max_k, max_q = consts["kMaxK"], consts["kMaxQ"]
+    assert sorted(table) == list(range(1, max_k + 1))
+    assert len({r["id"] for r in table.values() if r["gram"] == "fused"}) == consts["fused_ids"] > 0
+    assert len({r["id"] for r in table.values() if r["gram"] == "mid"}) == consts["mid_ids"] > 0
+
+    def nbuf(row, Q):
+        """k_obs tile buffers at Q; the rule only drops to one buffer as Q grows, so it is known wherever the
+        buffer counts at Q = 1 and Q = kMaxQ agree"""
+        at = dict(zip((1, 8, max_q), (int(b) for b in row["nbuf"].split(","))))
+        return at.get(Q, at[1] if at[1] == at[max_q] else None)
+
+    def all_loops(Q, U):
+        return Q >= U and Q % U >= 2 and Q % U % 2 == 1
+
+    def classes(K, Q):
+        """the classes a case with K columns and Q nodes reaches (Q = None: the structural ones alone)"""
+        row, c = table[K], set()
+        obs = []
+        if row["gram"] == "fused":
+            c.add("k_fused_eval id %s" % row["id"])
+            obs.append(("k_fused_eval", consts["kFuUnroll"]))
+        elif row["gram"] == "mid":
+            c.add("k_gram_mid id %s" % row["id"])
+        elif row["gram"] == "big":
+            c.add("k_gram_big plan %s (n_groups/TN/straddle)" % row["plan"])
+        if K == max_k:
+            c.add("K = kMaxK")
+        if row["chunks"] != "-":
+            c.add("k_obs_fused with %s column chunk(s)" % row["chunks"])
+            obs.append(("k_obs_fused", consts["kOfUnroll"]))
+        else:
+            obs.append(("k_obs", None))
+            if row["gram"] in ("wide", "big") and nbuf(row, max_q if Q is None else Q) == 1:
+                c.add("k_obs with one tile buffer beside k_gram_%s" % row["gram"])
+        for name, U in obs:
+            for q in (1, max_q):
+                if Q is None or Q == q:
+                    c.add("Q = %d on %s" % (q, name))
+            if U is not None and (Q is None or all_loops(Q, U)):
+                c.add("Q running all node loops of %s, e.g. Q = %d" % (name, U + 3))
+        return c
+
+    where = {}
+    for K in table:
+        for cls in classes(K, None):
+            where.setdefault(cls, []).append(K)
+    reached = set()
+    for case in CASES.values():
+        reached |= classes(case["K"], case["Q"])
+    assert reached <= set(where)
+    missing = sorted(set(where) - reached)
+    assert not missing, "no parity case reaches: " + "; ".join(
+        "%s (K = %s)" % (cls, _k_ranges(where[cls])) for cls in missing)
