@@ -525,10 +525,13 @@ __device__ __forceinline__ void scan_apply_body(int vb, int nblk, const int32_t*
 // ---- the whole export as ONE launch: the conditional export behind a refill ---------------------------
 // A refill is followed by a full export that runs only if the refill found the zero pattern changed.  As four
 // dependent launches its usual fate -- four early returns -- still costs four launch hops per evaluation; as
-// one launch of co-resident CTAs (2 per SM) that walk the same phases between grid-wide barriers it costs one.
+// one launch of co-resident CTAs (kCoopCtasPerSM per SM; ensure_csr_scratch checks that they fit) that walk the
+// same phases between grid-wide barriers it costs one.  A first export stays the chain of launches: there every
+// phase gets a grid of its own size, and the fixed grid of co-resident CTAs is slower (DESIGN.md section 3).
 // bar[0]: arrivals (monotonic over the phases of one launch), bar[1]: CTAs that left; the last one resets both.
 // A barrier that does not complete within ~2 s gives up (the export is then wrong, which the caller's
 // status check reports: mismatch stays raised) instead of hanging the device.
+constexpr int kCoopCtasPerSM = 2;
 __device__ __forceinline__ bool grid_barrier(unsigned* bar, unsigned target) {
   __shared__ int ok;
   __syncthreads();
@@ -667,6 +670,14 @@ static int ensure_csr_scratch(lrvb_glmm* h) {
   LRVB_TRY(raise_smem_limit(k_csr_pass<1>, smem));
   LRVB_TRY(raise_smem_limit(k_csr_pass<2>, csr_refill_smem(Dg, CG)));
   LRVB_TRY(raise_smem_limit(k_csr_export_coop, smem));
+  // the grid barriers of the one-launch export wait for every CTA of its grid: all of them must be resident at once
+  int fit = 0;
+  LRVB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, k_csr_export_coop, 256, smem));
+  if (fit < kCoopCtasPerSM) {
+    set_error("CSR export: %d CTAs of k_csr_export_coop (%zu B of shared memory) fit per SM, %d needed", fit, smem,
+              kCoopCtasPerSM);
+    return LRVB_ECUDA;
+  }
   h->csr_cg = CG;
   h->csr_nchunk = nchunk;
   LRVB_CUDA(cudaMalloc((void**)&h->rowcnt, sizeof(int32_t) * (size_t)(D + 1)));
@@ -720,10 +731,10 @@ static int csr_full_export(lrvb_glmm* h, int32_t* indptr_dev, int32_t* indices_d
 
   const int nA = cdiv(Dg, 8), nB = (G > 0) ? nchunk : 0, nL = (G > 0) ? cdiv(2 * (int64_t)G, 8) : 0;
   if (run_if) {
-    // the conditional export behind a refill: one launch of co-resident CTAs (two per SM)
+    // the conditional export behind a refill: one launch of co-resident CTAs
     int32_t* segb = chunkoff + (size_t)2 * Dg * nchunk;
     unsigned* bar = (unsigned*)(segb + (size_t)2 * Dg * nchunk);
-    LRVB_CUDA(launch_pdl(k_csr_export_coop, dim3(2 * kNumSMs), dim3(256), smem, st, (const double*)h->A,
+    LRVB_CUDA(launch_pdl(k_csr_export_coop, dim3(kCoopCtasPerSM * kNumSMs), dim3(256), smem, st, (const double*)h->A,
                          (const double*)h->B, (const double*)h->L, Dg, G, CG, nA, nB, cntA, chunkcnt, chunkoff, coltot,
                          segb, h->rowcnt, (int64_t)D, blk, nblk, indptr_dev, indices_dev, data_dev, (int64_t*)nnz_dev,
                          h->csrmask, bar, run_if));

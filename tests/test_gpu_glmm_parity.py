@@ -262,7 +262,9 @@ def test_cg_general_preconditioner(vb):
         solver.get_hinv_vec(b)
 
 
-@pytest.mark.parametrize("N,G", [(4000, 40), (30000, 3000)])    # the second: the conditional export walks its roles with a grid stride
+# the second: the conditional export walks its roles with a grid stride; the last two: D = 16 + 2 G = 262,142 and
+# 262,146, either side of the size where a full export's row pointers go from one CTA to the three-phase scan
+@pytest.mark.parametrize("N,G", [(4000, 40), (30000, 3000), (400_000, 131_063), (400_000, 131_065)])
 def test_csr_refill_follows_pattern_changes(vb, N, G):
     """The CSR export after the first one rewrites the values for the cached pattern and checks the zero
     mask on the device; when an entry becomes exactly zero (or stops being zero) the conditional full
@@ -273,12 +275,13 @@ def test_csr_refill_follows_pattern_changes(vb, N, G):
     model._csr_refill_min = 0                # the refill path whatever the size
     x = case["free"]
 
-    def dense_from_blocks():
-        A, B, L = [t.cpu().numpy() for t in model.blocks()]
-        return oracle.blocks_to_dense(oracle.lay, dict(A=A, B=B, L=L))
-
     def check(H):
-        ref = scipy.sparse.csr_matrix(dense_from_blocks())
+        # scipy's CSR of the cached blocks (exact zeros dropped, columns sorted), assembled without the dense matrix
+        A, B, L = [t.cpu().numpy() for t in model.blocks()]
+        diag = scipy.sparse.diags
+        ref = scipy.sparse.bmat([[A, B[:, 0].T, B[:, 1].T], [B[:, 0], diag(L[:, 0]), diag(L[:, 1])],
+                                 [B[:, 1], diag(L[:, 1]), diag(L[:, 2])]], format="csr")
+        ref.eliminate_zeros()
         ref.sort_indices()
         Hs = H.to_scipy()
         np.testing.assert_array_equal(Hs.indptr, ref.indptr)
