@@ -284,6 +284,17 @@ int lrvb_glmm_logo(lrvb_glmm* h, const double* Sinv_dev, const double* Pinv_dev,
  * c^T H^-1 c moves with the observation weights: d/dw_n = q_n - grad l_n . (H^-1 t).  No atomics: repeated calls are
  * bitwise equal.  LRVB_EINVAL for NULL pointers; allocates a (2N + 5G + O(K)) scratch in the handle on first use. */
 int lrvb_glmm_third_contract(lrvb_glmm* h, const double* a_dev, double* t_dev, double* q_dev, void* stream);
+/* The "meat" of the infinitesimal-jackknife (IJ) bootstrap covariance of the global parameters, at the cached Hessian
+ * (an order-2 evaluation in free coordinates, normally at the optimum; LRVB_ESTATE otherwise).  The IJ influence of
+ * a unit u (a row, unit = 0, or a whole group, unit = 1) on the globals is S^-1 V_u with V_u = v_glob - B_g^T L_g^-1
+ * v_loc, v = the unit's data gradient from W rows 0, 1 (lrvb_glmm_obs_weights), as in lrvb_glmm_logo.  Output:
+ *   meat_dev (Dg, Dg) row-major: sum_u V_u V_u^T, exactly symmetric
+ *   sum_dev  (Dg):               s = sum_u V_u (the same for both units: the column sums of the groups' V)
+ * so that the IJ covariance of the globals is S^-1 (meat - s s^T / U) S^-1 with U = the units of non-zero weight.
+ * Rows of weight 0 have V_u = 0 exactly.  No atomics: repeated calls are bitwise equal; nothing a later evaluation,
+ * solve or IJ call reads is changed.  LRVB_EINVAL for NULL pointers or a unit other than 0 or 1; allocates a scratch
+ * of about 5 N + G (4K + 3 Dg) doubles in the handle on first use. */
+int lrvb_glmm_ij_meat(lrvb_glmm* h, int32_t unit, double* meat_dev, double* sum_dev, void* stream);
 
 /* ---- batched exponential-family terms (ExponentialFamilies.py) --------------------------
  * All pointers dev; M = number of factors. */

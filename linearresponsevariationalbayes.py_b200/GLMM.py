@@ -67,6 +67,14 @@ delta_global (G, Dg) = the IJ shift of the global free parameters.  Scalars: elp
 sqrt(G') std(elpd_logo_group over the G' non-empty groups, ddof=1) (NaN when G' < 2).  An empty group has zero
 delta_global, cooks_distance and elpd_logo_group."""
 
+IJCovariance = namedtuple("IJCovariance", ["unit", "n_units", "global_cov", "moment_cov", "beta_cov", "beta_se_ij",
+                                           "beta_se_lr"])
+IJCovariance.__doc__ = """The infinitesimal-jackknife (IJ) approximation of the bootstrap covariance of the global
+parameters (``LinearResponseCovariances.get_ij_covariance``), with rows or whole groups resampled (unit = "row" or
+"group"; "group" is the cluster-robust sandwich covariance).  n_units = the units of non-zero weight; global_cov (Dg, Dg)
+in free coordinates; moment_cov (2+K, 2+K) of [E mu, E tau, E beta]; beta_cov (K, K) of E[beta]; beta_se_ij = the
+square root of its diagonal; beta_se_lr = the LRVB (posterior) standard deviations of E[beta], for comparison."""
+
 DropResult = namedtuple("DropResult", ["n_drop", "fraction", "dropped", "predicted_estimate", "predicted_sd"])
 DropResult.__doc__ = """One target of ``LinearResponseCovariances.get_approximate_max_influence``: the fewest units (rows or
 groups) whose removal the first-order prediction says is enough to reach the target, n_drop (None if no such set
@@ -922,6 +930,21 @@ class LogisticGLMM(object):
         fold = grp[1][self._group_nonempty]
         se = float(fold.std(correction=1)) * np.sqrt(fold.numel()) if fold.numel() > 1 else float("nan")
         return ApproximateLOGO(out[0], out[1], out[2], grp[1], grp[0], delta, float(out[0].sum()), se)
+
+    def ij_meat(self, unit):
+        """The meat of the infinitesimal-jackknife bootstrap covariance of the globals at the cached Hessian (normally
+        the optimum): (meat (Dg, Dg), s (Dg)) = (sum_u V_u V_u^T, sum_u V_u) over the rows (unit="row") or the groups
+        (unit="group"), where S^-1 V_u = the global block of H^-1 psi_u and psi_u = the unit's weighted score, as in
+        ``approximate_logo``.  The IJ covariance is S^-1 (meat - s s^T / U) S^-1 with U = the units of non-zero weight
+        (``LinearResponseCovariances.get_ij_covariance``).  CUDA tensors; device passes of csrc/ij.cu."""
+        torch = nat.require_cuda()
+        if unit not in ("row", "group"):
+            raise ValueError("unit must be 'row' or 'group', got %r" % (unit,))
+        meat = torch.empty(self.Dg, self.Dg, dtype=torch.float64, device=self.device)
+        s = torch.empty(self.Dg, dtype=torch.float64, device=self.device)
+        nat.check(self._lib.lrvb_glmm_ij_meat(self._h, 0 if unit == "row" else 1, nat.ptr(meat), nat.ptr(s),
+                                              nat.stream_ptr()))
+        return meat, s
 
     def prediction_jacobian(self, free, X_new, groups_new, quantity="prob"):
         """d prob / d free (or d eta / d free) of new rows as scipy CSR (M, D): a x on beta.mean, b x~ on

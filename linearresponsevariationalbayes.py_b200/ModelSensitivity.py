@@ -15,7 +15,7 @@ device conjugate gradient -- the dense ``cho_factor`` of the reference is O(D^3)
 import numpy as np
 import scipy.sparse
 
-from .GLMM import ApproximateMaxInfluence, DropResult
+from .GLMM import ApproximateMaxInfluence, DropResult, IJCovariance
 from ._tensors import is_torch, to_device
 
 
@@ -333,6 +333,54 @@ class LinearResponseCovariances(object):
         if host:
             mean_shift, sd_shift = mean_shift.cpu().numpy(), sd_shift.cpu().numpy()
         return ApproximateMaxInfluence(est, sd, z, mean_shift, sd_shift, targets)
+
+    def get_ij_covariance(self, unit="group", centered=True):
+        """The infinitesimal-jackknife (IJ) approximation of the bootstrap covariance of the global parameters at the
+        optimum (Giordano et al., "A Swiss Army Infinitesimal Jackknife"), resampling rows (unit="row") or whole groups
+        (unit="group": the cluster bootstrap, i.e. the cluster-robust sandwich covariance).  With S^-1 V_u the global
+        block of H^-1 psi_u (psi_u = the unit's weighted score), s = sum_u V_u and U the units of non-zero weight,
+
+            global_cov = S^-1 (sum_u V_u V_u^T - s s^T / U) S^-1,
+
+        without the s s^T / U term when ``centered`` is False (at an exact optimum s = 0 for the full data).  Returns a
+        ``GLMM.IJCovariance``: numpy for a numpy optimum, CUDA tensors for a CUDA one.  The sums over units are device
+        passes (csrc/ij.cu); always from S^-1, whatever ``method`` is."""
+        import torch
+        model = self.model
+        if getattr(model, "local", None) is not None:
+            raise NotImplementedError("the IJ covariance of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                      "and use its LinearResponseCovariances")
+        if unit not in ("row", "group"):
+            raise ValueError("unit must be 'row' or 'group', got %r" % (unit,))
+        dev = model.device
+        keep = torch.ones(model.N, dtype=torch.bool, device=dev) if model.w is None else model.w != 0
+        if unit == "row":
+            n_units = int(keep.sum())
+        else:
+            n_units = int((torch.bincount(model.g.to(torch.int64)[keep], minlength=model.G) > 0).sum())
+        if n_units == 0:
+            raise ValueError("the IJ covariance needs a %s of non-zero weight" % unit)
+        self._ensure_point()
+        if self._sinv is None:
+            self._sinv = model.global_covariance()
+        meat, s = model.ij_meat(unit)
+        if centered:
+            meat = meat - torch.outer(s, s) / n_units
+        sinv = self._sinv
+        cov = sinv @ meat @ sinv
+        cov = 0.5 * (cov + cov.t())
+        K, Dg = model.K, model.Dg
+        x = self._opt0.detach().cpu().numpy() if is_torch(self._opt0) else self._opt0
+        jac = torch.from_numpy(np.ascontiguousarray(model.moment_jacobian(x)[:2 + K, :Dg].toarray())).to(dev)
+        mcov = jac @ cov @ jac.t()
+        mcov = 0.5 * (mcov + mcov.t())
+        beta_cov = cov[4:4 + K, 4:4 + K]
+        se_ij = torch.sqrt(torch.diagonal(beta_cov))
+        se_lr = torch.sqrt(torch.diagonal(sinv[4:4 + K, 4:4 + K]))
+        out = [cov, mcov, beta_cov, se_ij, se_lr]
+        if not is_torch(self._opt0):
+            out = [t.cpu().numpy() for t in out]
+        return IJCovariance(unit, n_units, *out)
 
     def _contrast(self, c):
         """c (length K, numpy / list / torch) or an integer k -> chat (D,) numpy with c on the beta.mean block."""

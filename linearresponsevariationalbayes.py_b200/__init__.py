@@ -35,6 +35,6 @@ from .ConjugateGradient import ConjugateGradientSolver  # noqa: F401
 from .ModelSensitivity import (LinearResponseCovariances, ArrowheadCovariance,  # noqa: F401
                                WeightSensitivityLinearApproximation)
 from .GLMM import (LogisticGLMM, GLMMPrior, DeviceCSR, Prediction, ApproximateLOO, ApproximateLOGO,  # noqa: F401
-                   ApproximateMaxInfluence, DropResult)
+                   ApproximateMaxInfluence, DropResult, IJCovariance)
 
 __version__ = "0.1.0"

@@ -76,6 +76,7 @@ SIGNATURES = {
     "lrvb_glmm_loo": (c_int32, [_P, _P, _P, _P, _P, _P]),
     "lrvb_glmm_logo": (c_int32, [_P, _P, _P, _P, _P, _P, _P]),
     "lrvb_glmm_third_contract": (c_int32, [_P, _P, _P, _P, _P]),
+    "lrvb_glmm_ij_meat": (c_int32, [_P, c_int32, _P, _P, _P]),
     "lrvb_ef_gamma_entropy": (c_int32, [_P, _P, c_int64, _P, _P]),
     "lrvb_ef_e_log_gamma": (c_int32, [_P, _P, c_int64, _P, _P]),
     "lrvb_ef_gamma_terms": (c_int32, [_P, _P, c_int64, _P, _P, _P]),

@@ -44,7 +44,7 @@ int lrvb_glmm_destroy(lrvb_glmm* h) {
   void* ptrs[] = {h->gh, h->gptr, h->vec, h->W, h->klpart, h->gradpart, h->gsc, h->BR, h->locpart, h->fin_counter, h->fin_pre,
                   h->jobs, h->gslots, h->grampart, h->bval, h->wc_scratch, h->B, h->L, h->gradl, h->outg, h->rowcnt, h->scanblk, h->csrwork, h->csrmask,
                   h->cgbuf, h->hvppart, h->dotpart, h->scal, h->flags, h->Linv, h->T,
-                  h->schurpart, h->pred_B, h->logo_V, h->amip_work};
+                  h->schurpart, h->pred_B, h->logo_V, h->amip_work, h->ij_work};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   for (cudaEvent_t e : h->ev)

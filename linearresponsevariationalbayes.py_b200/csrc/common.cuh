@@ -367,6 +367,7 @@ struct lrvb_glmm {
   double* pred_B = nullptr;   // (3 Kp8, Kp4) scaled beta block of S^-1 for lrvb_glmm_predict_lr (predict.cu)
   double* logo_V = nullptr;   // (G, Dg) per-group gradients of lrvb_glmm_logo, then its (G, K) Cook's products (logo.cu)
   double* amip_work = nullptr;   // row coefficients, per-CTA and per-group partials of lrvb_glmm_third_contract (amip.cu)
+  double* ij_work = nullptr;     // weights, group sums, Gram and correction partials of lrvb_glmm_ij_meat (ij.cu)
 };
 
 namespace lrvb {

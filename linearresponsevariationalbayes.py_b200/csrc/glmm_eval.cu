@@ -1425,4 +1425,94 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
   return LRVB_OK;
 }
 
+// ------------------------------------------------------------------------------------------
+// Infinitesimal-jackknife meat (lrvb_glmm_ij_meat, ij.cu, DESIGN.md 3f): the row term sum_n h_n h_n^T is the
+// packed Gram of the evaluation with the weights (a, b, c) = (W_m^2, W_m W_v, W_v^2), and the per-group sums
+// E_g, F_g are k_group<2>'s on the same weights.  Both kernels are compiled here, so their IJ launches are too.
+//
+// K <= 24 has no stand-alone Gram kernel in the evaluation (the one-pass kernel of fused.cuh computes the Gram):
+// the k_gram_mid instantiations of T2 = 1 .. 6 serve the IJ there, through a lookup of their own so that the
+// evaluation's plan is unchanged.  Above, the IJ runs the handle's own Gram plan.
+static GramMidKernel gram_mid_kernel_ij(int K) {
+  if (K > kFuMaxK) return gram_mid_kernel(K);
+  const int T2 = (2 * K + 7) / 8, T0 = K / 8;
+  const bool M = (K % 8) != 0;
+#define LRVB_GM(T2_, T0_, M_)                                                                       \
+  if (T2 == T2_ && T0 == T0_ && M == M_) {                                                          \
+    constexpr GramMidGeom g = gram_mid_geom(T2_);                                                   \
+    return {k_gram_mid<T2_, T0_, M_, g.warps, g.P>, g.warps};                                        \
+  }
+  LRVB_GM(1, 0, true)
+  LRVB_GM(2, 0, true)
+  LRVB_GM(2, 1, false)
+  LRVB_GM(3, 1, true)
+  LRVB_GM(4, 1, true)
+  LRVB_GM(4, 2, false)
+  LRVB_GM(5, 2, true)
+  LRVB_GM(6, 2, true)
+  LRVB_GM(6, 3, false)
+#undef LRVB_GM
+  return {nullptr, 0};
+}
+
+// doubles of the IJ Gram partials: the layout of the kernel the IJ runs (packed (n_cta, NT, 64), or gram_big's)
+size_t ij_gram_parts(const lrvb_glmm* h) {
+  if (h->fused2) return (size_t)kNumSMs * gram_small_shape(h->K).NT * 64;
+  if (h->gram_mid || h->gram_wide) return (size_t)h->gram_grid_x * gram_small_shape(h->K).NT * 64;
+  return (size_t)h->gram_grid_x * kGbWarps * 16 * 64;
+}
+
+// Finish of the IJ Gram: the evaluation's Gram finish into `A` (the chain rule to free coordinates leaves
+// -diag(1, s) G diag(1, s) on the beta block, s_k = -(i_k - lb) / i_k^2); lrvb_glmm_ij_meat negates it.
+__global__ void __launch_bounds__(256)
+k_ij_gram_finish(const double* __restrict__ vec, const double* __restrict__ part, const GbJob* __restrict__ jobs,
+                 const GbSlot* __restrict__ slots, double* __restrict__ A, int K, int packed, int NT, int n_groups,
+                 int n_chunk, lrvb_glmm_bounds bd) {
+  const int Dg = 4 + 2 * K;
+  if (packed) gram_small_finish_body(blockIdx.x, part, vec, A, K, Dg, NT, n_chunk, bd, 0);
+  else gram_big_finish_body(blockIdx.x, part, jobs, slots, vec, A, K, Dg, n_groups, n_chunk, bd, 0);
+}
+
+// W5 (5, ldw) = (W_m, W_v, W_m^2, W_m W_v, W_v^2) of k_ij_weights.  Writes gsc (G, 5), BR (G, 4, K) and the
+// negated, scaled Gram term into A (Dg, Dg), which is cleared first (zero outside the beta block).
+int launch_ij_gram(lrvb_glmm* h, const double* W5, double* part, double* gsc, double* BR, double* A, cudaStream_t st) {
+  const int K = h->K, G = h->G, Dg = h->Dg;
+  const int64_t N = h->N;
+  LRVB_CUDA(cudaMemsetAsync(A, 0, sizeof(double) * Dg * Dg, st));
+  if (G > 0) {
+    const int ggrid = (int)((G + 7) / 8 < 148 * 8 ? (G + 7) / 8 : 148 * 8);
+    k_group<2><<<ggrid, 256, 0, st>>>(h->X, W5, h->gptr, gsc, BR, h->ldw, K, G);
+    LRVB_CHECK_LAUNCH();
+  }
+  if (N == 0) return LRVB_OK;
+  const double* Wabc = W5 + 2 * h->ldw;
+  int packed = 1, n_gf, n_chunk;
+  const int NT = gram_small_shape(K).NT;
+  if (h->fused2 || h->gram_mid) {
+    const GramMidKernel gk = h->fused2 ? gram_mid_kernel_ij(K) : GramMidKernel{h->gm_kernel, h->gm_warps};
+    const size_t smem = gram_mid_smem(K, gram_small_shape(K).T2);
+    LRVB_TRY(raise_smem_limit(gk.fn, smem));
+    LRVB_CUDA(launch_pdl(gk.fn, dim3(kNumSMs), dim3(32 * gk.warps), smem, st, h->X, Wabc, part, N, h->ldw, K));
+    n_gf = NT;
+    n_chunk = kNumSMs;
+  } else if (h->gram_wide) {
+    LRVB_CUDA(launch_pdl(k_gram_wide, dim3(h->gram_grid_x), dim3(32 * kGwWarps), h->gram_smem, st, h->X, Wabc, h->ldw,
+                         (const GwGroup*)h->jobs, (const GwCta*)h->gslots, part, N, K, NT));
+    n_gf = NT;
+    n_chunk = h->gram_grid_x;
+  } else {
+    LRVB_CUDA(launch_pdl(k_gram_big, dim3(h->gram_grid_x), dim3(32 * kGbWarps), h->gram_smem, st, h->X, Wabc, h->ldw,
+                         (const GbJob*)h->jobs, (const GbSlot*)h->gslots, part, N, K, h->gram_tn, h->gram_grid_y,
+                         h->gram_grid_x / h->gram_grid_y));
+    packed = 0;
+    n_gf = h->gram_jobs * 16;
+    n_chunk = h->gram_grid_x / h->gram_grid_y;
+  }
+  LRVB_CHECK_LAUNCH();
+  k_ij_gram_finish<<<n_gf, 256, 0, st>>>(h->vec, part, (const GbJob*)h->jobs, (const GbSlot*)h->gslots, A, K, packed,
+                                         NT, h->gram_grid_y, n_chunk, h->bounds);
+  LRVB_CHECK_LAUNCH();
+  return LRVB_OK;
+}
+
 }  // namespace lrvb

@@ -240,6 +240,16 @@ k_logo_rows(const double* __restrict__ X, const double* __restrict__ yv, const i
   }
 }
 
+// Pass 1 into V (G, Dg) for the infinitesimal-jackknife meat (ij.cu): its V_g is the group unit's influence and
+// its column sum the centring of both units
+int launch_logo_grad(lrvb_glmm* h, double* V, cudaStream_t st) {
+  if (h->G == 0) return LRVB_OK;
+  k_logo_grad<<<cdiv(h->G, 8), 256, 0, st>>>(h->X, h->W, h->ldw, h->gptr, h->vec, h->B, h->L, V, h->K, h->G,
+                                              h->bounds);
+  LRVB_CHECK_LAUNCH();
+  return LRVB_OK;
+}
+
 // V (G, Dg), allocated in the handle on first use; after pass 2's first product it holds Y (G, K)
 static int ensure_logo_V(lrvb_glmm* h) {
   if (h->logo_V) return LRVB_OK;

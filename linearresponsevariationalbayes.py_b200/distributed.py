@@ -498,6 +498,10 @@ class ShardedLogisticGLMM(object):
         raise NotImplementedError("the third derivative of a sharded model: build a single-GPU LogisticGLMM of the job "
                                   "and use LinearResponseCovariances.get_approximate_max_influence")
 
+    def ij_meat(self, *args, **kwargs):
+        raise NotImplementedError("the IJ covariance of a sharded model: build a single-GPU LogisticGLMM of the job "
+                                  "and use LinearResponseCovariances.get_ij_covariance")
+
     def moment_jacobian(self, free):
         import scipy.sparse
         free = np.asarray(free, dtype=np.float64).reshape(-1)
