@@ -75,6 +75,18 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
                      const double* w_dev, const double* gh_x_host, const double* gh_w_host,
                      const lrvb_glmm_prior* prior, const lrvb_glmm_bounds* bounds,
                      int32_t include_global_terms, void* stream);
+/* The Poisson log-link GLMM for counts (R's glmer(..., family = poisson) with offset(log(exposure))): the same
+ * variational family, layout, priors and calls as above with the observation term
+ *   E_q log p(y_n | eta_n) = w_n (y_n m_n - exp(m_n + v_n / 2) - lgamma(y_n + 1)),
+ * m_n = x_n . E[beta] + E[u_g] + offset_n, v_n = x_n^2 . Var[beta] + Var[u_g], exact under q (no quadrature, no Q).
+ *  y dev (N,) fp64 counts, finite and >= 0 (non-integer values are accepted); offset dev (N,) fp64 or NULL, finite,
+ *  16-byte aligned like y.  Validates on the device (syncs) and computes sum_n w_n lgamma(y_n + 1) once.
+ * lrvb_glmm_predict, _predict_lr, _loo, _logo and _third_contract evaluate the logistic likelihood and return
+ * LRVB_EINVAL on a Poisson handle; every other call works unchanged. */
+int lrvb_glmm_create_poisson(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, const double* X_dev,
+                             const double* y_dev, const int32_t* g_dev, const double* w_dev, const double* offset_dev,
+                             const lrvb_glmm_prior* prior, const lrvb_glmm_bounds* bounds,
+                             int32_t include_global_terms, void* stream);
 int lrvb_glmm_destroy(lrvb_glmm* h);
 /* Number of CUDA kernels this library has launched in this process (bench.py gpu_launches). */
 long long lrvb_launch_count(void);

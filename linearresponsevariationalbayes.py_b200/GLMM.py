@@ -1,4 +1,4 @@
-"""Logistic GLMM variational objective bound to the CUDA library (single GPU).
+"""Logistic and Poisson GLMM variational objectives bound to the CUDA library (single GPU).
 
 The reference has no GLMM class: its users compose this KL from ``UVNParam`` / ``GammaParam`` /
 ``UVNParamVector`` bundles, ``Modeling.get_e_logistic_term_guass_hermite`` (Modeling.py:35-52)
@@ -12,6 +12,10 @@ accepts it in place of ``fun``.
     KL(free) = -( sum_n w_n [y_n z_n - GH(z_mean_n, z_sd_n)]
                   + sum_g [-1/2 E[tau]((E mu - E u_g)^2 + Var mu + Var u_g) + 1/2 E log tau]
                   + entropies(mu, beta, u, tau) + priors(mu, beta, tau) )
+
+``PoissonGLMM`` is the same objective with the Poisson log-link observation term
+w_n [y_n m_n - exp(m_n + v_n / 2) - lgamma(y_n + 1)] (m_n, v_n: mean and variance of the linear predictor, offset
+included), exact under q.
 """
 import ctypes
 import weakref
@@ -268,34 +272,27 @@ def group_sort(groups):
     return g[perm], perm
 
 
-class LogisticGLMM(object):
-    """Data + variational parameters + device handle of one logistic GLMM (or one shard of it).
-
-    X (N,K) float64, y (N,) in {0,1}, groups (N,) integer ids in [0, num_groups); observations
-    are stably sorted by group if they are not already (``self.perm`` records the permutation).
-    ``gh_x, gh_w``: Gauss-Hermite nodes/weights (default ``hermgauss(num_gh_points)``).
-    """
+class _DeviceGLMM(object):
+    """What ``LogisticGLMM`` and ``PoissonGLMM`` share: the staging of the data, the variational parameters, the
+    device handle and every call that reads only the per-row weights of an evaluation (value, gradient, Hessian,
+    solves, LRVB covariances, weight sensitivity, IJ).  Prediction, LOO, LOGO and the third-derivative contraction
+    evaluate the logistic likelihood; ``PoissonGLMM`` refuses them."""
 
     _lrvb_device_model = True
+    family = "logistic"
 
-    def __init__(self, X, y, groups, num_gh_points=8, gh_x=None, gh_w=None, weights=None,
-                 prior=None, num_groups=None, min_info=0.0, min_shape=0.0, min_rate=0.0,
-                 include_global_terms=True, name="glmm_par"):
+    def _stage(self, X, y, groups, weights, offset, prior, num_groups, min_info, min_shape, min_rate, name):
+        """Checks the shapes, sorts the rows by group (``self.perm``; y, weights and offset follow X), puts the data
+        on the device 16-byte aligned and builds the parameter dictionary, the prior and the bounds."""
         torch = nat.require_cuda()
-        lib = nat.load()
-        if gh_x is None or gh_w is None:
-            gh_x, gh_w = np.polynomial.hermite.hermgauss(int(num_gh_points))
-        self.gh_x = np.ascontiguousarray(np.asarray(gh_x, dtype=np.float64))
-        self.gh_w = np.ascontiguousarray(np.asarray(gh_w, dtype=np.float64))
-        if self.gh_x.shape != self.gh_w.shape or self.gh_x.ndim != 1:
-            raise ValueError("gh_x and gh_w must be 1-d arrays of the same length")
         self.prior = prior or GLMMPrior()
 
         Xs = X.shape
         if len(Xs) != 2:
             raise ValueError("X must be (N, K)")
         N, K = int(Xs[0]), int(Xs[1])
-        for nm, v in (("y", y), ("groups", groups)) + ((("weights", weights),) if weights is not None else ()):
+        for nm, v in ((("y", y), ("groups", groups)) + ((("weights", weights),) if weights is not None else ())
+                      + ((("offset", offset),) if offset is not None else ())):
             if int(np.prod(v.shape)) != N:
                 raise ValueError("Wrong size for {}.  Expected {}, got {}".format(
                     nm, N, int(np.prod(v.shape))))
@@ -305,14 +302,17 @@ class LogisticGLMM(object):
         self.X = to_device(X)
         self.y = to_device(y).reshape(-1)
         self.w = None if weights is None else to_device(weights).reshape(-1)
+        self.offset = None if offset is None else to_device(offset).reshape(-1)
         if perm is not None:
             pd = to_device(perm, torch.int64)
             self.X = self.X.index_select(0, pd).contiguous()
             self.y = self.y.index_select(0, pd).contiguous()
             if self.w is not None:
                 self.w = self.w.index_select(0, pd).contiguous()
+            if self.offset is not None:
+                self.offset = self.offset.index_select(0, pd).contiguous()
         self.g = to_device(g_sorted, torch.int32).reshape(-1)
-        for nm in ("X", "y", "w", "g"):   # views into larger buffers: the library needs 16-B alignment
+        for nm in ("X", "y", "w", "offset", "g"):   # views into larger buffers: the library needs 16-B alignment
             t = getattr(self, nm)
             if t is not None and t.numel() and t.data_ptr() % 16:
                 setattr(self, nm, t.clone())
@@ -335,12 +335,10 @@ class LogisticGLMM(object):
         self._bounds_c = nat.Bounds(min_info, min_shape, min_rate, min_info, min_info)
         self.lower_bounds = dict(mu_info=min_info, tau_shape=min_shape, tau_rate=min_rate,
                                  beta_info=min_info, u_info=min_info)
-        h = ctypes.c_void_p()
-        nat.check(lib.lrvb_glmm_create(
-            ctypes.byref(h), N, K, self.G, self.gh_x.size, nat.ptr(self.X), nat.ptr(self.y),
-            nat.ptr(self.g), nat.ptr(self.w), nat.darray(self.gh_x), nat.darray(self.gh_w),
-            ctypes.byref(self._prior_c), ctypes.byref(self._bounds_c),
-            1 if include_global_terms else 0, nat.stream_ptr()))
+
+    def _bind(self, h, lib):
+        """Takes ownership of the created handle ``h`` and sets up the views and staging buffers of its results."""
+        torch = nat.require_cuda()
         self._h = h
         self._lib = lib
         dev = self.X.device
@@ -1005,3 +1003,66 @@ class LogisticGLMM(object):
         cols = [0, 2, 3] + list(range(4, 4 + K)) + list(range(Dg, Dg + G))
         vals = [1.0, np.exp(free[2]) / b, -a / (b * b) * np.exp(free[3])] + [1.0] * (K + G)
         return scipy.sparse.csr_matrix((vals, (rows, cols)), (2 + K + G, self.D))
+
+
+class LogisticGLMM(_DeviceGLMM):
+    """Data + variational parameters + device handle of one logistic GLMM (or one shard of it).
+
+    X (N,K) float64, y (N,) in {0,1}, groups (N,) integer ids in [0, num_groups); observations
+    are stably sorted by group if they are not already (``self.perm`` records the permutation).
+    ``gh_x, gh_w``: Gauss-Hermite nodes/weights (default ``hermgauss(num_gh_points)``).
+    """
+
+    def __init__(self, X, y, groups, num_gh_points=8, gh_x=None, gh_w=None, weights=None,
+                 prior=None, num_groups=None, min_info=0.0, min_shape=0.0, min_rate=0.0,
+                 include_global_terms=True, name="glmm_par"):
+        nat.require_cuda()
+        lib = nat.load()
+        if gh_x is None or gh_w is None:
+            gh_x, gh_w = np.polynomial.hermite.hermgauss(int(num_gh_points))
+        self.gh_x = np.ascontiguousarray(np.asarray(gh_x, dtype=np.float64))
+        self.gh_w = np.ascontiguousarray(np.asarray(gh_w, dtype=np.float64))
+        if self.gh_x.shape != self.gh_w.shape or self.gh_x.ndim != 1:
+            raise ValueError("gh_x and gh_w must be 1-d arrays of the same length")
+        self._stage(X, y, groups, weights, None, prior, num_groups, min_info, min_shape, min_rate, name)
+        h = ctypes.c_void_p()
+        nat.check(lib.lrvb_glmm_create(
+            ctypes.byref(h), self.N, self.K, self.G, self.gh_x.size, nat.ptr(self.X), nat.ptr(self.y),
+            nat.ptr(self.g), nat.ptr(self.w), nat.darray(self.gh_x), nat.darray(self.gh_w),
+            ctypes.byref(self._prior_c), ctypes.byref(self._bounds_c),
+            1 if include_global_terms else 0, nat.stream_ptr()))
+        self._bind(h, lib)
+
+
+class PoissonGLMM(_DeviceGLMM):
+    """Data + variational parameters + device handle of one Poisson log-link GLMM for counts (lme4's
+    ``glmer(y ~ x + (1 | g) + offset(log(exposure)), family = poisson)``).
+
+    X (N,K) float64, y (N,) counts (finite, >= 0; non-integer values are accepted), groups (N,) integer ids in
+    [0, num_groups), offset (N,) or None: added to the linear predictor (log exposure).  Rows are stably sorted by
+    group as in ``LogisticGLMM``.  Under q the observation term w [y m - exp(m + v/2) - lgamma(y + 1)] is exact, so
+    there is no quadrature.  Evaluation, Hessian, solves, ``LinearResponseCovariances`` (except prediction, LOO, LOGO
+    and AMIP), ``WeightSensitivityLinearApproximation`` and ``get_ij_covariance`` (cluster-robust standard errors for
+    overdispersed counts) work as for the logistic model.
+    """
+
+    family = "poisson"
+
+    def __init__(self, X, y, groups, offset=None, weights=None, prior=None, num_groups=None, min_info=0.0,
+                 min_shape=0.0, min_rate=0.0, include_global_terms=True, name="glmm_par"):
+        nat.require_cuda()
+        lib = nat.load()
+        self._stage(X, y, groups, weights, offset, prior, num_groups, min_info, min_shape, min_rate, name)
+        h = ctypes.c_void_p()
+        nat.check(lib.lrvb_glmm_create_poisson(
+            ctypes.byref(h), self.N, self.K, self.G, nat.ptr(self.X), nat.ptr(self.y), nat.ptr(self.g),
+            nat.ptr(self.w), nat.ptr(self.offset), ctypes.byref(self._prior_c), ctypes.byref(self._bounds_c),
+            1 if include_global_terms else 0, nat.stream_ptr()))
+        self._bind(h, lib)
+
+    def _logistic_only(self, *args, **kwargs):
+        raise NotImplementedError("not implemented for the Poisson family: prediction, approximate LOO / LOGO and the "
+                                  "third-derivative contraction of AMIP evaluate the logistic likelihood")
+
+    predict = predict_lr = prediction_jacobian = approximate_loo = approximate_logo = _logistic_only
+    third_derivative_contraction = _check_binary_y = _logistic_only

@@ -19,6 +19,13 @@ from .GLMM import ApproximateMaxInfluence, DropResult, IJCovariance
 from ._tensors import is_torch, to_device
 
 
+def _require_logistic(model, what):
+    """Prediction, LOO, LOGO and AMIP evaluate the logistic likelihood in their device epilogues."""
+    family = getattr(model, "family", "logistic")
+    if family != "logistic":
+        raise NotImplementedError("%s is not implemented for the %s family" % (what, family))
+
+
 class LinearResponseCovariances(object):
     def __init__(self, objective, opt_par_value, validate_optimum=False, grad_tol=1e-8,
                  method="schur", cg_tol=1e-8, cg_preconditioner="block_jacobi"):
@@ -191,6 +198,7 @@ class LinearResponseCovariances(object):
         if getattr(model, "local", None) is not None:
             raise NotImplementedError("prediction of a sharded model: build a single-GPU LogisticGLMM of the "
                                       "job and use its LinearResponseCovariances")
+        _require_logistic(model, "prediction")
         self._ensure_point()
         if self._sinv is None:
             self._sinv = model.global_covariance()
@@ -211,6 +219,7 @@ class LinearResponseCovariances(object):
         if getattr(model, "local", None) is not None:
             raise NotImplementedError("approximate LOO of a sharded model: build a single-GPU LogisticGLMM of the "
                                       "job and use its LinearResponseCovariances")
+        _require_logistic(model, "approximate LOO")
         model._check_binary_y()
         self._ensure_point()
         if self._sinv is None:
@@ -235,6 +244,7 @@ class LinearResponseCovariances(object):
         if getattr(model, "local", None) is not None:
             raise NotImplementedError("approximate LOGO of a sharded model: build a single-GPU LogisticGLMM of the "
                                       "job and use its LinearResponseCovariances")
+        _require_logistic(model, "approximate LOGO")
         model._check_binary_y()
         self._ensure_point()
         if self._sinv is None:
@@ -267,6 +277,7 @@ class LinearResponseCovariances(object):
         if getattr(model, "local", None) is not None:
             raise NotImplementedError("approximate maximum influence of a sharded model: build a single-GPU "
                                       "LogisticGLMM of the job and use its LinearResponseCovariances")
+        _require_logistic(model, "the approximate maximum influence")
         if unit not in ("row", "group"):
             raise ValueError("unit must be 'row' or 'group', got %r" % (unit,))
         level, max_fraction = float(level), float(max_fraction)

@@ -34,7 +34,7 @@ from .SparseObjectives import (Objective, Logger, Timer, make_index_param,  # no
 from .ConjugateGradient import ConjugateGradientSolver  # noqa: F401
 from .ModelSensitivity import (LinearResponseCovariances, ArrowheadCovariance,  # noqa: F401
                                WeightSensitivityLinearApproximation)
-from .GLMM import (LogisticGLMM, GLMMPrior, DeviceCSR, Prediction, ApproximateLOO, ApproximateLOGO,  # noqa: F401
+from .GLMM import (LogisticGLMM, PoissonGLMM, GLMMPrior, DeviceCSR, Prediction, ApproximateLOO, ApproximateLOGO,  # noqa: F401
                    ApproximateMaxInfluence, DropResult, IJCovariance)
 
 __version__ = "0.1.0"

@@ -42,6 +42,8 @@ SIGNATURES = {
     "lrvb_glmm_create": (c_int32, [POINTER(c_void_p), c_int64, c_int32, c_int32, c_int32, _P, _P,
                                    _P, _P, POINTER(c_double), POINTER(c_double), POINTER(Prior),
                                    POINTER(Bounds), c_int32, _P]),
+    "lrvb_glmm_create_poisson": (c_int32, [POINTER(c_void_p), c_int64, c_int32, c_int32, _P, _P, _P, _P, _P,
+                                           POINTER(Prior), POINTER(Bounds), c_int32, _P]),
     "lrvb_glmm_destroy": (c_int32, [_P]),
     "lrvb_launch_count": (ctypes.c_longlong, []),
     "lrvb_glmm_set_timing": (c_int32, [_P, c_int32]),

@@ -358,6 +358,7 @@ extern "C" {
 
 int lrvb_glmm_third_contract(lrvb_glmm* h, const double* a_dev, double* t_dev, double* q_dev, void* stream) {
   LRVB_REQUIRE(h != nullptr, "lrvb_glmm_third_contract: NULL handle");
+  LRVB_REQUIRE_LOGISTIC(h, "lrvb_glmm_third_contract");
   LRVB_REQUIRE(a_dev && t_dev && (q_dev || h->N == 0), "lrvb_glmm_third_contract: NULL argument");
   if (!h->point_valid || h->vecmode) {
     set_error("lrvb_glmm_third_contract: no evaluation in free coordinates cached (call lrvb_glmm_eval first)");

@@ -30,6 +30,33 @@ __global__ void k_gptr(const int32_t* __restrict__ g, int32_t* __restrict__ gptr
   for (int gg = prev + 1; gg <= cur; ++gg) gptr[gg] = (int32_t)n;
 }
 
+// Poisson data checks beside k_gptr's, on the same flags word: 4 = a y that is negative or not finite, 8 = an
+// offset that is not finite.  Per-CTA partials of c = sum_n w_n lgamma(y_n + 1) (grid fixed by N: a fixed order).
+constexpr int kPoisConstCtas = 1024;
+__global__ void __launch_bounds__(256)
+k_pois_check(const double* __restrict__ y, const double* __restrict__ w, const double* __restrict__ off, int64_t N,
+             int* flags, double* __restrict__ part) {
+  __shared__ double red[32];
+  int bad = 0;
+  double c = 0.0;
+  for (int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; n < N; n += (int64_t)gridDim.x * blockDim.x) {
+    const double yn = y[n];
+    if (!(yn >= 0.0) || !isfinite(yn)) bad |= 4;
+    else c += (w ? w[n] : 1.0) * lgamma(yn + 1.0);
+    if (off && !isfinite(off[n])) bad |= 8;
+  }
+  if (bad) atomicOr(flags, bad);
+  c = block_sum(c, red);
+  if (threadIdx.x == 0) part[blockIdx.x] = c;
+}
+__global__ void __launch_bounds__(256) k_pois_const(const double* __restrict__ part, int n, double* __restrict__ c) {
+  __shared__ double red[32];
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) s += part[i];
+  s = block_sum(s, red);
+  if (threadIdx.x == 0) *c = s;
+}
+
 }  // namespace lrvb
 
 using namespace lrvb;
@@ -44,7 +71,7 @@ int lrvb_glmm_destroy(lrvb_glmm* h) {
   void* ptrs[] = {h->gh, h->gptr, h->vec, h->W, h->klpart, h->gradpart, h->gsc, h->BR, h->locpart, h->fin_counter, h->fin_pre,
                   h->jobs, h->gslots, h->grampart, h->bval, h->wc_scratch, h->B, h->L, h->gradl, h->outg, h->rowcnt, h->scanblk, h->csrwork, h->csrmask,
                   h->cgbuf, h->hvppart, h->dotpart, h->scal, h->flags, h->Linv, h->T,
-                  h->schurpart, h->pred_B, h->logo_V, h->amip_work, h->ij_work};
+                  h->schurpart, h->pred_B, h->logo_V, h->amip_work, h->ij_work, h->pois_work};
   for (void* p : ptrs)
     if (p) cudaFree(p);
   for (cudaEvent_t e : h->ev)
@@ -124,6 +151,101 @@ int lrvb_glmm_create(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, int32_t Q
   if (hflag) {
     set_error(hflag & 1 ? "lrvb_glmm_create: group id outside [0, G)"
                         : "lrvb_glmm_create: group ids must be non-decreasing (group-sorted)");
+    lrvb_glmm_destroy(h);
+    return LRVB_EINVAL;
+  }
+
+  CREATE_TRY(dev_alloc(&h->vec, (size_t)h->D + 8 + (size_t)K + (size_t)G));   // + k_prep's derived factors (prep_aux)
+  h->ldw = (N + 7) / 8 * 8;
+  CREATE_TRY(dev_alloc(&h->W, 5 * (size_t)h->ldw));
+
+  CREATE_TRY(plan_eval(h, st));
+
+  CREATE_TRY(dev_alloc(&h->B, (size_t)G * 2 * Dg));
+  CREATE_TRY(dev_alloc(&h->L, (size_t)G * 3));
+  CREATE_TRY(dev_alloc(&h->gradl, 2 * (size_t)G));
+  CREATE_TRY(dev_alloc(&h->outg, 1 + (size_t)Dg + (size_t)Dg * Dg));
+  h->A = h->outg + 1 + Dg;
+  CREATE_TRY(dev_alloc(&h->scal, 32));
+  CREATE_CUDA(cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking));
+  CREATE_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
+  CREATE_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
+  CREATE_CUDA(cudaStreamSynchronize(st));
+#undef CREATE_TRY
+#undef CREATE_CUDA
+  *out = h;
+  return LRVB_OK;
+}
+
+int lrvb_glmm_create_poisson(lrvb_glmm** out, int64_t N, int32_t K, int32_t G, const double* X_dev,
+                             const double* y_dev, const int32_t* g_dev, const double* w_dev, const double* offset_dev,
+                             const lrvb_glmm_prior* prior, const lrvb_glmm_bounds* bounds,
+                             int32_t include_global_terms, void* stream) {
+  LRVB_REQUIRE(out != nullptr, "lrvb_glmm_create_poisson: out is NULL");
+  *out = nullptr;
+  LRVB_REQUIRE(N >= 0 && N < (int64_t)2147483000, "lrvb_glmm_create_poisson: N = %lld out of range", (long long)N);
+  LRVB_REQUIRE(K >= 1 && K <= kMaxK, "lrvb_glmm_create_poisson: K = %d not in [1, %d]", K, kMaxK);
+  LRVB_REQUIRE(G >= 0, "lrvb_glmm_create_poisson: G = %d negative", G);
+  LRVB_REQUIRE(N == 0 || (X_dev && y_dev && g_dev), "lrvb_glmm_create_poisson: X, y, g must be non-NULL");
+  LRVB_REQUIRE(N == 0 || G >= 1, "lrvb_glmm_create_poisson: observations but no groups");
+  LRVB_REQUIRE(prior && bounds, "lrvb_glmm_create_poisson: NULL argument");
+  LRVB_REQUIRE((((uintptr_t)X_dev) & 15) == 0, "lrvb_glmm_create_poisson: X not 16-byte aligned");
+  LRVB_REQUIRE(N == 0 || ((((uintptr_t)y_dev) | ((uintptr_t)g_dev) | ((uintptr_t)w_dev) | ((uintptr_t)offset_dev)) &
+                          15) == 0,
+               "lrvb_glmm_create_poisson: y, g, w, offset must be 16-byte aligned (bulk async copies)");
+  cudaStream_t st = (cudaStream_t)stream;
+
+  lrvb_glmm* h = new (std::nothrow) lrvb_glmm();
+  LRVB_REQUIRE(h != nullptr, "out of host memory");
+  h->family = kFamilyPoisson;
+  h->N = N; h->K = K; h->G = G; h->Q = 0;
+  h->Dg = 4 + 2 * K;
+  h->D = h->Dg + 2 * (int64_t)G;
+  h->KT = (K + 7) / 8;
+  h->include_global = include_global_terms ? 1 : 0;
+  h->X = X_dev; h->y = y_dev; h->g = g_dev; h->w = w_dev; h->offset = N > 0 ? offset_dev : nullptr;
+  h->prior = *prior;
+  h->bounds = *bounds;
+  const int Dg = h->Dg;
+
+#define CREATE_TRY(expr)                         \
+  do {                                           \
+    int rc__ = (expr);                           \
+    if (rc__ != LRVB_OK) { lrvb_glmm_destroy(h); return rc__; } \
+  } while (0)
+#define CREATE_CUDA(call)                                                      \
+  do {                                                                         \
+    cudaError_t e__ = (call);                                                  \
+    if (e__ != cudaSuccess) {                                                  \
+      set_error("%s failed: %s", #call, cudaGetErrorString(e__));              \
+      lrvb_glmm_destroy(h);                                                    \
+      return LRVB_ECUDA;                                                       \
+    }                                                                          \
+  } while (0)
+
+  CREATE_TRY(dev_alloc(&h->flags, 8));
+  CREATE_CUDA(cudaMemsetAsync(h->flags, 0, sizeof(int) * 8, st));
+  CREATE_TRY(dev_alloc(&h->gptr, (size_t)G + 1));
+  k_gptr<<<cdiv(N + 1, 256), 256, 0, st>>>(g_dev, h->gptr, h->flags, N, G);
+  CREATE_CUDA(cudaGetLastError());
+  // c = sum_n w_n lgamma(y_n + 1), the part of the log-likelihood that does not depend on the parameters
+  const int nc = N == 0 ? 1 : (cdiv(N, 256) < kPoisConstCtas ? cdiv(N, 256) : kPoisConstCtas);
+  CREATE_TRY(dev_alloc(&h->pois_work, 1 + (size_t)nc));
+  CREATE_CUDA(cudaMemsetAsync(h->pois_work, 0, sizeof(double) * (1 + (size_t)nc), st));
+  if (N > 0) {
+    k_pois_check<<<nc, 256, 0, st>>>(y_dev, w_dev, h->offset, N, h->flags, h->pois_work + 1);
+    CREATE_CUDA(cudaGetLastError());
+    k_pois_const<<<1, 256, 0, st>>>(h->pois_work + 1, nc, h->pois_work);
+    CREATE_CUDA(cudaGetLastError());
+  }
+  int hflag = 0;
+  CREATE_CUDA(cudaMemcpyAsync(&hflag, h->flags, sizeof(int), cudaMemcpyDeviceToHost, st));
+  CREATE_CUDA(cudaStreamSynchronize(st));
+  if (hflag) {
+    set_error(hflag & 1 ? "lrvb_glmm_create_poisson: group id outside [0, G)"
+              : hflag & 2 ? "lrvb_glmm_create_poisson: group ids must be non-decreasing (group-sorted)"
+              : hflag & 4 ? "lrvb_glmm_create_poisson: y must be finite and >= 0 (counts)"
+                          : "lrvb_glmm_create_poisson: the offset must be finite");
     lrvb_glmm_destroy(h);
     return LRVB_EINVAL;
   }

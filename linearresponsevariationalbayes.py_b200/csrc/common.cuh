@@ -54,6 +54,14 @@ constexpr int kRT = 4;        // Schur warp job = kRT x kRT output tiles of 8x8 
 
 static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
+// The likelihood of a handle (lrvb_glmm_create / lrvb_glmm_create_poisson).  Only the observation pass depends on it;
+// the entry points whose epilogues evaluate the logistic likelihood refuse the other families.
+constexpr int kFamilyLogistic = 0;
+constexpr int kFamilyPoisson = 1;
+#define LRVB_REQUIRE_LOGISTIC(h, who)                                                             \
+  LRVB_REQUIRE((h)->family == lrvb::kFamilyLogistic,                                             \
+               "%s: not available for the Poisson family (its epilogue evaluates the logistic likelihood)", who)
+
 // Shared memory of k_obs (the observation pass for K > 62, glmm_eval.cu): nbuf 64-row tiles of X, the Q
 // quadrature nodes and weights (each padded to whole node slots of 4), 32 reduction values and 2 spare.
 inline size_t obs_smem(int K, int Q, int nbuf) {
@@ -282,10 +290,13 @@ struct lrvb_glmm {
   int64_t shard_g0 = 0, shard_G = 0;   // shard_G > 0: eval reads the FULL layout of a job with shard_G groups
   const double *X = nullptr, *y = nullptr, *w = nullptr;
   const int32_t* g = nullptr;
+  int family = 0;             // lrvb::kFamilyLogistic / kFamilyPoisson
+  const double* offset = nullptr;   // Poisson: (N) offset of the linear predictor, or NULL
+  double* pois_work = nullptr;      // Poisson: [c = sum_n w_n lgamma(y_n + 1) | per-CTA partials of c]
   lrvb_glmm_prior prior;
   lrvb_glmm_bounds bounds;
   // ---- device-owned ----
-  double* gh = nullptr;       // [2][Q]: c_q = sqrt(2) x_q ; what_q = w_q / sqrt(pi)
+  double* gh = nullptr;       // [2][Q]: c_q = sqrt(2) x_q ; what_q = w_q / sqrt(pi) (NULL and Q = 0 for Poisson)
   int32_t* gptr = nullptr;    // (G+1) first observation of each group
   double* vec = nullptr;      // (D) constrained values
   double* W = nullptr;        // (5, ldw) per-observation derivative weights

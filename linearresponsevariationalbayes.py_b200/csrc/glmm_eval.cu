@@ -15,8 +15,10 @@
 //     K <= 24, order 2   k_fused_eval (fused.cuh) also computes the Gram: one pass over X
 //     K <= 62            k_obs_fused (obs_fused.cuh), one-slot rings
 //     K > 62             k_obs, then k_group
+//     Poisson handles    k_obs_pois (pois.cuh, closed form, every K), then k_group
 //   Gram            X^T diag(a) X, X^T diag(b) S, S^T diag(c) S on the FP64 tensor cores (DMMA), order 2:
-//                   k_gram_mid (K <= 104), k_gram_wide (gram_wide_eligible), k_gram_big (the rest)
+//                   k_gram_mid (K <= 104; K <= 24 only for Poisson handles), k_gram_wide (gram_wide_eligible),
+//                   k_gram_big (the rest)
 //   k_finish, k_global_post   straddling-group fix-up, chain rule to free coordinates, non-data terms
 #include <stdlib.h>
 #include "common.cuh"
@@ -28,6 +30,7 @@
 #define LRVB_GRAM_WIDE_KERNELS
 #include "gram_wide.cuh"
 #include "fused.cuh"
+#include "pois.cuh"
 
 namespace lrvb {
 
@@ -536,6 +539,22 @@ k_group(const double* __restrict__ X, const double* __restrict__ W,
 // the per-CTA partials of X^T l_m, S^T l_v go to gradpart (*n_gp of them), the per-group sums to gsc and BR.  The
 // cached evaluation's W (lrvb_glmm_obs_weights) stays intact.  K <= 62: the two-slot fused observation pass,
 // which writes no W, then k_obs_fixup<1>; K > 62: k_obs<1>, writing l_m, l_v into a scratch block, then k_group<1>.
+// Poisson handles: k_obs_pois<1> into the scratch block, then k_group<1>.
+static PoisArgs pois_args(const lrvb_glmm* h, const double* w) {
+  PoisArgs a;
+  a.X = h->X; a.y = h->y; a.g = h->g; a.w = w; a.off = h->offset; a.vec = h->vec; a.N = h->N; a.K = h->K; a.G = h->G;
+  return a;
+}
+// the Poisson observation pass with weights w into W (the caller checks the launch)
+static void launch_obs_pois(lrvb_glmm* h, const double* w, int order, double* W, cudaStream_t st) {
+  const PoisArgs a = pois_args(h, w);
+  if (order == 0)
+    k_obs_pois<0><<<h->obs_grid, kPoThreads, h->obs_smem, st>>>(a, h->pois_work, W, h->ldw, h->klpart, h->gradpart);
+  else if (order == 1)
+    k_obs_pois<1><<<h->obs_grid, kPoThreads, h->obs_smem, st>>>(a, h->pois_work, W, h->ldw, h->klpart, h->gradpart);
+  else
+    k_obs_pois<2><<<h->obs_grid, kPoThreads, h->obs_smem, st>>>(a, h->pois_work, W, h->ldw, h->klpart, h->gradpart);
+}
 int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t st) {
   const int K = h->K, G = h->G, Q = h->Q;
   const int64_t N = h->N;
@@ -564,8 +583,11 @@ int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t s
                 sizeof(double) * 2 * (size_t)h->ldw);
       return LRVB_ECUDA;
     }
-    k_obs<1><<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, h->wc_scratch, h->klpart,
-                                                    h->gradpart, N, h->ldw, K, G, Q, h->obs_nbuf);
+    if (h->family == kFamilyPoisson)
+      launch_obs_pois(h, dw, 1, h->wc_scratch, st);
+    else
+      k_obs<1><<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, dw, h->vec, h->gh, h->wc_scratch, h->klpart,
+                                                      h->gradpart, N, h->ldw, K, G, Q, h->obs_nbuf);
     LRVB_CHECK_LAUNCH();
     *n_gp = h->obs_grid;
   }
@@ -581,6 +603,12 @@ int launch_wide_influence(lrvb_glmm* h, const double* v, double* out, cudaStream
   LRVB_TRY(raise_smem_limit(k_obs_influence_wide, h->obs_smem));
   k_obs_influence_wide<<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, h->vec, h->gh, v, out, h->N, h->K,
                                                              h->G, h->Q, h->obs_nbuf, h->bounds, h->vecmode);
+  LRVB_CHECK_LAUNCH();
+  return LRVB_OK;
+}
+// The influence pass of Poisson handles (lrvb_glmm_weight_cross_rmatvec)
+int launch_pois_influence(lrvb_glmm* h, const double* v, double* out, cudaStream_t st) {
+  k_pois_influence<<<h->obs_grid, kPoThreads, h->obs_smem, st>>>(pois_args(h, nullptr), v, out, h->bounds, h->vecmode);
   LRVB_CHECK_LAUNCH();
   return LRVB_OK;
 }
@@ -1095,6 +1123,8 @@ k_global_post(const double* __restrict__ vec, const double* locpart, int K, int 
   global_post<ORDER>(vec, ga, locpart, K, G, bd, vecmode);
 }
 
+static GramMidKernel gram_mid_kernel_ij(int K);
+
 // ------------------------------------------------------------------------------------------
 int plan_eval(lrvb_glmm* h, cudaStream_t st) {
   const int K = h->K, G = h->G, Q = h->Q;
@@ -1107,7 +1137,21 @@ int plan_eval(lrvb_glmm* h, cudaStream_t st) {
     h->obs_grid = (int)(nt < kNumSMs ? nt : kNumSMs);
     if (h->obs_grid < 1) h->obs_grid = 1;
   }
-  if (K <= kOfMaxK) {
+  if (h->family == kFamilyPoisson) {
+    // k_obs_pois (pois.cuh) at every K, persistent CTAs: as many as fit on the device, at most one per tile.  No
+    // fused kernel: K <= 62 takes the K > 62 path, with k_gram_mid for the Gram down to K = 1.
+    h->obs_smem = pois_smem(K);
+    LRVB_TRY(raise_smem_limit(k_obs_pois<0>, h->obs_smem));
+    LRVB_TRY(raise_smem_limit(k_obs_pois<1>, h->obs_smem));
+    LRVB_TRY(raise_smem_limit(k_obs_pois<2>, h->obs_smem));
+    LRVB_TRY(raise_smem_limit(k_pois_influence, h->obs_smem));
+    int per_sm = 0;
+    LRVB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_obs_pois<2>, kPoThreads, h->obs_smem));
+    if (per_sm < 1) per_sm = 1;
+    const int64_t nt = (N + pois_rows(K) - 1) / pois_rows(K);
+    h->obs_grid = (int)(nt < (int64_t)per_sm * kNumSMs ? nt : (int64_t)per_sm * kNumSMs);
+    if (h->obs_grid < 1) h->obs_grid = 1;
+  } else if (K <= kOfMaxK) {
     // fused observation + group pass: every warp owns a contiguous multiple-of-32 range of rows.  The two-slot
     // geometry (of_*) serves the weight-cross pass (launch_weight_pass) and the influence pass (k_obs_influence).
     h->obs_fused = 1;
@@ -1193,8 +1237,9 @@ int plan_eval(lrvb_glmm* h, cudaStream_t st) {
     // no Gram kernel: the one-pass kernel (fused.cuh) writes the packed partials, one slab per CTA
     npart = (size_t)h->fu_grid * gram_small_shape(K).NT * 64;
   } else if (K <= kGmMaxK) {
-    // 24 < K <= 104: one warp or a team of warps = the whole packed triangle (gram_mid.cuh)
-    const GramMidKernel gk = gram_mid_kernel(K);
+    // 24 < K <= 104 (Poisson handles: K <= 104): one warp or a team of warps = the whole packed triangle
+    // (gram_mid.cuh); K <= 24 takes the instantiations of the IJ
+    const GramMidKernel gk = gram_mid_kernel_ij(K);
     h->gram_mid = 1;
     h->gm_kernel = gk.fn;
     h->gm_warps = gk.warps;
@@ -1310,7 +1355,8 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
 #define LRVB_OBS(O)                                                                          \
   k_obs<O><<<h->obs_grid, 256, h->obs_smem, st>>>(h->X, h->y, h->g, h->w, h->vec, h->gh, \
                                                    h->W, h->klpart, h->gradpart, N, h->ldw, K, G, Q, h->obs_nbuf)
-    if (order == 0) LRVB_OBS(0);
+    if (h->family == kFamilyPoisson) launch_obs_pois(h, h->w, order, h->W, st);
+    else if (order == 0) LRVB_OBS(0);
     else if (order == 1) LRVB_OBS(1);
     else LRVB_OBS(2);
 #undef LRVB_OBS
@@ -1430,9 +1476,10 @@ int launch_eval(lrvb_glmm* h, const double* free_dev, int order, double* out_glo
 // packed Gram of the evaluation with the weights (a, b, c) = (W_m^2, W_m W_v, W_v^2), and the per-group sums
 // E_g, F_g are k_group<2>'s on the same weights.  Both kernels are compiled here, so their IJ launches are too.
 //
-// K <= 24 has no stand-alone Gram kernel in the evaluation (the one-pass kernel of fused.cuh computes the Gram):
-// the k_gram_mid instantiations of T2 = 1 .. 6 serve the IJ there, through a lookup of their own so that the
-// evaluation's plan is unchanged.  Above, the IJ runs the handle's own Gram plan.
+// K <= 24 has no stand-alone Gram kernel in the logistic evaluation (the one-pass kernel of fused.cuh computes the
+// Gram): the k_gram_mid instantiations of T2 = 1 .. 6 serve the IJ there, through a lookup of their own so that the
+// logistic evaluation's plan is unchanged; they are also the Gram kernels of Poisson handles with K <= 24.  Above,
+// the IJ runs the handle's own Gram plan.
 static GramMidKernel gram_mid_kernel_ij(int K) {
   if (K > kFuMaxK) return gram_mid_kernel(K);
   const int T2 = (2 * K + 7) / 8, T0 = K / 8;

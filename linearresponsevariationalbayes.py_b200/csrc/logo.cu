@@ -272,6 +272,7 @@ extern "C" {
 int lrvb_glmm_logo(lrvb_glmm* h, const double* Sinv_dev, const double* Pinv_dev, double* delta_dev,
                    double* group_out_dev, double* row_out_dev, void* stream) {
   LRVB_REQUIRE(h != nullptr, "lrvb_glmm_logo: NULL handle");
+  LRVB_REQUIRE_LOGISTIC(h, "lrvb_glmm_logo");
   if (!h->hess_valid || h->vecmode) {
     set_error("lrvb_glmm_logo: no Hessian in free coordinates cached (call lrvb_glmm_eval with order 2)");
     return LRVB_ESTATE;

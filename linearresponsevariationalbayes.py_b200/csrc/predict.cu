@@ -413,6 +413,7 @@ extern "C" {
 int lrvb_glmm_predict(lrvb_glmm* h, const double* free_dev, const double* X_dev, int32_t K, const int32_t* g_dev, const int64_t* order_dev,
                       int64_t M, double* out_dev, void* stream) {
   LRVB_TRY(check_rows(h, "lrvb_glmm_predict", X_dev, K, g_dev, M, out_dev));
+  LRVB_REQUIRE_LOGISTIC(h, "lrvb_glmm_predict");
   LRVB_REQUIRE(free_dev != nullptr, "lrvb_glmm_predict: free is NULL");
   if (M == 0) return LRVB_OK;
   return launch_predict<false, 0>(h, free_dev, X_dev, g_dev, order_dev, M, nullptr, nullptr, nullptr, out_dev, (cudaStream_t)stream);
@@ -439,6 +440,7 @@ int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cro
                          const double* X_dev, int32_t K, const int32_t* g_dev, const int64_t* order_dev, int64_t M,
                          double* out_dev, void* stream) {
   LRVB_TRY(check_rows(h, "lrvb_glmm_predict_lr", X_dev, K, g_dev, M, out_dev));
+  LRVB_REQUIRE_LOGISTIC(h, "lrvb_glmm_predict_lr");
   if (!h->hess_valid || h->vecmode) {
     set_error("lrvb_glmm_predict_lr: no Hessian in free coordinates cached (call lrvb_glmm_eval with order 2)");
     return LRVB_ESTATE;
@@ -459,6 +461,7 @@ int lrvb_glmm_predict_lr(lrvb_glmm* h, const double* Sinv_dev, const double* cro
 int lrvb_glmm_loo(lrvb_glmm* h, const double* Sinv_dev, const double* cross_dev, const double* localcov_dev,
                   double* out_dev, void* stream) {
   LRVB_REQUIRE(h != nullptr, "lrvb_glmm_loo: NULL handle");
+  LRVB_REQUIRE_LOGISTIC(h, "lrvb_glmm_loo");
   if (!h->hess_valid || h->vecmode) {
     set_error("lrvb_glmm_loo: no Hessian in free coordinates cached (call lrvb_glmm_eval with order 2)");
     return LRVB_ESTATE;

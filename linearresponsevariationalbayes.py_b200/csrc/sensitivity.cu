@@ -18,6 +18,7 @@ namespace lrvb {
 // glmm_eval.cu: the observation and group passes with dw as the weights; the influence pass for K > 62
 int launch_weight_pass(lrvb_glmm* h, const double* dw, int* n_gp, cudaStream_t st);
 int launch_wide_influence(lrvb_glmm* h, const double* v, double* out, cudaStream_t st);
+int launch_pois_influence(lrvb_glmm* h, const double* v, double* out, cudaStream_t st);
 
 // out = C dw from the sums of the fused pass run with weights dw (gradpart: X^T l_m, S^T l_v per
 // CTA; gsc: per-group sum l_m, sum l_v).  Signs / Jacobians as in k_global / k_local (data terms only).
@@ -208,6 +209,7 @@ int lrvb_glmm_weight_cross_rmatvec(lrvb_glmm* h, const double* v_dev, double* ou
     return LRVB_ESTATE;
   }
   if (h->N == 0) return LRVB_OK;
+  if (h->family == kFamilyPoisson) return launch_pois_influence(h, v_dev, out_dev, (cudaStream_t)stream);
   if (!h->obs_fused) return launch_wide_influence(h, v_dev, out_dev, (cudaStream_t)stream);
   const size_t smem = h->of_smem + sizeof(double) * (2 * (size_t)h->K + 2);
   LRVB_TRY(raise_smem_limit(k_obs_influence, smem));
